@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Benchmark of the LAPF step-2 hot path on B200 (contract: see the task statement / DESIGN.md).
+"""Benchmark of the LAPF step-2 hot path on B200 (see DESIGN.md).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] ...               # the reference algorithm on host cores
+    python bench.py --dump-outputs DIR ...                        # also write the last timed step's chain rows
 
 Workload (BASELINE.json configs[2], the single-GPU throughput configuration): 65,536 independent
 walkers per GPU spread over 100 synthetic NIRC2-like epochs, 64 x 64 stamps, 2-body model.
@@ -30,6 +31,7 @@ if ROOT not in sys.path:
 HEADER = {"itime": 1.0, "coadds": 1, "multisam": 1, "sampmode": 2}
 METRIC = "pixel_model_evals_per_sec"
 UNIT = "pixel-evals/s"
+DUMP_BYTES = 32 << 20           # --dump-outputs: small enough to keep and compare two builds' dumps
 
 
 def parse_args():
@@ -51,7 +53,16 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-latency", action="store_true", help="skip the 1-walker / 64-walker block (BASELINE configs 1-2)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the chain rows the last timed step returned (rank 0's walkers, "
+                         "float64) to DIR/chain.npy; above %d MiB a sample of walkers drawn with --seed stands for them"
+                         % (DUMP_BYTES >> 20))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's chain; --impl reference keeps none")
+    return a
 
 
 def workload_name(a):
@@ -242,6 +253,22 @@ def latency_block(a, dev):
     return out
 
 
+def dump_outputs(out_dir, chain, seed):
+    """Write chain rows [rows, walkers, P+1] to out_dir/chain.npy.  When they exceed DUMP_BYTES, a
+    sample of walkers (drawn from ``seed``, kept in walker order) is written instead, the same
+    walkers for the same arguments, so the dumps of two builds compare element for element."""
+    import torch
+    rows, walkers, cols = chain.shape
+    keep = min(walkers, DUMP_BYTES // max(1, rows * cols * chain.element_size()))
+    if keep < 1:
+        raise SystemExit("--dump-outputs: the rows of one walker exceed %d bytes" % DUMP_BYTES)
+    if keep < walkers:
+        idx = np.sort(np.random.default_rng(seed).choice(walkers, keep, replace=False))
+        chain = chain.index_select(1, torch.from_numpy(idx).to(chain.device))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "chain.npy"), chain.cpu().numpy())
+
+
 def run_b200(a):
     cpu = None
     world_env = int(os.environ.get("WORLD_SIZE", 1))
@@ -340,6 +367,8 @@ def run_b200(a):
     secs = ms * 1e-3
     updates = float(W) * U * a.steps * world
     value = updates * S * S / secs
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, chain[:rows], a.seed)
 
     # ---- end to end through the public API, host buffers in, host buffers out --------------
     # Every e2e step is a NEW batch of epochs: frames, starting points come from pinned host
