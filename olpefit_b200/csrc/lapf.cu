@@ -577,10 +577,12 @@ __global__ void __launch_bounds__(NW * 32, MINB) gibbs_kernel(const __grid_const
 // coefficients of the trial vector, culling bounds, accept/reject, counters, chain row -- is done
 // with ONE WALKER PER LANE, once per round, and costs 1/LW of a warp instruction per update.  In
 // between, the warp evaluates the trial vectors one after the other (a "pass": block table, lane
-// constants, pixel loop, butterfly sum), reading each walker's coefficients from its
-// shared-memory image.  FP64 state lives in global memory (L1/L2 resident: one parameter read
-// and at most one written per update).  The arithmetic per walker is the one of run_walker: chains
-// are bit-identical between the two forms.
+// constants, pixel loop, FP64 reduction of the lane partials), reading each walker's coefficients
+// from its shared-memory image.  At 64 pixels the reduction of all passes waits for the end of the
+// round: a pass leaves its lane partials in the image it has read, and each walker's lane adds its
+// 32 partials in the butterfly's order (warp_sum_f64_of).  FP64 state lives in global memory
+// (L1/L2 resident: one parameter read and at most one written per update).  The arithmetic per
+// walker is the one of run_walker: chains are bit-identical between the two forms.
 // ---------------------------------------------------------------------------------------------
 // `frame0`, `frame1`: the frames in the two pixel-store slots (frame1 < 0: none; both uniform over the CTA);
 // `slot`: the slot of the lane's walker; `la`: lanes [0, la) of this warp use one slot, [la, nl) the other
@@ -594,6 +596,9 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
     using L = Layout<NB>;
     using I = CoefImg<NB, Geo<NX>::PANELS>;
     constexpr int P = L::P;
+    // one-panel, one-table stamps evaluated one walker per pass (64 pixels): see the passes below
+    constexpr bool LANE_SUMS = WPP == 1 && Geo<NX>::PANELS == 1 && Rows<NY, 1>::HALVES == 1;
+    static_assert(!LANE_SUMS || I::STRIDE >= 32, "a walker's image holds the 32 lane partials of its pass");
     const bool mine = wl >= 0;
     const uint64_t gid = (uint64_t)(a.id_base + (int64_t)wl * a.id_stride);
     const bool two = TM == 1 && frame1 >= 0;
@@ -645,13 +650,31 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
             // pass.  (With two vectors per pass it keeps its partner company in the factorised loop instead.)
             skip = nv != nv;
             if (skip && WPP > 1) cf.fast = true;
+            if (LANE_SUMS && !skip) n_exps += cf.nexp;
             store_coef<NB, Geo<NX>::PANELS>(img + lane * I::STRIDE, cf, slot | (skip ? 2 : 0));
         }
         __syncwarp();
 
         // ---- passes: the warp evaluates chi-square of its walkers' trial vectors in turn --------
         double chi_t = 0.0;
-        if constexpr (WPP == 1) {
+        if constexpr (LANE_SUMS) {
+            // each pass leaves its 32 lane partials in its walker's image (read, hence dead, by then); the
+            // walker's lane reduces them after the last pass: one reduction per round instead of a butterfly per pass
+#pragma unroll 1
+            for (int i = 0; i < nl; ++i) {
+                Coef<NB> cf;
+                int sl = 0;
+                float* slot_img = img + i * I::STRIDE;
+                load_coef<NB, 1>(cf, slot_img, &sl);
+                if (sl & 2) continue;                   // a nan proposal: no pass (uniform: the image is the warp's)
+                __syncwarp();                           // every lane has read the image before any lane overwrites it
+                const float part = lane_chi2<NB, NX, NY, TM>(cf, rt, sd, sw, lane,
+                                                             TM == 1 ? tmem + (uint32_t)(sl & 1) * slot_cols : tmem);   // :314-316
+                slot_img[lane] = part;
+            }
+            __syncwarp();
+            if (mine) chi_t = warp_sum_f64_of(img + lane * I::STRIDE);
+        } else if constexpr (WPP == 1) {
 #pragma unroll 1
             for (int i = 0; i < nl; ++i) {
                 Coef<NB> cf;

@@ -69,6 +69,24 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
     return v;   // identical in every lane: xor-butterfly adds the same pairs everywhere
 }
 
+// warp_sum_f64 of the lane values (double)p[0..31], worked out by ONE thread from the 32 values in
+// shared memory (16-byte aligned).  Lane 0 of the butterfly adds p[0] + p[16], then the partner
+// 8, 4, 2, 1 lanes away; this is that tree, operand for operand, so the result is bit-identical.
+__device__ __forceinline__ double warp_sum_f64_of(const float* __restrict__ p) {
+    double v[16];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+        const float4 a = reinterpret_cast<const float4*>(p)[q], b = reinterpret_cast<const float4*>(p)[q + 4];
+        v[4 * q] = (double)a.x + (double)b.x; v[4 * q + 1] = (double)a.y + (double)b.y;
+        v[4 * q + 2] = (double)a.z + (double)b.z; v[4 * q + 3] = (double)a.w + (double)b.w;
+    }
+#pragma unroll
+    for (int off = 8; off >= 1; off >>= 1)
+#pragma unroll
+        for (int l = 0; l < off; ++l) v[l] += v[l + off];
+    return v[0];
+}
+
 // mbarrier + 1-D TMA bulk copy (global -> shared), used to stage a stamp once per frame.
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -258,12 +276,13 @@ __device__ __forceinline__ void load_shape(Coef<NB>& cf, int which, const float*
 
 // Shared-memory image of a Coef: 16-byte slots, an ODD number of them per walker, so that both the
 // one-walker-per-lane accesses of the batched sampler and its broadcast reads are conflict-free
-// 128-bit transactions.
+// 128-bit transactions.  At least 32 floats: once its pass has read it, the batched sampler reuses a
+// walker's image for the pass's 32 lane partials of chi-square.
 template <int NB, int PANELS>
 struct CoefImg {
     static constexpr int K = 2 * NB;
     static constexpr int WORDS = 3 * K + 7 + 4 * PANELS + 3;   // x0 y0 amp | sa sb sc floor | segments | nexp fast slot
-    static constexpr int V4 = ((WORDS + 3) / 4) | 1;
+    static constexpr int V4 = ((WORDS + 3) / 4 > 8 ? (WORDS + 3) / 4 : 8) | 1;
     static constexpr int STRIDE = 4 * V4;             // floats per walker
 };
 
@@ -368,12 +387,15 @@ struct Geo {
 // Block table: everything that depends on the rows only, computed ONCE per proposal by the warp
 // (one 2-row block per lane) instead of once per step by every lane.  One entry of Tab::RS floats
 // per block, with yb the centre of its two rows and dyb_k = yb - y0_k:
-//   [2k], [2k+1]              sb_k * dyb_k,  sc_k * dyb_k^2        for component k < K
+//   [4q .. 4q + 3]            sb dyb_ka, sb dyb_kb, sc dyb_ka^2, sc dyb_kb^2   piece q < NB: the components
+//                             ka = Tab::ka(q), kb = Tab::kb(q), each with the sb, sc of its own class
 //   [2K + 8c .. 2K + 8c + 7]  T_c,ij = 2^(j (sb dyb_c + i sb) + 2 i sc dyb_c + sc / 4)   shape class c,
 //                             i = -1/2 then +1/2 (row), j = -3/2, -1/2, 1/2, 3/2 (column)
-// The first pair gives the exponent of component k at the centre of a lane's block,
+// The first terms give the exponent of component k at the centre of a lane's block,
 //   q0 = fma(dxa, fma(sa, dxa, sb*dyb), sc*dyb^2),        dxa = anchor column - x0_k;
-// T moves it to the 8 pixels of the block (see row_steps_fast).  y0_c is the centre of the class's
+// T moves it to the 8 pixels of the block (see row_steps_fast).  Pieces 0 and 1 are the two objects'
+// components of class 0 and of class 1: they share sa, so one packed FMA pair (fma.rn.f32x2, rounded
+// per element like fma.rn.f32) works out both exponents.  y0_c is the centre of the class's
 // FIRST component; the other components of the class fold their offset into the lane constants.
 // The entry is padded to 28 floats so the blocks of a warp step read distinct banks.
 template <int NB>
@@ -381,7 +403,10 @@ struct Tab {
     static constexpr int K = 2 * NB;
     static constexpr int RS = 28;
     static constexpr int OFF_T = 2 * K;
+    static_assert(NB == 2 || NB == 3, "pieces 0, 1: class 0, 1 of objects 0 and 1; piece 2: object 2");
     static_assert(OFF_T + 16 <= RS && OFF_T % 4 == 0, "block table entry layout");
+    __host__ __device__ static constexpr int ka(int q) { return q < 2 ? q : 4; }
+    __host__ __device__ static constexpr int kb(int q) { return q < 2 ? q + 2 : 5; }
 };
 
 // A table covers TR rows of the stamp; taller stamps are walked table by table ("half").  A team
@@ -411,7 +436,7 @@ struct Scratch {
     static constexpr int TEAM_FLOATS = TEAM * TAB + Geo<NX>::PANELS * CT;
 };
 
-// A block's entry is 2 + K/2 independent 16-byte pieces (K/2 component pairs, 4 (class, row)
+// A block's entry is 2 + K/2 independent 16-byte pieces (K/2 anchor pieces, 4 (class, row)
 // factor quadruples).  Team members, whose tables have 8 blocks or fewer, spread the pieces of a
 // block over 4 lanes, with the same instruction stream in every lane (the piece is picked with
 // selects): a quarter of the instructions and of the serialised MUFUs on the latency path of an
@@ -440,18 +465,24 @@ __device__ __forceinline__ void build_row_table(float* __restrict__ rt, const Co
             const int step = (jb / G::BPS) * TEAM + tw;
             const float yb = (float)(row0 + step * G::RG + 2 * (jb % G::BPS)) + 0.5f;
             float4* o = reinterpret_cast<float4*>(rt + jb * T::RS);
-            // component pairs q = part, part + SPLIT, ...: (sb dyb, sc dyb^2) of the object's core and wing
+            // anchor pieces q = part, part + SPLIT, ...: (sb dyb, sc dyb^2) of components T::ka(q), T::kb(q)
 #pragma unroll
             for (int q0 = 0; q0 < NQ; q0 += SPLIT) {
                 const int q = q0 + part;
                 if (NQ % SPLIT == 0 || q < NQ) {
-                    float y0a = cf.y0[2 * q0], y0b = cf.y0[2 * q0 + 1];
+                    float y0a = cf.y0[T::ka(q0)], y0b = cf.y0[T::kb(q0)];
+                    float sba = cf.sb[T::ka(q0) & 1], sbb = cf.sb[T::kb(q0) & 1];
+                    float sca = cf.sc[T::ka(q0) & 1], scb = cf.sc[T::kb(q0) & 1];
 #pragma unroll
                     for (int t = 1; t < SPLIT; ++t)
-                        if (q0 + t < NQ && part == t) { y0a = cf.y0[2 * (q0 + t)]; y0b = cf.y0[2 * (q0 + t) + 1]; }
+                        if (q0 + t < NQ && part == t) {
+                            const int ka = T::ka(q0 + t), kb = T::kb(q0 + t);
+                            y0a = cf.y0[ka]; y0b = cf.y0[kb];
+                            sba = cf.sb[ka & 1]; sbb = cf.sb[kb & 1]; sca = cf.sc[ka & 1]; scb = cf.sc[kb & 1];
+                        }
                     const float yda = __fsub_rn(yb, y0a), ydb = __fsub_rn(yb, y0b);
-                    o[q] = make_float4(__fmul_rn(cf.sb[0], yda), __fmul_rn(__fmul_rn(cf.sc[0], yda), yda),
-                                       __fmul_rn(cf.sb[1], ydb), __fmul_rn(__fmul_rn(cf.sc[1], ydb), ydb));
+                    o[q] = make_float4(__fmul_rn(sba, yda), __fmul_rn(sbb, ydb),
+                                       __fmul_rn(__fmul_rn(sca, yda), yda), __fmul_rn(__fmul_rn(scb, ydb), ydb));
                 }
             }
             // factor quadruples pr = 2 c + ii = part, part + SPLIT, ...
@@ -775,9 +806,10 @@ __device__ __forceinline__ void row_steps(const Coef<NB>& cf, const float2 (&xd)
 //                                                       dy0_k = y0_c - y0_k
 //     T_c,ij = 2^(j sb (dyb_c + i) + 2 i sc dyb_c + sc / 4)                          block table, shared by the class
 // and a class adds  T_c,ij * sum_k C_k,ij E_k  to the pixel: per pixel pair NB + 1 packed
-// operations for NB components, plus 2 FFMA + 1 MUFU per component for the anchor.  A warp step
-// of 8 pixels x 4 components is 32 packed + 8 scalar FP32 instructions and 4 MUFU (plain loop: 56
-// packed and 32 MUFU): the loop is bound by FP32 issue, not by the SFU.
+// operations for NB components, plus 2 FMA (one packed FMA pair serves the two objects' components
+// of a class) + 1 MUFU per component for the anchor.  A warp step of 8 pixels x 4 components is 36
+// packed FP32 instructions and 4 MUFU (plain loop: 56 packed and 32 MUFU): the loop is bound by FP32
+// issue, not by the SFU.
 template <int NB>
 struct LaneK {
     static constexpr int K = 2 * NB;
@@ -938,23 +970,30 @@ __device__ __forceinline__ void row_steps_fast(const Coef<NB>& cf, const LaneK<N
 #pragma unroll
         for (int j = 0; j < 4; ++j) m[j] = make_float2(cf.floor, cf.floor);
         if (KIND > 0) {
-            float rc[2 * K];
-#pragma unroll
-            for (int q = 0; q < 2 * K / 4; ++q) {
-                const float4 t4 = reinterpret_cast<const float4*>(rp)[q];
-                rc[4 * q] = t4.x; rc[4 * q + 1] = t4.y; rc[4 * q + 2] = t4.z; rc[4 * q + 3] = t4.w;
-            }
 #pragma unroll
             for (int c = (KIND == 2 ? 0 : 1); c < 2; ++c) {
                 const float4 T0 = reinterpret_cast<const float4*>(rp + T::OFF_T)[2 * c];
                 const float4 T1 = reinterpret_cast<const float4*>(rp + T::OFF_T)[2 * c + 1];
+                // anchor exponents of the class: objects 0 and 1 as one packed pair (table piece c), object 2 on its own
+                float ea[NB];
+                {
+                    const float4 r = reinterpret_cast<const float4*>(rp)[c];
+                    const float2 dx = make_float2(lk.dxa[c], lk.dxa[2 + c]);
+                    const float2 q = __ffma2_rn(dx, __ffma2_rn(make_float2(cf.sa[c], cf.sa[c]), dx, make_float2(r.x, r.y)),
+                                                make_float2(r.z, r.w));
+                    ea[0] = ex2_approx(q.x);
+                    ea[1] = ex2_approx(q.y);
+                }
+                if (NB > 2) {
+                    const float4 r = reinterpret_cast<const float4*>(rp)[2];
+                    const float dx = lk.dxa[4 + c];
+                    ea[NB - 1] = ex2_approx(__fmaf_rn(dx, __fmaf_rn(cf.sa[c], dx, c ? r.y : r.x), c ? r.w : r.z));
+                }
                 float2 u[4];
 #pragma unroll
                 for (int o = 0; o < NB; ++o) {
                     const int k = 2 * o + c;
-                    const float q = __fmaf_rn(lk.dxa[k], __fmaf_rn(cf.sa[c], lk.dxa[k], rc[2 * k]), rc[2 * k + 1]);
-                    const float e = ex2_approx(q);
-                    const float2 e2 = make_float2(e, e);
+                    const float2 e2 = make_float2(ea[o], ea[o]);
 #pragma unroll
                     for (int p = 0; p < 4; ++p)
                         u[p] = (o == 0) ? __fmul2_rn(lk.C[k][p], e2) : __ffma2_rn(lk.C[k][p], e2, u[p]);
@@ -985,6 +1024,77 @@ __device__ __forceinline__ void row_steps_fast(const Coef<NB>& cf, const LaneK<N
     sp.rp = rp; sp.dp = dp; sp.wp = wp; sp.mp = mp; sp.tm = tm;
 }
 
+// This lane's FP32 partial of chi-square over one panel of one table ("half") of the stamp, by ONE
+// warp, with the block table of that half already built in `scratch` (if cf.fast).  The column
+// table goes to the scratch behind it.
+template <int NB, int NX, int NY, bool STORE, bool PREP, int TM = 0>
+__device__ __forceinline__ float panel_chi2(const Coef<NB>& cf, float* __restrict__ scratch,
+                                            const float* __restrict__ d, const float* __restrict__ w,
+                                            float* __restrict__ model_out, int lane, int half, int pan, uint32_t tmem) {
+    using G = Geo<NX>;
+    using T = Tab<NB>;
+    using R = Rows<NY, 1>;
+    constexpr int K = 2 * NB;
+    constexpr int TR = R::TR;
+    constexpr int STEPS = TR / G::RG;            // warp steps per table (per panel)
+    static_assert(TM == 0 || PREP, "the TMEM pixel store holds prepared stamps");
+    static_assert(TM != 1 || (R::HALVES == 1 && G::PANELS == 1), "both planes fit the 512 TMEM columns up to 64 x 64 pixels");
+    constexpr int TM_STEP = TM == 1 ? 16 : 8;     // TMEM columns per warp step
+    static_assert(TR % G::RG == 0, "unsupported stamp height");
+    const float* rt = scratch;
+    float* ct = scratch + Scratch<NB, NX, NY>::TAB;
+    const int a = lane % G::GPR, b = lane / G::GPR;
+    const int off0 = (half * TR + 2 * b) * NX + pan * G::PW + 4 * a;   // the lane's block of warp step 0
+    // segments of this panel, clipped to the warp steps of this table:
+    //   [0,wlo) none, [wlo,nlo) wings, [nlo,nhi1) all, [nhi1,whi1) wings, [whi1,STEPS) none
+    const bool p1 = G::PANELS > 1 && pan > 0;   // (constant indices keep the coefficients in registers)
+    int wlo = p1 ? cf.seg[1][0] : cf.seg[0][0], nlo = p1 ? cf.seg[1][1] : cf.seg[0][1];
+    int nhi1 = p1 ? cf.seg[1][2] : cf.seg[0][2], whi1 = p1 ? cf.seg[1][3] : cf.seg[0][3];
+    if (R::HALVES > 1) {
+        const int base = half * STEPS;
+        wlo = min(max(wlo - base, 0), STEPS); nlo = min(max(nlo - base, 0), STEPS);
+        nhi1 = min(max(nhi1 - base, 0), STEPS); whi1 = min(max(whi1 - base, 0), STEPS);
+    }
+    float2 s0 = make_float2(0.f, 0.f), s1 = make_float2(0.f, 0.f);
+    if (cf.fast) {
+        LaneK<NB> lk;
+        coop_consts<NB, NX>(lk, ct, cf, lane, pan);
+        // contiguous steps: the pointers run through the segments
+        StepPtrs sp{rt + b * T::RS, d + off0, w + off0, STORE ? model_out + off0 : nullptr,
+                    tmem + (uint32_t)((half * G::PANELS + pan) * STEPS * TM_STEP), 0.f};
+        int i = 0;
+        if (NX < 64) {
+            // 32-pixel stamps have no far field (set_cull is never called for them)
+            row_steps_fast<NB, NX, NY, STORE, PREP, 2, TM>(cf, lk, s0, s1, i, STEPS, sp);
+        } else {
+            row_steps_fast<NB, NX, NY, STORE, PREP, 0, TM>(cf, lk, s0, s1, i, wlo, sp);
+            row_steps_fast<NB, NX, NY, STORE, PREP, 1, TM>(cf, lk, s0, s1, i, nlo, sp);
+            row_steps_fast<NB, NX, NY, STORE, PREP, 2, TM>(cf, lk, s0, s1, i, nhi1, sp);
+            row_steps_fast<NB, NX, NY, STORE, PREP, 1, TM>(cf, lk, s0, s1, i, whi1, sp);
+            row_steps_fast<NB, NX, NY, STORE, PREP, 0, TM>(cf, lk, s0, s1, i, STEPS, sp);
+        }
+    } else {
+        float2 xd[K][2];   // column offsets of the lane's pixel pairs (0,1) and (2,3)
+        const float fa = (float)(pan * G::PW + 4 * a);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float2 nx0 = make_float2(-cf.x0[k], -cf.x0[k]);
+            xd[k][0] = __fadd2_rn(make_float2(fa, fa + 1.f), nx0);
+            xd[k][1] = __fadd2_rn(make_float2(fa + 2.f, fa + 3.f), nx0);
+        }
+#pragma unroll 1
+        for (int st = 0; st < STEPS; ++st) {
+            const int so = st * G::RG * NX;
+            StepPtrs sp{nullptr, d + off0 + so, w + off0 + so, STORE ? model_out + off0 + so : nullptr,
+                        TM == 1 ? tmem + (uint32_t)(st * 16) : 0u, (float)(half * TR + st * G::RG + 2 * b)};
+            int i = 0;
+            row_steps<NB, NX, NY, STORE, PREP, 1, (TM == 1 ? 1 : 0)>(cf, xd, s0, s1, i, 1, sp);
+        }
+    }
+    // at most 16 steps x 8 pixels over 4 accumulators
+    return (s0.x + s0.y) + (s1.x + s1.y);
+}
+
 // chi-square of one parameter vector over the stamp by ONE warp (a team member's share: team_chi2).
 // Builds the block and column tables in `scratch` (Scratch<NB, NX, NY>::FLOATS
 // floats of this warp's own shared memory) itself.  `exps` counts the component evaluations
@@ -996,81 +1106,27 @@ __device__ __forceinline__ double warp_chi2(const Coef<NB>& cf, float* __restric
                                             unsigned* exps = nullptr, uint32_t tmem = 0) {
     static_assert(TEAM == 1, "whole-warp passes only");
     using G = Geo<NX>;
-    using T = Tab<NB>;
     using R = Rows<NY, TEAM>;
-    constexpr int K = 2 * NB;
-    constexpr int TR = R::TR;
-    constexpr int STEPS = TR / G::RG;            // warp steps per table (per panel)
-    static_assert(TM == 0 || (TEAM == 1 && PREP), "the TMEM pixel store holds prepared stamps for whole-warp passes");
-    static_assert(TM != 1 || (R::HALVES == 1 && G::PANELS == 1), "both planes fit the 512 TMEM columns up to 64 x 64 pixels");
-    constexpr int TM_STEP = TM == 1 ? 16 : 8;     // TMEM columns per warp step
-    static_assert(TR % G::RG == 0, "unsupported stamp height");
-    static_assert(STEPS % TEAM == 0, "team size must divide the warp steps");
-    float* rt = scratch;
-    float* ct = scratch + Scratch<NB, NX, NY, TEAM>::TAB;
-    const int a = lane % G::GPR, b = lane / G::GPR;
     double acc = 0.0;
     if (exps) *exps += cf.nexp;
 #pragma unroll 1
     for (int half = 0; half < R::HALVES; ++half) {
-        if (cf.fast) build_row_table<NB, NX, TR, TEAM>(rt, cf, lane, half * TR, tw);
+        if (cf.fast) build_row_table<NB, NX, R::TR, TEAM>(scratch, cf, lane, half * R::TR, tw);
 #pragma unroll 1
-        for (int pan = 0; pan < G::PANELS; ++pan) {
-            const int off0 = (half * TR + 2 * b) * NX + pan * G::PW + 4 * a;   // the lane's block of warp step 0
-            // segments of this panel, clipped to the warp steps of this table:
-            //   [0,wlo) none, [wlo,nlo) wings, [nlo,nhi1) all, [nhi1,whi1) wings, [whi1,STEPS) none
-            const bool p1 = G::PANELS > 1 && pan > 0;   // (constant indices keep the coefficients in registers)
-            int wlo = p1 ? cf.seg[1][0] : cf.seg[0][0], nlo = p1 ? cf.seg[1][1] : cf.seg[0][1];
-            int nhi1 = p1 ? cf.seg[1][2] : cf.seg[0][2], whi1 = p1 ? cf.seg[1][3] : cf.seg[0][3];
-            if (R::HALVES > 1) {
-                const int base = half * STEPS;
-                wlo = min(max(wlo - base, 0), STEPS); nlo = min(max(nlo - base, 0), STEPS);
-                nhi1 = min(max(nhi1 - base, 0), STEPS); whi1 = min(max(whi1 - base, 0), STEPS);
-            }
-            float2 s0 = make_float2(0.f, 0.f), s1 = make_float2(0.f, 0.f);
-            if (cf.fast) {
-                LaneK<NB> lk;
-                coop_consts<NB, NX>(lk, ct, cf, lane, pan);
-                {
-                    // contiguous steps: the pointers run through the segments
-                    StepPtrs sp{rt + b * T::RS, d + off0, w + off0, STORE ? model_out + off0 : nullptr,
-                                tmem + (uint32_t)((half * G::PANELS + pan) * STEPS * TM_STEP), 0.f};
-                    int i = 0;
-                    if (NX < 64) {
-                        // 32-pixel stamps have no far field (set_cull is never called for them)
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 2, TM>(cf, lk, s0, s1, i, STEPS, sp);
-                    } else {
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 0, TM>(cf, lk, s0, s1, i, wlo, sp);
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 1, TM>(cf, lk, s0, s1, i, nlo, sp);
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 2, TM>(cf, lk, s0, s1, i, nhi1, sp);
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 1, TM>(cf, lk, s0, s1, i, whi1, sp);
-                        row_steps_fast<NB, NX, NY, STORE, PREP, 0, TM>(cf, lk, s0, s1, i, STEPS, sp);
-                    }
-                }
-            } else {
-                float2 xd[K][2];   // column offsets of the lane's pixel pairs (0,1) and (2,3)
-                const float fa = (float)(pan * G::PW + 4 * a);
-#pragma unroll
-                for (int k = 0; k < K; ++k) {
-                    const float2 nx0 = make_float2(-cf.x0[k], -cf.x0[k]);
-                    xd[k][0] = __fadd2_rn(make_float2(fa, fa + 1.f), nx0);
-                    xd[k][1] = __fadd2_rn(make_float2(fa + 2.f, fa + 3.f), nx0);
-                }
-#pragma unroll 1
-                for (int mth = 0; mth < STEPS / TEAM; ++mth) {
-                    const int st = mth * TEAM + tw;
-                    const int so = st * G::RG * NX;
-                    StepPtrs sp{nullptr, d + off0 + so, w + off0 + so, STORE ? model_out + off0 + so : nullptr,
-                                TM == 1 ? tmem + (uint32_t)(st * 16) : 0u, (float)(half * TR + st * G::RG + 2 * b)};
-                    int i = 0;
-                    row_steps<NB, NX, NY, STORE, PREP, 1, (TM == 1 ? 1 : 0)>(cf, xd, s0, s1, i, 1, sp);
-                }
-            }
-            // FP32 partial sums of one panel (at most 16 steps x 8 pixels over 4 accumulators) -> FP64
-            acc += (double)((s0.x + s0.y) + (s1.x + s1.y));
-        }
+        for (int pan = 0; pan < G::PANELS; ++pan)     // FP32 partial sums of one panel -> FP64
+            acc += (double)panel_chi2<NB, NX, NY, STORE, PREP, TM>(cf, scratch, d, w, model_out, lane, half, pan, tmem);
     }
     return warp_sum_f64(acc);
+}
+
+// One-table, one-panel stamps: this lane's partial of warp_chi2, unreduced.  The caller reduces
+// (warp_sum_f64, or warp_sum_f64_of on the 32 partials gathered in shared memory) and counts cf.nexp.
+template <int NB, int NX, int NY, int TM>
+__device__ __forceinline__ float lane_chi2(const Coef<NB>& cf, float* __restrict__ scratch, const float* __restrict__ d,
+                                           const float* __restrict__ w, int lane, uint32_t tmem) {
+    static_assert(Geo<NX>::PANELS == 1 && Rows<NY, 1>::HALVES == 1, "one table, one panel");
+    if (cf.fast) build_row_table<NB, NX, NY, 1>(scratch, cf, lane, 0, 0);
+    return panel_chi2<NB, NX, NY, false, true, TM>(cf, scratch, d, w, nullptr, lane, 0, 0, tmem);
 }
 
 // TEAM > 1: this warp's share of chi-square of one parameter vector (the caller adds the TEAM partials
