@@ -159,7 +159,8 @@ int64_t lapf_sampler_rows_for(const lapf_sampler* s, int64_t n_updates);
 /* Advance every walker by n_updates Gibbs updates (one proposed parameter each).
  *   chain_out  device [rows][n_walkers][P+1] double (P parameters then chi-square, the column
  *              order of <rank>_finalarray_mpi.csv, apf_step2.py:346-351), or NULL to record
- *              nothing; rows_cap = capacity in rows (must be >= lapf_sampler_rows_for). */
+ *              nothing; rows_cap = capacity in rows (must be >= lapf_sampler_rows_for).  In the
+ *              event formats below chain_out must also hold lapf_sampler_chain_bytes bytes. */
 int lapf_sampler_run(lapf_sampler* s, int64_t n_updates, void* chain_out, int64_t rows_cap,
                      void* stream);
 
@@ -170,10 +171,29 @@ int lapf_sampler_run(lapf_sampler* s, int64_t n_updates, void* chain_out, int64_
  *                         precision lost where it matters -- a chain stays within a few jump
  *                         widths of its start, so the float carries the difference to ~1e-7 of
  *                         itself (positions: 512.3 +- 0.003 would keep only 2e-5 as plain floats).
- * Replaces the text rows of apf_step2.py:346-360 for batches of 10^4 .. 10^6 walkers. */
+ * Replaces the text rows of apf_step2.py:346-360 for batches of 10^4 .. 10^6 walkers.
+ *
+ * Event formats (thin = 1 only: then a row differs from the one before it in at most one parameter
+ * and chi-square).  The values are doubles (LAPF_CHAIN_EVENTS_F64) or float differences from the
+ * starting point computed exactly as LAPF_CHAIN_F32_DELTA does (LAPF_CHAIN_EVENTS_F32_DELTA).  With
+ * e = 8 or 4 bytes per value, a run that records R rows of W walkers writes one contiguous buffer:
+ *   key     e * [W][P+1]   row 0 of this run, byte for byte what the dense format writes as row 0
+ *   codes   uint8 [R][W], padded with zeros to a multiple of 16 bytes: bits 0-4 = k, the parameter
+ *           drawn for the update of row r; bit 7 = that update was accepted
+ *   values  e * [R][W]     column k of row r after accept / reject (the old value when rejected)
+ *   chi     e * [R][W]     chi-square column of row r
+ * Row r is row r-1 with row[k] = value and row[P] = chi (row -1 = key).  Event 0 repeats the key on
+ * purpose: the codes are then a trace of every recorded update (with burn_in = 0 they count exactly
+ * the tries and accepts of lapf_sampler_state).  Every byte is written: equal runs, equal buffers. */
 #define LAPF_CHAIN_F64 0
 #define LAPF_CHAIN_F32_DELTA 1
+#define LAPF_CHAIN_EVENTS_F64 2
+#define LAPF_CHAIN_EVENTS_F32_DELTA 3
+/* LAPF_ERR_INVALID for an event format on a sampler with thin != 1 (lapf_sampler_run checks again). */
 int lapf_sampler_set_chain_format(lapf_sampler* s, int32_t format);
+/* Bytes the next lapf_sampler_run of n_updates writes to chain_out in the current format: dense
+ * formats rows * W * (P+1) * e, event formats the layout above (0 when the run records no row). */
+int64_t lapf_sampler_chain_bytes(const lapf_sampler* s, int64_t n_updates);
 /* The starting point of every walker and its chi-square: start_out device double [n_walkers][P+1]
  * (the reference point of LAPF_CHAIN_F32_DELTA rows and of the running moments). */
 int lapf_sampler_start(lapf_sampler* s, double* start_out, void* stream);

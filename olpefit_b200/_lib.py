@@ -47,6 +47,7 @@ SYMBOLS = {
     "lapf_sampler_rows_for": (C.c_int64, [C.c_void_p, C.c_int64]),
     "lapf_sampler_run": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     "lapf_sampler_set_chain_format": (C.c_int, [C.c_void_p, C.c_int32]),
+    "lapf_sampler_chain_bytes": (C.c_int64, [C.c_void_p, C.c_int64]),
     "lapf_sampler_start": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "lapf_sampler_sketch_enable": (C.c_int, [C.c_void_p, C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "lapf_sampler_sketch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -102,39 +102,134 @@ def write_acceptance(path, accepts, tries):
         fh.write(str(rate))
 
 
+# ----------------------------------------------------------------------------------------------
+# chain events (LAPF_CHAIN_EVENTS_*, include/lapf.h): the one place on the host that knows the layout
+# ----------------------------------------------------------------------------------------------
+EVENT_MAGIC = b"LAPFEVT1"
+EVENT_HEADER = 32         # magic, rows (int64), walkers (int64), columns (int32), bytes per value (int32)
+
+
+def _event_parts(rows, n_walkers, n_cols, itemsize):
+    """Byte offsets of (codes, values, chi-square) and the total size of an event buffer."""
+    codes = itemsize * n_walkers * n_cols
+    values = codes + (rows * n_walkers + 15) // 16 * 16
+    chi = values + itemsize * rows * n_walkers
+    return codes, values, chi, chi + itemsize * rows * n_walkers
+
+
+def event_bytes(rows, n_walkers, n_cols, dtype):
+    """Size of the event buffer of ``rows`` rows (0 rows: nothing, not even the key)."""
+    return _event_parts(rows, n_walkers, n_cols, np.dtype(dtype).itemsize)[3] if rows else 0
+
+
+def decode_events(buf, rows, n_walkers, n_cols, dtype):
+    """The dense chain rows [rows, n_walkers, n_cols] of one event buffer (a uint8 array as
+    ``lapf_sampler_run`` wrote it in an event format): float64 values, or float32 differences
+    from the starting point -- bit for bit what the dense format of that precision writes.
+    Row r is row r-1 with column k replaced by the event's value and the last column by its
+    chi-square; vectorised over rows: per column, the last event at or before each row."""
+    dt = np.dtype(dtype)
+    W, C, R = int(n_walkers), int(n_cols), int(rows)
+    if R == 0:
+        return np.empty((0, W, C), dtype=dt)
+    buf = np.asarray(buf, dtype=np.uint8).reshape(-1)
+    o_code, o_val, o_chi, end = _event_parts(R, W, C, dt.itemsize)
+    if buf.size < end:
+        raise ValueError("event buffer of %d bytes is shorter than the %d of %d rows x %d walkers" % (buf.size, end, R, W))
+    key = buf[:o_code].view(dt).reshape(W, C)
+    k = (buf[o_code:o_code + R * W] & 31).reshape(R, W)
+    values = buf[o_val:o_chi].view(dt).reshape(R, W)
+    out = np.empty((R, W, C), dtype=dt)
+    out[:, :, C - 1] = buf[o_chi:end].view(dt).reshape(R, W)
+    rix = np.arange(1, R + 1, dtype=np.int32)[:, None]
+    # blocks of walkers keep each column's gather inside the cache (3x faster at 65,536 walkers)
+    for w0 in range(0, W, 256):
+        n = min(W, w0 + 256) - w0
+        kb, ob = k[:, w0:w0 + n], out[:, w0:w0 + n]
+        src = np.empty((R + 1, n), dtype=dt)        # row 0: the key, row 1 + r: the values of event r
+        src[1:] = values[:, w0:w0 + n]
+        flat, cols = src.reshape(-1), np.arange(n, dtype=np.int32)[None, :]
+        for c in range(C - 1):
+            src[0] = key[w0:w0 + n, c]
+            last = np.maximum.accumulate(np.where(kb == c, rix, 0), axis=0)   # 0: no event of column c yet
+            ob[:, :, c] = flat[last * n + cols]
+    return out
+
+
+def _event_segments(path):
+    """[(offset of the payload, rows, walkers, columns, bytes per value)] of the complete segments of
+    an event file, and the byte size they cover (a torn last segment is not included)."""
+    segs, pos = [], 0
+    size = os.path.getsize(path)
+    with open(path, "rb") as fh:
+        while pos + EVENT_HEADER <= size:
+            fh.seek(pos)
+            head = fh.read(EVENT_HEADER)
+            if head[:8] != EVENT_MAGIC:
+                raise ValueError("%s: no event segment at byte %d" % (path, pos))
+            rows, walkers = (int(v) for v in np.frombuffer(head, dtype="<i8", count=2, offset=8))
+            cols, item = (int(v) for v in np.frombuffer(head, dtype="<i4", count=2, offset=24))
+            end = pos + EVENT_HEADER + _event_parts(rows, walkers, cols, item)[3]
+            if end > size:
+                break
+            segs.append((pos + EVENT_HEADER, rows, walkers, cols, item))
+            pos = end
+    return segs, pos
+
+
 class PackedChainWriter:
     """Packed binary chain: [row][walker][P+1] appended segment by segment to ``<base>.bin`` with a
     JSON sidecar ``<base>.json``; for batches of 10^4..10^6 walkers where one text file per walker
     is not workable.  dtype 'float64' holds the values; 'float32' holds differences from the
     walkers' starting points, which are stored once as float64 in ``<base>.start.bin``
     (LAPF_CHAIN_F32_DELTA).  ``resume=True`` appends to an existing file of the same shape (the
-    sidecar tells the row count so far).  ``read_packed`` / ``unpack_to_csv`` convert back."""
+    sidecar tells the row count so far).  ``read_packed`` / ``unpack_to_csv`` convert back.
 
-    def __init__(self, base, n_walkers, n_cols, meta=None, dtype="float64", start=None, resume=False):
+    ``events=True`` stores the event buffers of an event chain format instead (thin = 1; about a
+    seventh of the bytes) in ``<base>.events``, one self-describing segment per ``append_events``:
+    a 32-byte header (magic LAPFEVT1, rows, walkers, columns, bytes per value) and the buffer as the
+    device wrote it.  Resuming walks the headers and drops a torn last segment."""
+
+    def __init__(self, base, n_walkers, n_cols, meta=None, dtype="float64", start=None, resume=False, events=False):
         self.base, self.n_walkers, self.n_cols = base, int(n_walkers), int(n_cols)
         self.dtype = np.dtype(dtype)
         if self.dtype not in (np.dtype("float64"), np.dtype("float32")):
             raise ValueError("packed chains are float64 or float32 (differences from the start)")
+        self.events = bool(events)
+        self.path = base + (".events" if self.events else ".bin")
         self.rows = 0
         self.meta = dict(meta or {})
         if resume:
             with open(base + ".json") as fh:
                 old = json.load(fh)
-            if (old["n_walkers"], old["n_cols"], old["dtype"]) != (self.n_walkers, self.n_cols, self.dtype.name):
-                raise ValueError("%s.bin holds %s walkers x %s columns of %s: cannot append %d x %d of %s"
-                                 % (base, old["n_walkers"], old["n_cols"], old["dtype"], self.n_walkers,
-                                    self.n_cols, self.dtype.name))
-            have = os.path.getsize(base + ".bin")
-            want = old["rows"] * self.n_walkers * self.n_cols * self.dtype.itemsize
-            if have < want:
-                raise ValueError("%s.bin is shorter than its sidecar says" % base)
-            self.rows = int(old["rows"])
+            if (old["n_walkers"], old["n_cols"], old["dtype"], old.get("format", "rows")) != (
+                    self.n_walkers, self.n_cols, self.dtype.name, "events" if self.events else "rows"):
+                raise ValueError("%s holds %s walkers x %s columns of %s (%s): cannot append %d x %d of %s"
+                                 % (base, old["n_walkers"], old["n_cols"], old["dtype"], old.get("format", "rows"),
+                                    self.n_walkers, self.n_cols, self.dtype.name))
+            if self.events:
+                # keep the complete segments the sidecar counts; a torn or uncounted tail is dropped
+                segs, _ = _event_segments(self.path)
+                want = 0
+                for off, rows, _, _, item in segs:
+                    if self.rows + rows > old["rows"]:
+                        break
+                    self.rows += rows
+                    want = off + _event_parts(rows, self.n_walkers, self.n_cols, item)[3]
+                if self.rows != old["rows"]:
+                    raise ValueError("%s holds fewer rows than its sidecar says" % self.path)
+            else:
+                have = os.path.getsize(self.path)
+                want = old["rows"] * self.n_walkers * self.n_cols * self.dtype.itemsize
+                if have < want:
+                    raise ValueError("%s.bin is shorter than its sidecar says" % base)
+                self.rows = int(old["rows"])
             self.meta = {**old, **self.meta}
-            self.fh = open(base + ".bin", "r+b")
+            self.fh = open(self.path, "r+b")
             self.fh.truncate(want)                      # drop a partial segment of an interrupted run
             self.fh.seek(want)
         else:
-            self.fh = open(base + ".bin", "wb")
+            self.fh = open(self.path, "wb")
             if self.dtype == np.dtype("float32"):
                 if start is None:
                     raise ValueError("float32 chains are differences: the starting points are needed")
@@ -143,16 +238,35 @@ class PackedChainWriter:
                 st.tofile(base + ".start.bin")
 
     def append(self, segment):
+        if self.events:
+            raise ValueError("an event file takes event buffers (append_events)")
         seg = np.ascontiguousarray(segment, dtype=self.dtype)
         assert seg.shape[1:] == (self.n_walkers, self.n_cols)
         self.fh.write(seg.tobytes())
         self.rows += seg.shape[0]
+
+    def append_events(self, payload, rows):
+        """One event buffer of ``rows`` rows, as ``GibbsSampler.run`` / ``ChainStreamer`` return it."""
+        if not self.events:
+            raise ValueError("a row file takes rows (append)")
+        payload = np.asarray(payload, dtype=np.uint8).reshape(-1)
+        n = event_bytes(rows, self.n_walkers, self.n_cols, self.dtype)
+        if rows == 0:
+            return
+        if payload.size < n:
+            raise ValueError("event buffer of %d bytes, %d rows need %d" % (payload.size, rows, n))
+        head = EVENT_MAGIC + np.array([rows, self.n_walkers], dtype="<i8").tobytes() + \
+            np.array([self.n_cols, self.dtype.itemsize], dtype="<i4").tobytes()
+        self.fh.write(head)
+        self.fh.write(payload[:n].tobytes())
+        self.rows += int(rows)
 
     def close(self, **extra):
         self.fh.close()
         self.meta.update(extra)
         self.meta.update({"rows": self.rows, "n_walkers": self.n_walkers, "n_cols": self.n_cols,
                           "dtype": self.dtype.name, "order": "[row][walker][column]",
+                          "format": "events" if self.events else "rows",
                           "values": "differences from <base>.start.bin" if self.dtype == np.dtype("float32") else "absolute"})
         with open(self.base + ".json", "w") as fh:
             json.dump(self.meta, fh, indent=1)
@@ -164,7 +278,19 @@ def read_packed(base):
         meta = json.load(fh)
     shape = (meta["rows"], meta["n_walkers"], meta["n_cols"])
     dt = np.dtype(meta.get("dtype", "float64"))
-    arr = np.fromfile(base + ".bin", dtype=dt, count=int(np.prod(shape))).reshape(shape)
+    if meta.get("format", "rows") == "events":
+        raw = np.memmap(base + ".events", dtype=np.uint8, mode="r")
+        parts, have = [], 0
+        for off, rows, walkers, cols, _ in _event_segments(base + ".events")[0]:
+            if have + rows > shape[0]:
+                break
+            parts.append(decode_events(raw[off:], rows, walkers, cols, dt))
+            have += rows
+        if have != shape[0]:
+            raise ValueError("%s.events holds fewer rows than its sidecar says" % base)
+        arr = np.concatenate(parts, axis=0) if parts else np.empty(shape, dtype=dt)
+    else:
+        arr = np.fromfile(base + ".bin", dtype=dt, count=int(np.prod(shape))).reshape(shape)
     if dt == np.dtype("float32"):
         start = np.fromfile(base + ".start.bin", dtype=np.float64).reshape(shape[1:])
         arr = start[None] + arr.astype(np.float64)

@@ -57,9 +57,12 @@ def _parser(kind):
     ap.add_argument("--segment", type=int, default=4096, help="updates per kernel launch")
     ap.add_argument("--team", type=int, default=0, choices=[0, 1, 4, 16],
                     help="warps cooperating on one walker (0: pick from the total walker count)")
-    ap.add_argument("--format", choices=["csv", "bin"], default="csv", help="per-walker reference CSV files, or one packed binary")
+    ap.add_argument("--format", choices=["csv", "bin", "events"], default="csv",
+                    help="per-walker reference CSV files, one packed binary, or (--thin 1 only) one packed file of "
+                         "chain events: per update the parameter that was drawn, its value and chi-square, about a "
+                         "seventh of the bytes of the rows; chains.read_packed / unpack_to_csv rebuild the rows")
     ap.add_argument("--chain-dtype", choices=["f64", "f32"], default="f64",
-                    help="--format bin only: f32 stores float32 differences from each walker's starting point "
+                    help="--format bin / events only: f32 stores float32 differences from each walker's starting point "
                          "(half the bytes off the device and on disk; chains.read_packed restores the values)")
     ap.add_argument("--no-chains", action="store_true",
                     help="record no chain rows at all: only the acceptance files and step2_summary.json (statistics "
@@ -94,6 +97,8 @@ def _frame_list(args):
 
 def run(kind, nbody, argv=None):
     args = _parser(kind).parse_args(argv)
+    if args.format == "events" and args.thin != 1:
+        raise SystemExit("--format events needs --thin 1: rows further apart differ in more than one parameter")
     import torch
     from . import chains, dist, frame, layout, sampler as smp, stats
 
@@ -192,18 +197,24 @@ def run(kind, nbody, argv=None):
         sam.enable_sketch(centers=centers)
 
     record = not args.no_chains
+    f32 = args.format != "csv" and args.chain_dtype == "f32"
+    # At --thin 1 consecutive rows differ in one parameter and chi-square: the rows leave the device as
+    # events (a seventh of the bytes) and are rebuilt bit for bit on the host before the writers below.
+    events = record and args.thin == 1
+    if events:
+        sam.set_chain_format("events_f32delta" if f32 else "events_f64")
+    elif f32 and record:
+        sam.set_chain_format("f32delta")
     packed = None
-    if args.format == "bin" and record:
-        if args.chain_dtype == "f32":
-            sam.set_chain_format("f32delta")
+    if args.format != "csv" and record:
         packed = chains.PackedChainWriter(
             outdirs[0] + "chains_rank%d" % rank, max(n_local, 1), P + 1,
             {"walker_ids": ids.tolist(), "walkers_per_frame": per_frame, "frames": images, "seed": seed,
              "id_layout": "walker_id = walker * n_frames + frame",
              "burn_in": burn_in, "thin": args.thin, "nbody": nbody, "origin": [int(v) for v in cuts[0]],
              "cuts": cuts.tolist(), "stamp": args.stamp},
-            dtype="float32" if args.chain_dtype == "f32" else "float64",
-            start=sam.start().cpu().numpy() if args.chain_dtype == "f32" else None, resume=args.resume)
+            dtype="float32" if f32 else "float64",
+            start=sam.start().cpu().numpy() if f32 else None, resume=args.resume, events=args.format == "events")
 
     streamer = smp.ChainStreamer(sam, args.segment) if record else None
     first = [True]
@@ -221,10 +232,15 @@ def run(kind, nbody, argv=None):
     def consume(seg):
         if seg is None or n_local == 0:
             return
-        if packed is not None:
-            packed.append(seg)
+        if args.format == "events":
+            packed.append_events(*seg)
         else:
-            chains.write_segment_csv(paths, seg, first[0])
+            if events:
+                seg = chains.decode_events(*seg, sam.n_walkers, P + 1, np.float32 if f32 else np.float64)
+            if packed is not None:
+                packed.append(seg)
+            else:
+                chains.write_segment_csv(paths, seg, first[0])
         first[0] = False
 
     def advance(n):

@@ -316,12 +316,18 @@ struct RunArgs {
     uint32_t* accepts;           // [W][P]
     unsigned long long* exps;    // [W] exponentials actually evaluated (after far-field culling)
     void* chain;                 // [rows][W][P+1] double, or float (value - shift) when chain_f32; or nullptr
+                                 // (chain_ev: row 0 only, the key of the event buffer)
+    // event formats (chain_ev): per recorded row and walker one code byte (k | accepted << 7), the value of
+    // column k and chi-square, as double or as float (value - shift) like the rows; parts of the chain buffer
+    unsigned char* ev_code;      // [rows][W]
+    void* ev_val;                // [rows][W]
+    void* ev_chi;                // [rows][W]
     // separation / position-angle sketches of the recorded rows (apf_step3.py:255-256,283-291), or nullptr
     uint32_t* sk_hist;           // [F][NB-1][2][sk_bins + 2]: underflow, bins, overflow
     const double* sk_center;     // [F][NB-1][2]: separation (pixels), position angle (degrees) of bin sk_bins / 2
     double* sk_mom;              // [W][NB-1][2][2]: per walker sum / sum of squares of (value - centre)
     double sk_inv_sep, sk_inv_pa;   // 1 / bin width
-    int sk_bins, chain_f32;
+    int sk_bins, chain_f32, chain_ev;
     double* probe;               // self-test only: [rows][W][3] = parameter index, proposed value, TRIAL chi-square
     unsigned long long* cta_times;   // diagnosis only (LAPF_CTA_TIMES): [CTAs][3] = start, end (globaltimer ns), SM id
     int64_t n_walkers;
@@ -499,9 +505,15 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
                 const size_t mi = (size_t)wl * (P + 1) + lane;
                 const double v = (lane == P) ? chi_c : p;
                 const double dl = v - a.shift[mi];
-                if (a.chain) {
+                if (a.chain && (row == 0 || !a.chain_ev)) {           // events: row 0 is the key
                     const size_t ci = ((size_t)row * a.n_walkers + wl) * (P + 1) + lane;
                     if (a.chain_f32) static_cast<float*>(a.chain)[ci] = (float)dl; else static_cast<double*>(a.chain)[ci] = v;
+                }
+                if (a.chain_ev && (lane == k || lane == P)) {            // the lanes that hold column k and chi-square
+                    const size_t ei = (size_t)row * a.n_walkers + wl;
+                    if (lane == k) a.ev_code[ei] = (unsigned char)(k | (acc ? 0x80 : 0));
+                    void* dst = (lane == k) ? a.ev_val : a.ev_chi;
+                    if (a.chain_f32) static_cast<float*>(dst)[ei] = (float)dl; else static_cast<double*>(dst)[ei] = v;
                 }
                 atomicAdd(&a.moments[2 * mi], dl);                    // single writer: plain RED, in order
                 atomicAdd(&a.moments[2 * mi + 1], dl * dl);
@@ -728,15 +740,28 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
                 st[k] = nv;                                               // :325
                 chi_c = chi_t;                                            // :327
             }
+            if (a.chain_ev && u == next_rec) {                            // the event of this row
+                const size_t ei = (size_t)row * a.n_walkers + wl, si = (size_t)wl * (P + 1);
+                a.ev_code[ei] = (unsigned char)(k | (acc ? 0x80 : 0));
+                const double kv = st[k];
+                if (a.chain_f32) {
+                    static_cast<float*>(a.ev_val)[ei] = (float)(kv - a.shift[si + k]);
+                    static_cast<float*>(a.ev_chi)[ei] = (float)(chi_c - a.shift[si + P]);
+                } else {
+                    static_cast<double*>(a.ev_val)[ei] = kv;
+                    static_cast<double*>(a.ev_chi)[ei] = chi_c;
+                }
+            }
         }
         if (u == next_rec) {                                              // :342-351
             if (mine) {
+                const bool dense = a.chain && (row == 0 || !a.chain_ev);   // events: row 0 is the key
 #pragma unroll 1
                 for (int j = 0; j <= P; ++j) {
                     const size_t mi = (size_t)wl * (P + 1) + j;
                     const double v = (j == P) ? chi_c : st[j];
                     const double dl = v - a.shift[mi];
-                    if (a.chain) {
+                    if (dense) {
                         const size_t ci = ((size_t)row * a.n_walkers + wl) * (P + 1) + j;
                         if (a.chain_f32) static_cast<float*>(a.chain)[ci] = (float)dl; else static_cast<double*>(a.chain)[ci] = v;
                     }
@@ -1755,6 +1780,23 @@ int64_t lapf_sampler_rows_for(const lapf_sampler* s, int64_t n_updates) {
            rows_upto(s->count, s->cfg.burn_in, s->cfg.thin);
 }
 
+static bool is_event_format(int format) { return format == LAPF_CHAIN_EVENTS_F64 || format == LAPF_CHAIN_EVENTS_F32_DELTA; }
+static bool is_f32_format(int format) { return format == LAPF_CHAIN_F32_DELTA || format == LAPF_CHAIN_EVENTS_F32_DELTA; }
+static int64_t event_codes_bytes(int64_t rows, int64_t W) { return (rows * W + 15) & ~(int64_t)15; }
+
+// Bytes a run that records `rows` rows writes in the current format (include/lapf.h: the event layout).
+static int64_t chain_bytes_for_rows(const lapf_sampler* s, int64_t rows) {
+    const int64_t W = s->cfg.n_walkers, e = is_f32_format(s->chain_format) ? 4 : 8;
+    if (!is_event_format(s->chain_format)) return rows * W * (s->P + 1) * e;
+    if (rows == 0) return 0;
+    return e * W * (s->P + 1) + event_codes_bytes(rows, W) + 2 * e * rows * W;
+}
+
+int64_t lapf_sampler_chain_bytes(const lapf_sampler* s, int64_t n_updates) {
+    const int64_t rows = lapf_sampler_rows_for(s, n_updates);
+    return rows < 0 ? rows : chain_bytes_for_rows(s, rows);
+}
+
 int64_t lapf_sampler_count(const lapf_sampler* s) { return s ? s->count : fail(LAPF_ERR_INVALID, "sampler is NULL"); }
 int64_t lapf_sampler_launches(const lapf_sampler* s) { return s ? s->launches : fail(LAPF_ERR_INVALID, "sampler is NULL"); }
 
@@ -1767,7 +1809,15 @@ static void fill_run_args(const lapf_sampler* s, RunArgs& a, int64_t n_updates, 
     a.state = s->state; a.shift = s->shift; a.moments = s->moments;
     a.tries = s->tries; a.accepts = s->accepts; a.exps = s->exps;
     a.chain = chain_out;
-    a.chain_f32 = s->chain_format == LAPF_CHAIN_F32_DELTA ? 1 : 0;
+    a.chain_f32 = is_f32_format(s->chain_format) ? 1 : 0;
+    a.chain_ev = (chain_out && is_event_format(s->chain_format)) ? 1 : 0;
+    a.ev_code = nullptr; a.ev_val = nullptr; a.ev_chi = nullptr;
+    if (a.chain_ev) {
+        const int64_t rows = lapf_sampler_rows_for(s, n_updates), W = s->cfg.n_walkers, e = a.chain_f32 ? 4 : 8;
+        a.ev_code = static_cast<unsigned char*>(chain_out) + e * W * (s->P + 1);
+        a.ev_val = a.ev_code + event_codes_bytes(rows, W);
+        a.ev_chi = static_cast<unsigned char*>(a.ev_val) + e * rows * W;
+    }
     a.sk_hist = s->sk_hist; a.sk_center = s->sk_center; a.sk_mom = s->sk_mom;
     a.sk_bins = s->sk_bins;
     a.sk_inv_sep = s->sk_bins ? 1.0 / s->sk_sep_bin : 0.0;
@@ -1791,11 +1841,18 @@ int lapf_sampler_run(lapf_sampler* s, int64_t n_updates, void* chain_out, int64_
     if (n_updates < 0 || n_updates > ((int64_t)1 << 30))
         return fail(LAPF_ERR_INVALID, "n_updates must be in [0, 2^30] per launch");
     if (n_updates == 0) return LAPF_OK;
+    if (is_event_format(s->chain_format) && s->cfg.thin != 1)
+        return fail(LAPF_ERR_INVALID, "event chain formats need thin = 1 (thin is %d)", s->cfg.thin);
     const int64_t rows = lapf_sampler_rows_for(s, n_updates);
     if (chain_out && rows_cap < rows)
         return fail(LAPF_ERR_INVALID, "chain_out holds %lld rows but this run records %lld", (long long)rows_cap, (long long)rows);
     RunArgs a;
     fill_run_args(s, a, n_updates, chain_out);
+    if (a.chain_ev && rows > 0) {
+        // the padding of the codes: every byte of the buffer is written, so equal runs give equal buffers
+        const int64_t n_codes = rows * s->cfg.n_walkers, pad = event_codes_bytes(rows, s->cfg.n_walkers) - n_codes;
+        if (pad) CU(cudaMemsetAsync(a.ev_code + n_codes, 0, (size_t)pad, (cudaStream_t)stream));
+    }
     // diagnosis (LAPF_CTA_TIMES=<file>): start, end and SM of every CTA of the batched kernel, one text line per launch
     const char* times_path = s->team == 1 ? getenv("LAPF_CTA_TIMES") : nullptr;
     if (times_path) CU(cudaMalloc((void**)&a.cta_times, sizeof(unsigned long long) * 3 * s->launch_grid));
@@ -1901,6 +1958,8 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     a.thin = 1;
     a.next_record = a.t0 + 1;
     a.chain_f32 = 0;
+    a.chain_ev = 0;
+    a.ev_code = nullptr; a.ev_val = nullptr; a.ev_chi = nullptr;
     a.sk_hist = nullptr;
     a.probe = probe;
     rc = launch_dispatch(s, a, st);
@@ -1948,8 +2007,11 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
 
 int lapf_sampler_set_chain_format(lapf_sampler* s, int32_t format) {
     if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
-    if (format != LAPF_CHAIN_F64 && format != LAPF_CHAIN_F32_DELTA)
+    if (format != LAPF_CHAIN_F64 && format != LAPF_CHAIN_F32_DELTA && !is_event_format(format))
         return fail(LAPF_ERR_INVALID, "unknown chain format %d", format);
+    if (is_event_format(format) && s->cfg.thin != 1)
+        return fail(LAPF_ERR_INVALID, "event chain formats need thin = 1 (thin is %d): rows further apart differ in more "
+                    "than one parameter", s->cfg.thin);
     s->chain_format = format;
     return LAPF_OK;
 }

@@ -45,6 +45,7 @@ class GibbsSampler:
                           p.data_ptr(), w_arr, int(burn_in), int(thin), int(team_warps))
         self.burn_in, self.thin = int(burn_in), int(thin)
         self.chain_dtype = torch.float64
+        self.events = False
         self._sketch = None
         handle = C.c_void_p()
         _lib.check(self.lib.lapf_sampler_create(C.byref(cfg), C.byref(handle), _stream_ptr(dev)))
@@ -105,10 +106,14 @@ class GibbsSampler:
     def set_chain_format(self, fmt: str):
         """'f64': rows are the values themselves (default).  'f32delta': rows are float32 differences
         from the walker's starting point (``start()``) -- half the bytes to drain, and exact to ~1e-7
-        of the distance travelled (see include/lapf.h)."""
-        code = {"f64": 0, "f32delta": 1}[fmt]
+        of the distance travelled (see include/lapf.h).  'events_f64' / 'events_f32delta' (thin = 1
+        only): each run writes the rows of the dense format of that precision as one changed parameter
+        and chi-square per row and walker; ``run`` returns that buffer and
+        ``chains.decode_events`` rebuilds the rows."""
+        code = {"f64": 0, "f32delta": 1, "events_f64": 2, "events_f32delta": 3}[fmt]
         _lib.check(self.lib.lapf_sampler_set_chain_format(self._h, code))
-        self.chain_dtype = torch.float32 if code else torch.float64
+        self.chain_dtype = torch.float32 if code in (1, 3) else torch.float64
+        self.events = code >= 2
 
     def start(self):
         """[W, P+1] float64 device tensor: every walker's starting point and its chi-square."""
@@ -156,11 +161,18 @@ class GibbsSampler:
     def rows_for(self, n_updates: int) -> int:
         return int(_lib.check(self.lib.lapf_sampler_rows_for(self._h, int(n_updates))))
 
+    def chain_bytes(self, n_updates: int) -> int:
+        """Bytes the next ``run(n_updates)`` records in the current chain format."""
+        return int(_lib.check(self.lib.lapf_sampler_chain_bytes(self._h, int(n_updates))))
+
     def run(self, n_updates: int, record=True, out=None):
         """Advance all walkers by ``n_updates`` updates.  Returns the chain rows recorded by this
         call as a device tensor [rows, n_walkers, P+1] (float64, or float32 differences from
-        ``start()`` after ``set_chain_format('f32delta')``; None when record is False)."""
+        ``start()`` after ``set_chain_format('f32delta')``; None when record is False).  In an event
+        format: (device uint8 tensor of ``chain_bytes(n_updates)`` bytes, rows)."""
         rows = self.rows_for(n_updates)
+        if self.events:
+            return self._run_events(n_updates, rows, record, out)
         chain = None
         if record:
             if out is not None:
@@ -177,6 +189,20 @@ class GibbsSampler:
             return chain.reshape(-1)[: rows * self.n_walkers * (self.nparam + 1)].view(
                 rows, self.n_walkers, self.nparam + 1)
         return chain
+
+    def _run_events(self, n_updates, rows, record, out):
+        nbytes = self.chain_bytes(n_updates)
+        buf = None
+        if record:
+            if out is not None:
+                if out.dtype != torch.uint8 or out.numel() < nbytes:
+                    raise ValueError("out must be uint8 and hold %d bytes" % nbytes)
+                buf = out.reshape(-1)[:nbytes]
+            else:
+                buf = torch.empty(nbytes, dtype=torch.uint8, device=self.domain.device)
+        _lib.check(self.lib.lapf_sampler_run(self._h, int(n_updates), buf.data_ptr() if buf is not None and rows > 0 else None,
+                                             rows, _stream_ptr(self.domain.device)))
+        return None if buf is None else (buf, rows)
 
     def state(self):
         """(state [W, P+1], tries [W, P], accepts [W, P]) device tensors: parameters + chi-square,
@@ -214,28 +240,40 @@ class ChainStreamer:
         streamer = ChainStreamer(sampler, max_updates_per_segment)
         seg = streamer.run(n)      # launches n updates; returns the PREVIOUS segment (numpy) or None
         seg = streamer.finish()    # the last segment
+
+    A segment is the rows [rows, W, P+1] of the sampler's chain format, or in an event format the
+    tuple (uint8 event buffer, rows) for ``chains.decode_events``.  Buffers are sized in bytes
+    (``GibbsSampler.chain_bytes``) and grow if a later segment needs more.
     """
 
     def __init__(self, sampler: GibbsSampler, max_updates: int):
         self.s = sampler
-        dev = sampler.domain.device
-        cap_rows = max(1, -(-int(max_updates) // sampler.thin) + 1)
-        shape = (cap_rows, sampler.n_walkers, sampler.nparam + 1)
-        self.dev = [torch.empty(shape, dtype=sampler.chain_dtype, device=dev) for _ in range(2)]
-        self.host = [torch.empty(shape, dtype=sampler.chain_dtype).pin_memory() for _ in range(2)]
-        self.copy_stream = torch.cuda.Stream(device=dev)
-        self.done = [torch.cuda.Event(), torch.cuda.Event()]
-        self.pending = None          # (buffer index, rows)
-        self.i = 0
         self.max_updates = int(max_updates)
+        cap = max(16, sampler.chain_bytes(self.max_updates))
+        self.dev = [self._device_buffer(cap) for _ in range(2)]
+        self.host = [self._host_buffer(cap) for _ in range(2)]
+        self.copy_stream = torch.cuda.Stream(device=sampler.domain.device)
+        self.done = [torch.cuda.Event(), torch.cuda.Event()]
+        self.pending = None          # (buffer index, rows, bytes)
+        self.i = 0
+
+    def _device_buffer(self, nbytes):
+        return torch.empty(-(-nbytes // 8) * 8, dtype=torch.uint8, device=self.s.domain.device)
+
+    def _host_buffer(self, nbytes):
+        return torch.empty(-(-nbytes // 8) * 8, dtype=torch.uint8).pin_memory()
 
     def _collect(self):
         if self.pending is None:
             return None
-        j, rows = self.pending
+        j, rows, nbytes = self.pending
         self.pending = None
         self.done[j].synchronize()
-        return self.host[j][:rows].numpy()
+        raw = self.host[j][:nbytes].numpy()
+        if self.s.events:
+            return raw, rows
+        dt = np.float32 if self.s.chain_dtype == torch.float32 else np.float64
+        return raw.view(dt).reshape(rows, self.s.n_walkers, self.s.nparam + 1)
 
     def run(self, n_updates: int):
         if n_updates > self.max_updates:
@@ -243,15 +281,19 @@ class ChainStreamer:
         s, i = self.s, self.i
         compute = torch.cuda.current_stream(s.domain.device)
         compute.wait_event(self.done[i])            # the copy out of dev[i] two segments ago is finished
-        chain = s.run(n_updates, out=self.dev[i])
-        rows = int(chain.shape[0])
-        if rows:
-            nbytes = rows * s.n_walkers * (s.nparam + 1) * self.dev[i].element_size()
+        nbytes = s.chain_bytes(n_updates)
+        if nbytes > self.dev[i].numel():            # host[i] was collected by the previous call
+            self.dev[i], self.host[i] = self._device_buffer(nbytes), self._host_buffer(nbytes)
+        if s.events:
+            _, rows = s.run(n_updates, out=self.dev[i])
+        else:
+            rows = int(s.run(n_updates, out=self.dev[i].view(s.chain_dtype)).shape[0])
+        if nbytes:
             _lib.check(s.lib.lapf_chain_drain(self.dev[i].data_ptr(), self.host[i].data_ptr(), nbytes,
                                               compute.cuda_stream, self.copy_stream.cuda_stream))
         self.done[i].record(self.copy_stream)
         prev = self._collect()                      # overlaps with the segment just launched
-        self.pending = (i, rows)
+        self.pending = (i, rows, nbytes)
         self.i = 1 - i
         return prev
 
