@@ -235,6 +235,32 @@ int lapf_sampler_sketch_enable(lapf_sampler* s, int32_t n_bins, double sep_bin_p
  *                (value - centre)^2, number of values (position-angle differences wrapped to +-180) */
 int lapf_sampler_sketch(lapf_sampler* s, uint32_t* hist_out, double* summary_out, void* stream);
 
+/* K4c -- batch means of the recorded rows without the chain: the ingredients of a Monte Carlo standard
+ * error and an effective sample size for every walker (DESIGN.md, "Batch means").  Quantity c < P+1 is
+ * chain column c minus the walker's starting point (what the running moments add up); if sketches were
+ * enabled before, quantities P+1 + 2(o-1) + q follow, the separation (q = 0) and position angle (q = 1)
+ * of companion o minus the frame's sketch centre, exactly as the sketch sums add them: C quantities.
+ * Every walker keeps, per quantity and level l < levels, two doubles: snap, its running sum M1 at the
+ * last row count that is a multiple of b_l = batch_rows * 2^l (the sum of its complete level-l batches),
+ * and s2, the sum of the squared sums of those batches.  A row that brings the walker's recorded-row
+ * count to a multiple of b_l does S = M1 - snap; s2 = s2 + S*S; snap = M1 (rounded to nearest, never
+ * fused); rows that close no batch cost nothing more.  The state depends neither on how runs are split
+ * into launches nor on the chain format.
+ * Batch means of every recorded value at batch lengths batch_rows * 2^l rows, l < levels
+ * (1 <= batch_rows <= 2^30, 1 <= levels <= 24).  LAPF_ERR_INVALID once any row has been recorded.  Runs
+ * lapf_sampler_selftest with the batch means active (unless LAPF_NO_SELFTEST) and leaves the sampler as
+ * it was.  Once they are on, lapf_sampler_sketch_enable returns LAPF_ERR_INVALID (C would change);
+ * lapf_sampler_reset zeroes them; checkpoints carry them after the sketch sections, behind a 32-byte
+ * descriptor (int64 magic, batch_rows, levels, C) that lapf_sampler_load checks against the sampler. */
+int lapf_sampler_batchmeans_enable(lapf_sampler* s, int32_t batch_rows, int32_t levels, void* stream);
+/*   walker_out device double [W][C][levels][2] (snap, s2) or NULL
+ *   frame_out  device double [F][C][1 + levels] or NULL: [0] sum over the frame's walkers of the
+ *              population variance of their recorded values (np.std()**2), [1+l] sum over the frame's
+ *              walkers of the sample variance of their level-l batch means, each
+ *              (s2 - snap^2 / J) / (b_l^2 (J - 1)) with J = rows / b_l complete batches (0 where J < 2).
+ *              Sums over walkers: all-reduce them over GPUs like the moments. */
+int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_out, void* stream);
+
 /* Total update count so far (same for every walker). */
 int64_t lapf_sampler_count(const lapf_sampler* s);
 /* Kernel launches issued by this sampler so far (for benchmark accounting). */

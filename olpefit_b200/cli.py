@@ -76,8 +76,79 @@ def _parser(kind):
                     help="write <results>/checkpoint_rank<r>.pt when done (exact state of every walker)")
     ap.add_argument("--resume", action="store_true",
                     help="continue from <results>/checkpoint_rank<r>.pt, appending to the existing chain files")
+    if kind != "step2a":
+        ap.add_argument("--mcse", action="store_true",
+                        help="keep batch means of every recorded value on the device: step2_summary.json gains the "
+                             "effective sample size and Monte Carlo standard error of every parameter and of each "
+                             "companion's separation and position angle")
+        ap.add_argument("--ess-min", type=float, default=None,
+                        help="(implies --mcse) stop once the separation and position-angle ESS of every companion "
+                             "of every epoch is at least this; --accept-min stays the upper bound")
+        ap.add_argument("--rhat-max", type=float, default=None,
+                        help="stop once the Gelman-Rubin RC of every parameter of every epoch is at most this "
+                             "(needs --walkers >= 2); with --ess-min both must hold")
     ap.add_argument("--quiet", action="store_true")
     return ap
+
+
+MCSE_BATCH_ROWS, MCSE_LEVELS = 64, 16
+
+
+def _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on):
+    """Everything the summary and the stop rule read, reduced on the device and summed over ranks:
+    Gelman-Rubin RC per epoch and parameter (apf_step3.py:260-278), the separation / position-angle
+    sketch summary (:283-291,436-437) and the batch-means ESS / MCSE.  Every rank must call it."""
+    import torch
+    from . import chains, dist, stats
+    out = {"rows": 0, "gelman_rubin": None, "sketch": None, "bm": None}
+    P = sam.nparam
+    stt = sam.stats(moments=True)
+    n_rows = int(stt["rows"].item())
+    out["rows"] = n_rows
+    if kind != "step2a" and per_frame > 1 and n_rows > 1:
+        mom = dist.allreduce_sum(stt["moments"] if n_local else torch.zeros_like(stt["moments"]))
+        if world > 1:                     # the reference value of a frame is rank-local; all starts of a frame are equal here
+            mom[:, :, 0] = mom[:, :, 0] / world
+        mom = mom.cpu().numpy()
+        out["gelman_rubin"] = [[float(v) for v in chains.gelman_rubin_from_moments(mom[f, :P], n_rows, per_frame)[1]]
+                               for f in range(n_frames)]
+    if kind != "step2a" and n_rows > 0:
+        sk = sam.sketch()
+        if not n_local:
+            sk["hist"].zero_(); sk["summary"][..., 1:].zero_()
+        sk["hist"] = dist.allreduce_sum(sk["hist"])
+        sums = dist.allreduce_sum(sk["summary"][..., 1:].contiguous())
+        sk["summary"] = torch.cat([sk["summary"][..., :1], sums], dim=-1)
+        out["sketch"] = {k: v.cpu().numpy() for k, v in stats.sketch_summary(sk).items()}
+    if bm_on and n_rows > 0:
+        bm = sam.batch_means()
+        bm["frame"] = dist.allreduce_sum(bm["frame"] if n_local else torch.zeros_like(bm["frame"]))
+        res = stats.batch_means_summary(bm, torch.full((n_frames,), float(per_frame), dtype=torch.float64), n_rows)
+        out["bm"] = {"ess": res["ess"].cpu().numpy(), "mcse": res["mcse"].cpu().numpy(),
+                     "batch_rows": res["batch_rows_used"], "names": bm["names"]}
+    return out
+
+
+def _sep_pa_quantities(nbody):
+    """Batch-mean quantities of the companions' separation and position angle (after the P+1 columns)."""
+    p1 = 3 * nbody + 11
+    return list(range(p1, p1 + 2 * (nbody - 1)))
+
+
+def _converged(es, nbody, ess_min, rhat_max):
+    """The stop rule on the output of _epoch_stats: every epoch meets every criterion given."""
+    if ess_min is not None:
+        bm = es["bm"]
+        if bm is None or bm["batch_rows"] is None:
+            return False
+        ess = bm["ess"][:, _sep_pa_quantities(nbody)]
+        if not (ess >= ess_min).all():          # nan (no level with enough batches yet) fails
+            return False
+    if rhat_max is not None:
+        gr = es["gelman_rubin"]
+        if gr is None or not (np.asarray(gr)[:, : 3 * nbody + 10] <= rhat_max).all():
+            return False
+    return True
 
 
 def _frame_list(args):
@@ -99,6 +170,10 @@ def run(kind, nbody, argv=None):
     args = _parser(kind).parse_args(argv)
     if args.format == "events" and args.thin != 1:
         raise SystemExit("--format events needs --thin 1: rows further apart differ in more than one parameter")
+    stop_rule = kind != "step2a" and (args.ess_min is not None or args.rhat_max is not None)
+    bm_on = kind != "step2a" and (args.mcse or args.ess_min is not None)
+    if stop_rule and args.rhat_max is not None and args.walkers < 2:
+        raise SystemExit("--rhat-max needs at least 2 walkers per epoch (Gelman-Rubin compares walkers)")
     import torch
     from . import chains, dist, frame, layout, sampler as smp, stats
 
@@ -195,6 +270,8 @@ def run(kind, nbody, argv=None):
                 dx, dy = params[f][2 * o] - params[f][0], params[f][2 * o + 1] - params[f][1]
                 centers[f, o - 1] = (np.hypot(dx, dy), np.degrees(np.arctan2(-dx, dy)))
         sam.enable_sketch(centers=centers)
+    if bm_on:
+        sam.enable_batch_means(MCSE_BATCH_ROWS, MCSE_LEVELS)
 
     record = not args.no_chains
     f32 = args.format != "csv" and args.chain_dtype == "f32"
@@ -249,6 +326,7 @@ def run(kind, nbody, argv=None):
         else:
             sam.run(n, record=False)
 
+    stop = {"reason": "accept_min", "updates": 0}
     t_start = time.time()
     if kind == "step2a":
         left = args.n_steps                                   # apf_step2a.py:271
@@ -276,6 +354,16 @@ def run(kind, nbody, argv=None):
             if sam.count % (10 * args.segment) < n:
                 say("Loop count:", sam.count, " min tries:", int(mn.item()),
                     " acceptance rate:", (accepts.double() / tries.double().clamp(min=1)).cpu().numpy())
+            if stop_rule and sam.count >= burn_in:
+                # decided on rank 0 from all-reduced sums and broadcast: every rank stops at the same update
+                es = _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on)
+                done = torch.tensor([1 if (rank == 0 and _converged(es, nbody, args.ess_min, args.rhat_max)) else 0],
+                                    dtype=torch.int64, device=device)
+                if world > 1:
+                    torch.distributed.broadcast(done, 0)
+                if int(done.item()):
+                    stop["reason"] = "converged"
+                    break
     if record:
         consume(streamer.finish())
     if packed is None and record and first[0] and n_local:
@@ -294,27 +382,16 @@ def run(kind, nbody, argv=None):
     # of each companion (median, 68 % interval, mean, std; :283-291,436-437; without the distortion,
     # rotation and refraction corrections, whose tables are not part of the checkout).
     summaries = [dict(image=images[f], walkers=per_frame, updates=sam.count) for f in range(n_frames)]
-    stt = sam.stats(moments=True)
-    n_rows = int(stt["rows"].item())
-    if kind != "step2a" and per_frame > 1 and n_rows > 1:
-        mom = dist.allreduce_sum(stt["moments"] if n_local else torch.zeros_like(stt["moments"]))
-        if world > 1:                     # the reference value of a frame is rank-local; all starts of a frame are equal here
-            mom[:, :, 0] = mom[:, :, 0] / world
-        mom = mom.cpu().numpy()
+    es = _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on)
+    n_rows = es["rows"]
+    if es["gelman_rubin"] is not None:
         for f in range(n_frames):
-            _, rc = chains.gelman_rubin_from_moments(mom[f, :P], n_rows, per_frame)
-            summaries[f]["gelman_rubin"] = [float(v) for v in rc]
+            summaries[f]["gelman_rubin"] = es["gelman_rubin"][f]
         say("Gelman-Rubin stat per parameter (recorded rows, all walkers%s):" % ("" if n_frames == 1 else ", first epoch"),
             np.round(summaries[0]["gelman_rubin"], 4))
         say("GR for positions:", *np.round(summaries[0]["gelman_rubin"][:2 * nbody], 4))
     if want_sketch and n_rows > 0:
-        sk = sam.sketch()
-        if not n_local:
-            sk["hist"].zero_(); sk["summary"][..., 1:].zero_()
-        sk["hist"] = dist.allreduce_sum(sk["hist"])
-        sums = dist.allreduce_sum(sk["summary"][..., 1:].contiguous())
-        sk["summary"] = torch.cat([sk["summary"][..., :1], sums], dim=-1)
-        res = {k: v.cpu().numpy() for k, v in stats.sketch_summary(sk).items()}
+        res = es["sketch"]
         names = ["companion"] if nbody == 2 else ["b", "c"]
         for f in range(n_frames):
             for o, nm in enumerate(names):
@@ -327,6 +404,21 @@ def run(kind, nbody, argv=None):
                                "std": float(res["pa_std"][f, o])},
                     "rows": int(res["count"][f, o]), "outside_histogram": float(res["outside"][f, o].max()),
                     "pixscale_mas": float(chains.PIXSCALE_PRE2015)}
+        if es["bm"] is not None:
+            # Monte Carlo error of the means from the batch means (separation scaled to mas like the summary)
+            bm = es["bm"]
+            pnames = bm["names"][:P]
+            for f in range(n_frames):
+                summaries[f]["batch_rows"] = bm["batch_rows"]
+                summaries[f]["ess"] = {nm: float(bm["ess"][f, j]) for j, nm in enumerate(pnames)}
+                summaries[f]["mcse"] = {nm: float(bm["mcse"][f, j]) for j, nm in enumerate(pnames)}
+                for o, nm in enumerate(names):
+                    c = P + 1 + 2 * o
+                    d = summaries[f]["sep_pa_%s" % nm]
+                    d["sep_mas"]["ess"] = float(bm["ess"][f, c])
+                    d["sep_mas"]["mcse"] = float(bm["mcse"][f, c] * chains.PIXSCALE_PRE2015)
+                    d["pa_deg"]["ess"] = float(bm["ess"][f, c + 1])
+                    d["pa_deg"]["mcse"] = float(bm["mcse"][f, c + 1])
         for f in range(min(n_frames, 8)):
             for nm in names:
                 s_ = summaries[f]["sep_pa_%s" % nm]
@@ -335,6 +427,14 @@ def run(kind, nbody, argv=None):
                        s_["sep_mas"]["median"] - s_["sep_mas"]["lo"], s_["sep_mas"]["std"], s_["pa_deg"]["median"],
                        s_["pa_deg"]["hi"] - s_["pa_deg"]["median"], s_["pa_deg"]["median"] - s_["pa_deg"]["lo"],
                        s_["pa_deg"]["std"], s_["rows"]))
+                if "ess" in s_["sep_mas"]:
+                    say("epoch %d %s: ESS r %.0f pa %.0f, MCSE r %.4f mas pa %.5f deg  [batches of %s rows]"
+                        % (f, nm, s_["sep_mas"]["ess"], s_["pa_deg"]["ess"], s_["sep_mas"]["mcse"],
+                           s_["pa_deg"]["mcse"], summaries[f]["batch_rows"]))
+    if stop_rule or bm_on:
+        stop["updates"] = sam.count
+        for f in range(n_frames):
+            summaries[f]["stop"] = dict(stop)
     if rank == 0 and kind != "step2a":
         for f in range(n_frames):
             with open(outdirs[f] + "step2_summary.json", "w") as fh:

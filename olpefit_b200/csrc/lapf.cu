@@ -328,6 +328,12 @@ struct RunArgs {
     double* sk_mom;              // [W][NB-1][2][2]: per walker sum / sum of squares of (value - centre)
     double sk_inv_sep, sk_inv_pa;   // 1 / bin width
     int sk_bins, chain_f32, chain_ev;
+    // batch means (lapf_sampler_batchmeans_enable), or nullptr: per walker, quantity (the P+1 columns, then
+    // the sketch slots) and level l the running sum at the last level-l boundary and the sum of squared batch sums
+    double* bm;                  // [W][bm_c][bm_levels][2]
+    int64_t bm_q0;               // complete bm_rows-row batches of every walker before this launch
+    int bm_rows, bm_phase;       // batch length of level 0; rows recorded since the last level-0 boundary
+    int bm_levels, bm_c;
     double* probe;               // self-test only: [rows][W][3] = parameter index, proposed value, TRIAL chi-square
     unsigned long long* cta_times;   // diagnosis only (LAPF_CTA_TIMES): [CTAs][3] = start, end (globaltimer ns), SM id
     int64_t n_walkers;
@@ -339,6 +345,40 @@ struct RunArgs {
     uint32_t log_mask;
     int thin, floor_index, n_items, cull, plain;
 };
+
+// Batch means: the number of levels that launch-relative row `row` closes.  With it the walker has
+// recorded bm_q0 * bm_rows + bm_phase + row + 1 rows; level l closes when that count is a multiple
+// of bm_rows * 2^l.  0 when batch means are off or the row closes no batch (all but one row in bm_rows).
+__device__ __forceinline__ int bm_closing(const RunArgs& a, int row) {
+    if (!a.bm) return 0;
+    const int r = a.bm_phase + row + 1;
+    if (r % a.bm_rows) return 0;
+    return min(__ffsll((long long)(a.bm_q0 + r / a.bm_rows)), a.bm_levels);
+}
+
+// Close the first n_lev levels of quantity c (< bm_c) of walker wl once the row's running sums are
+// stored: S = M1 - snap, s2 += S*S, snap = M1, never contracted (DESIGN.md 5: the tests restate it bit
+// for bit).  M1 is read back from L2, where this thread -- its single writer -- performed its atomics:
+// exactly the value the last atomicAdd stored.  So the moment updates stay fire-and-forget REDs, with
+// batch means on or off, and no return value is held in registers through the row.
+template <int NB>
+__device__ __forceinline__ void bm_close(const RunArgs& a, int wl, int c, int n_lev) {
+    constexpr int P = Layout<NB>::P;
+    const double m1 = __ldcg(c <= P ? a.moments + 2 * ((size_t)wl * (P + 1) + c)
+                                    : a.sk_mom + 2 * ((size_t)wl * (a.bm_c - P - 1) + (c - P - 1)));
+    double* b = a.bm + ((size_t)wl * a.bm_c + c) * a.bm_levels * 2;
+#pragma unroll 1
+    for (int l = 0; l < n_lev; ++l) {
+        const double S = __dsub_rn(m1, b[2 * l]);
+        b[2 * l + 1] = __dadd_rn(b[2 * l + 1], __dmul_rn(S, S));
+        b[2 * l] = m1;
+    }
+}
+
+// Quantities a recorded row adds to: the P+1 columns, and the sketch slots when sketches are recorded
+// (the self-test records none)
+template <int NB>
+__device__ __forceinline__ int bm_quantities(const RunArgs& a) { return a.sk_hist ? a.bm_c : Layout<NB>::P + 1; }
 
 // One recorded row of one walker enters the sketches of its frame: for every companion the
 // separation sqrt(dx^2 + dy^2) in pixels and the position angle degrees(atan2(-dx, dy))
@@ -517,12 +557,18 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
                 }
                 atomicAdd(&a.moments[2 * mi], dl);                    // single writer: plain RED, in order
                 atomicAdd(&a.moments[2 * mi + 1], dl * dl);
+                if (const int n_lev = bm_closing(a, row)) bm_close<NB>(a, wl, lane, n_lev);   // lane c closes column c
             }
             if (a.sk_hist) {
                 double xy[2 * NB];
 #pragma unroll
                 for (int j = 0; j < 2 * NB; ++j) xy[j] = shfl_f64(p, j);
-                if (lane == 0 && tw == 0) record_sketch<NB>(a, wl, frame, xy);
+                if (lane == 0 && tw == 0) {
+                    record_sketch<NB>(a, wl, frame, xy);
+                    if (const int n_lev = bm_closing(a, row))
+#pragma unroll 1
+                        for (int c = Layout<NB>::P + 1; c < a.bm_c; ++c) bm_close<NB>(a, wl, c, n_lev);
+                }
             }
             ++row;
             next_rec += a.thin;   // (saturates harmlessly: a launch is shorter than 2^30)
@@ -773,6 +819,14 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
 #pragma unroll
                     for (int j = 0; j < 2 * NB; ++j) xy[j] = st[j];
                     record_sketch<NB>(a, wl, (two && slot) ? frame1 : frame0, xy);
+                }
+                if (a.bm) {
+                    const int n_lev = bm_closing(a, row);
+                    if (n_lev) {
+                        const int nq = bm_quantities<NB>(a);
+#pragma unroll 1
+                        for (int c = 0; c < nq; ++c) bm_close<NB>(a, wl, c, n_lev);
+                    }
                 }
                 if (a.probe) {                                            // lapf_sampler_selftest
                     double* pb = a.probe + ((size_t)row * a.n_walkers + wl) * 3;
@@ -1080,6 +1134,44 @@ __global__ void sketch_reduce_kernel(const double* __restrict__ sk_mom, const do
     }
 }
 
+// Batch means per frame, one CTA per frame; warp i takes the items i, i + warps, ... of [C][1 + L] and
+// reduces over the frame's walkers in the fixed order of moments_kernel.  Item (c, 0): sum of the
+// walkers' population variance of quantity c over their recorded rows (np.std()**2, apf_step3.py:270),
+// from the running moments (columns) or the sketch sums (separation / position angle).  Item (c, 1 + l):
+// sum of the sample variances of the walkers' level-l batch means, each from its (snap, s2) and J
+// complete batches of b = b0 * 2^l rows: (s2 - snap^2 / J) / (b^2 (J - 1)); 0 where J < 2.
+__global__ void batchmeans_reduce_kernel(const double* __restrict__ bm, const double* __restrict__ moments,
+                                         const double* __restrict__ sk_mom, const int32_t* __restrict__ walker_of,
+                                         const int32_t* __restrict__ frame_start, int P, int C, int L, int b0,
+                                         int64_t n_rows, double* __restrict__ out /*[F][C][1 + L]*/) {
+    const int f = blockIdx.x, lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+    const int b = frame_start[f], e = frame_start[f + 1], slots = C - (P + 1);
+    for (int it = threadIdx.x >> 5; it < C * (1 + L); it += warps) {
+        const int c = it / (1 + L), j = it % (1 + L);
+        double s = 0.0;
+        if (j == 0 && n_rows > 0) {
+            const double inv = 1.0 / (double)n_rows;
+            for (int i = b + lane; i < e; i += 32) {
+                const size_t w = (size_t)walker_of[i];
+                const double* m = (c <= P) ? moments + (w * (P + 1) + c) * 2 : sk_mom + (w * slots + (c - P - 1)) * 2;
+                const double m1 = m[0] * inv, m2 = m[1] * inv;
+                s += m2 - m1 * m1;
+            }
+        } else if (j > 0) {
+            const int64_t bl = (int64_t)b0 << (j - 1), J = n_rows / bl;
+            if (J >= 2) {
+                const double inv_j = 1.0 / (double)J, scale = 1.0 / ((double)bl * (double)bl * (double)(J - 1));
+                for (int i = b + lane; i < e; i += 32) {
+                    const double* q = bm + (((size_t)walker_of[i] * C + c) * L + (j - 1)) * 2;
+                    s += (q[1] - q[0] * q[0] * inv_j) * scale;
+                }
+            }
+        }
+        s = warp_sum_f64(s);
+        if (lane == 0) out[((size_t)f * C + c) * (1 + L) + j] = s;
+    }
+}
+
 // The same cut-out + mask + noise map with the pixels fetched by the TMA unit: a 3-D tensor map over
 // the frames [F][fy][fx] and one box of kPrepRows x (nx + 4) pixels per CTA (cp.async.bulk.tensor,
 // SASS UTMALDG) -- rows of a cut-out are nx * 4 bytes long and fx * 4 bytes apart, which is exactly
@@ -1251,6 +1343,9 @@ struct lapf_sampler {
     uint32_t* sk_hist = nullptr;
     double* sk_center = nullptr;
     double* sk_mom = nullptr;
+    // batch means (lapf_sampler_batchmeans_enable): [W][bm_c][bm_levels][2]
+    double* bm = nullptr;
+    int bm_rows = 0, bm_levels = 0, bm_c = 0;
     int chunk = 0;                 // batched kernel: walkers per item at most (warps x walkers per warp)
     int launch_grid = 0;           // batched kernel: CTAs that have work
 };
@@ -1502,6 +1597,7 @@ static void free_sampler(lapf_sampler* s) {
     cudaFree(s->item_count); cudaFree(s->cta_item); cudaFree(s->frame_of);
     cudaFree(s->item_frame2); cudaFree(s->item_count_a); cudaFree(s->item_slot_a);
     cudaFree(s->sk_hist); cudaFree(s->sk_center); cudaFree(s->sk_mom);
+    cudaFree(s->bm);
     delete s;
 }
 
@@ -1661,6 +1757,10 @@ int lapf_sampler_create(const lapf_config* cfg, lapf_sampler** out, void* stream
     return LAPF_OK;
 }
 
+static size_t bm_state_bytes(const lapf_sampler* s) {
+    return s->bm ? sizeof(double) * (size_t)s->cfg.n_walkers * s->bm_c * s->bm_levels * 2 : 0;
+}
+
 int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed, void* stream) {
     if (!s || !init_params) return fail(LAPF_ERR_INVALID, "sampler/init_params is NULL");
     cudaStream_t st = (cudaStream_t)stream;
@@ -1693,12 +1793,16 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
             s->launches++;
         }
     }
+    if (s->bm) CU(cudaMemsetAsync(s->bm, 0, bm_state_bytes(s), st));
     return LAPF_OK;
 }
 
 // Checkpoint layout (device blob, 8-byte units): [count][seed][jump widths x LAPF_MAX_PARAMS] state shift
-// moments(2x) exps tries accepts [sketch sums, sketch histograms]
+// moments(2x) exps tries accepts [sketch sums, sketch histograms] [batch-means descriptor, batch-means state]
 constexpr size_t kCkptHead = 8 * (2 + LAPF_MAX_PARAMS);
+// batch-means descriptor: int64 [magic, batch_rows, levels, C]
+constexpr size_t kCkptBmDesc = 32;
+constexpr int64_t kBmMagic = 0x31304d424650414cLL;   // the bytes 'LAPFBM01'
 static size_t sketch_hist_bytes(const lapf_sampler* s) {
     return s->sk_hist ? sizeof(uint32_t) * (size_t)s->cfg.problem.n_frames * 2 * (s->cfg.problem.nbody - 1) * (s->sk_bins + 2) : 0;
 }
@@ -1708,7 +1812,8 @@ static size_t sketch_mom_bytes(const lapf_sampler* s) {
 static size_t checkpoint_bytes(const lapf_sampler* s) {
     const size_t W = (size_t)s->cfg.n_walkers, P = (size_t)s->P, nst = W * (P + 1);
     return kCkptHead + sizeof(double) * nst * 4 + sizeof(unsigned long long) * W + sizeof(uint32_t) * W * P * 2 +
-           sketch_mom_bytes(s) + sketch_hist_bytes(s);      // the sketches too, once they are enabled
+           sketch_mom_bytes(s) + sketch_hist_bytes(s) +     // the sketches too, once they are enabled
+           (s->bm ? kCkptBmDesc + bm_state_bytes(s) : 0);   // and the batch means
 }
 
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s) {
@@ -1729,8 +1834,17 @@ static int checkpoint_copy(lapf_sampler* s, unsigned char* blob, bool save, cuda
                            cudaMemcpyDeviceToDevice, st));
         off += p.bytes;
     }
+    if (s->bm) {
+        // the descriptor was written (save) or checked (load) by the caller
+        off += kCkptBmDesc;
+        CU(cudaMemcpyAsync(save ? (void*)(blob + off) : (void*)s->bm, save ? (const void*)s->bm : (const void*)(blob + off),
+                           bm_state_bytes(s), cudaMemcpyDeviceToDevice, st));
+    }
     return LAPF_OK;
 }
+
+// Offset of the batch-means descriptor in the blob (batch means on)
+static size_t bm_desc_offset(const lapf_sampler* s) { return checkpoint_bytes(s) - bm_state_bytes(s) - kCkptBmDesc; }
 
 int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* stream) {
     if (!s || !blob) return fail(LAPF_ERR_INVALID, "sampler/blob is NULL");
@@ -1739,7 +1853,9 @@ int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* str
     int64_t head[2 + LAPF_MAX_PARAMS] = {s->count, (int64_t)s->cfg.seed};
     memcpy(head + 2, s->widths, sizeof(double) * LAPF_MAX_PARAMS);   // --adapt may have changed them
     CU(cudaMemcpyAsync(blob, head, kCkptHead, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));   // `head` lives on this stack frame
+    const int64_t desc[4] = {kBmMagic, s->bm_rows, s->bm_levels, s->bm_c};
+    if (s->bm) CU(cudaMemcpyAsync((unsigned char*)blob + bm_desc_offset(s), desc, kCkptBmDesc, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));   // `head` and `desc` live on this stack frame
     return checkpoint_copy(s, (unsigned char*)blob, true, st);
 }
 
@@ -1755,6 +1871,15 @@ int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, voi
     bool ok = head[0] >= 0;
     for (int i = 0; i < s->P; ++i) ok = ok && wd[i] >= 0.0 && std::isfinite(wd[i]);
     if (!ok) return fail(LAPF_ERR_INVALID, "corrupt checkpoint (count %lld)", (long long)head[0]);
+    if (s->bm) {
+        int64_t desc[4] = {0, 0, 0, 0};
+        CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + bm_desc_offset(s), kCkptBmDesc, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (desc[0] != kBmMagic || desc[1] != s->bm_rows || desc[2] != s->bm_levels || desc[3] != s->bm_c)
+            return fail(LAPF_ERR_INVALID, "checkpoint batch means (batch_rows %lld, levels %lld, %lld quantities) do not match "
+                        "this sampler's (%d, %d, %d)", (long long)desc[1], (long long)desc[2], (long long)desc[3],
+                        s->bm_rows, s->bm_levels, s->bm_c);
+    }
     s->count = head[0];
     s->cfg.seed = (uint64_t)head[1];
     memcpy(s->widths, wd, sizeof(wd));
@@ -1832,6 +1957,13 @@ static void fill_run_args(const lapf_sampler* s, RunArgs& a, int64_t n_updates, 
     a.thin = s->cfg.thin; a.floor_index = pb.floor_index; a.n_items = s->n_items;
     a.cull = cull_enabled(&pb);
     a.plain = plain_loop(&pb);
+    a.bm = s->bm; a.bm_rows = s->bm_rows; a.bm_levels = s->bm_levels; a.bm_c = s->bm_c;
+    a.bm_q0 = 0; a.bm_phase = 0;
+    if (s->bm) {
+        const int64_t r0 = rows_upto(s->count, s->cfg.burn_in, s->cfg.thin);
+        a.bm_q0 = r0 / s->bm_rows;
+        a.bm_phase = (int)(r0 % s->bm_rows);
+    }
     a.probe = nullptr;
     a.cta_times = nullptr;
 }
@@ -1961,6 +2093,9 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     a.chain_ev = 0;
     a.ev_code = nullptr; a.ev_val = nullptr; a.ev_chi = nullptr;
     a.sk_hist = nullptr;
+    // batch means (if on) with batch length 1: every recorded row closes a batch, so the update after each
+    // closing row is checked too; the load below restores their state
+    a.bm_rows = 1; a.bm_q0 = 0; a.bm_phase = 0;
     a.probe = probe;
     rc = launch_dispatch(s, a, st);
     if (rc) { cleanup(); return rc; }
@@ -2031,6 +2166,8 @@ int lapf_sampler_sketch_enable(lapf_sampler* s, int32_t n_bins, double sep_bin, 
     cudaStream_t st = (cudaStream_t)stream;
     const int F = s->cfg.problem.n_frames, nbody = s->cfg.problem.nbody, slots = 2 * (nbody - 1);
     const int64_t W = s->cfg.n_walkers;
+    if (s->bm)
+        return fail(LAPF_ERR_INVALID, "sketches cannot be enabled after batch means (the batch means would change shape)");
     CU(cudaStreamSynchronize(st));
     cudaFree(s->sk_hist); cudaFree(s->sk_center); cudaFree(s->sk_mom);
     s->sk_hist = nullptr; s->sk_center = nullptr; s->sk_mom = nullptr;
@@ -2068,6 +2205,48 @@ int lapf_sampler_sketch(lapf_sampler* s, uint32_t* hist_out, double* summary_out
         const int64_t n_rows = rows_upto(s->count, s->cfg.burn_in, s->cfg.thin);
         sketch_reduce_kernel<<<F, 32 * slots, 0, st>>>(s->sk_mom, s->sk_center, s->walker_of, s->frame_start, slots, n_rows,
                                                       summary_out);
+        CU(cudaGetLastError());
+        s->launches++;
+    }
+    return LAPF_OK;
+}
+
+int lapf_sampler_batchmeans_enable(lapf_sampler* s, int32_t batch_rows, int32_t levels, void* stream) {
+    if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
+    if (batch_rows < 1 || batch_rows > (1 << 30) || levels < 1 || levels > 24)
+        return fail(LAPF_ERR_INVALID, "batch means need batch_rows in [1, 2^30] and levels in [1, 24]");
+    if (rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) > 0)
+        return fail(LAPF_ERR_INVALID, "batch means must be enabled before the first recorded row");
+    cudaStream_t st = (cudaStream_t)stream;
+    CU(cudaStreamSynchronize(st));
+    cudaFree(s->bm);
+    s->bm = nullptr;
+    const int C = s->P + 1 + (s->sk_hist ? 2 * (s->cfg.problem.nbody - 1) : 0);
+    const size_t bytes = sizeof(double) * (size_t)s->cfg.n_walkers * C * levels * 2;
+    CU(cudaMalloc((void**)&s->bm, bytes));
+    s->bm_rows = batch_rows;
+    s->bm_levels = levels;
+    s->bm_c = C;
+    CU(cudaMemsetAsync(s->bm, 0, bytes, st));
+    int rc = LAPF_OK;
+    if (!getenv("LAPF_NO_SELFTEST") && (rc = lapf_sampler_selftest(s, st))) {
+        cudaStreamSynchronize(st);
+        cudaFree(s->bm);
+        s->bm = nullptr;
+    }
+    return rc;
+}
+
+int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_out, void* stream) {
+    if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
+    if (!s->bm) return fail(LAPF_ERR_INVALID, "batch means are not enabled (lapf_sampler_batchmeans_enable)");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (walker_out) CU(cudaMemcpyAsync(walker_out, s->bm, bm_state_bytes(s), cudaMemcpyDeviceToDevice, st));
+    if (frame_out) {
+        const int64_t n_rows = rows_upto(s->count, s->cfg.burn_in, s->cfg.thin);
+        batchmeans_reduce_kernel<<<s->cfg.problem.n_frames, 256, 0, st>>>(s->bm, s->moments, s->sk_mom, s->walker_of,
+                                                                        s->frame_start, s->P, s->bm_c, s->bm_levels,
+                                                                        s->bm_rows, n_rows, frame_out);
         CU(cudaGetLastError());
         s->launches++;
     }

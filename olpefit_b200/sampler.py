@@ -47,6 +47,7 @@ class GibbsSampler:
         self.chain_dtype = torch.float64
         self.events = False
         self._sketch = None
+        self._bm = None
         handle = C.c_void_p()
         _lib.check(self.lib.lapf_sampler_create(C.byref(cfg), C.byref(handle), _stream_ptr(dev)))
         self._h = handle
@@ -148,6 +149,46 @@ class GibbsSampler:
         summ = torch.empty(shape + (4,), dtype=torch.float64, device=dev)
         _lib.check(self.lib.lapf_sampler_sketch(self._h, hist.data_ptr(), summ.data_ptr(), _stream_ptr(dev)))
         return {"hist": hist.long() & 0xFFFFFFFF, "summary": summ, "n_bins": n_bins, "sep_bin": sep_bin, "pa_bin": pa_bin}
+
+    # -- batch means: Monte Carlo standard errors without the chain --------------------------
+    def enable_batch_means(self, batch_rows=64, levels=12):
+        """From now on every walker keeps batch means of every recorded value at batch lengths
+        batch_rows * 2^l rows, l < levels: the chain columns and, if ``enable_sketch`` was called
+        before, the separation and position angle of each companion.  Call before the first recorded
+        row.  ``stats.batch_means_summary`` turns them into effective sample sizes and standard errors."""
+        _lib.check(self.lib.lapf_sampler_batchmeans_enable(self._h, int(batch_rows), int(levels),
+                                                           _stream_ptr(self.domain.device)))
+        names = list(self._param_names()) + ["chi2"]
+        if self._sketch is not None:
+            for o in range(1, self.domain.nbody):
+                names += ["sep%d" % o, "pa%d" % o]
+        self._bm = (int(batch_rows), int(levels), names)
+
+    def _param_names(self):
+        from . import layout
+        return layout.names(self.domain.nbody)
+
+    def batch_means(self):
+        """dict(walker [W, C, levels, 2] (snap, s2), frame [F, C, 1 + levels] (sum over the frame's walkers
+        of their row variance, then of the sample variance of their level-l batch means) as float64 device
+        tensors, batch_rows, levels, rows (recorded per walker), names [C]) -- see include/lapf.h."""
+        if self._bm is None:
+            raise _lib.LapfError("batch means are not enabled")
+        dev = self.domain.device
+        batch_rows, levels, names = self._bm
+        c = len(names)
+        walker = torch.empty((self.n_walkers, c, levels, 2), dtype=torch.float64, device=dev)
+        frame = torch.empty((self.domain.n_frames, c, 1 + levels), dtype=torch.float64, device=dev)
+        _lib.check(self.lib.lapf_sampler_batchmeans(self._h, walker.data_ptr(), frame.data_ptr(), _stream_ptr(dev)))
+        return {"walker": walker, "frame": frame, "batch_rows": batch_rows, "levels": levels,
+                "rows": self.rows_recorded(), "names": names}
+
+    def rows_recorded(self) -> int:
+        """Chain rows every walker has recorded since the last reset."""
+        n = self.count
+        if n < self.burn_in or n < 1:
+            return 0
+        return (n - self.burn_in) // self.thin + (1 if self.burn_in > 0 else 0)
 
     # -- the loop ------------------------------------------------------------------------
     @property

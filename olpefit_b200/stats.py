@@ -60,6 +60,44 @@ def gelman_rubin(chain_cols, python2_division=True):
 
 
 # ----------------------------------------------------------------------------------------------
+# Monte Carlo error from the on-device batch means (lapf_sampler_batchmeans): no chain needed
+# ----------------------------------------------------------------------------------------------
+def batch_means_summary(bm, walkers_per_frame, rows, min_batches=20):
+    """Per frame and quantity, from ``GibbsSampler.batch_means()`` (its ``frame`` sums and the walker
+    counts all-reduced over ranks if the walkers are sharded) with M walkers of ``rows`` rows each:
+    the largest batch length b = batch_rows * 2^l with J = rows // b >= ``min_batches`` complete
+    batches is used; with s2 the mean over walkers of the sample variance of their batch means and
+    sigma2 the mean of their row variances,
+        tau = b * s2 / sigma2  (integrated autocorrelation time, rows),  ess = M * rows / tau,
+        mcse = sqrt(s2 / (J * M))  (standard error of the mean pooled over the frame's walkers).
+    Returns a dict of float64 tensors: tau, ess, mcse [F, C] (nan where no level qualifies),
+    tau_levels [F, C, levels] (nan at the levels with fewer than ``min_batches`` batches: a reader
+    sees whether tau has levelled off), batch_rows_used (int, or None if no level qualifies)."""
+    frame = torch.as_tensor(bm["frame"], dtype=torch.float64)
+    b0, levels, rows = int(bm["batch_rows"]), int(bm["levels"]), int(rows)
+    m = torch.as_tensor(walkers_per_frame, dtype=torch.float64, device=frame.device).reshape(-1, 1)
+    sigma2 = frame[..., 0] / m
+    nan = torch.full_like(sigma2, float("nan"))
+    tau_levels, use = [], None
+    for lv in range(levels):
+        b = b0 << lv
+        if rows // b >= min_batches:
+            tau_levels.append(b * (frame[..., 1 + lv] / m) / sigma2)
+            use = lv
+        else:
+            tau_levels.append(nan)
+    if use is None:
+        return {"tau": nan, "ess": nan.clone(), "mcse": nan.clone(), "tau_levels": torch.stack(tau_levels, dim=-1),
+                "batch_rows_used": None}
+    b = b0 << use
+    j = rows // b
+    s2 = frame[..., 1 + use] / m
+    tau = b * s2 / sigma2
+    return {"tau": tau, "ess": m * rows / tau, "mcse": torch.sqrt(s2 / (j * m)),
+            "tau_levels": torch.stack(tau_levels, dim=-1), "batch_rows_used": b}
+
+
+# ----------------------------------------------------------------------------------------------
 # the same summary from the on-device sketches (lapf_sampler_sketch): no chain needed
 # ----------------------------------------------------------------------------------------------
 def quantiles_from_hist(hist, center, bin_width, q=Q68):
