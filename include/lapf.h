@@ -261,6 +261,25 @@ int lapf_sampler_batchmeans_enable(lapf_sampler* s, int32_t batch_rows, int32_t 
  *              Sums over walkers: all-reduce them over GPUs like the moments. */
 int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_out, void* stream);
 
+/* K4d -- posterior draws: a uniformly random sample of K recorded rows per walker, kept on the device
+ * (DESIGN.md, "Posterior draws").  Reservoir sampling (algorithm R) over the rows the moments see (after
+ * burn-in and thinning, with or without chain_out): walker row n (0 for the first recorded row, counted
+ * across launches) fills slot n if n < K; otherwise it replaces slot j = mulhi64(r, n + 1) if j < K, where
+ * r = r0 | r1 << 32 of philox4x32_10(counter = (n low, n high, seed high, 'LAPR'), key = (seed low, walker
+ * id)), the walker id of make_draw (id_base + w * id_stride).  The selection depends on (seed, walker id, n)
+ * only; the update stream is untouched.  mulhi64 without rejection biases j by at most (n + 1) / 2^64.
+ * A slot holds the row's P+1 values (state after accept / reject, chain column order, frame coordinates)
+ * and n; an empty slot has n = -1 and all-ones (NaN) values.  Memory W * K * (P + 2) * 8 bytes.
+ * 1 <= per_walker <= 65536.  LAPF_ERR_INVALID once any row has been recorded, or if draws are already on.
+ * Independent of sketches and batch means, in either order.  Runs lapf_sampler_selftest with the reservoir
+ * active and one slot (unless LAPF_NO_SELFTEST), so that self-test rows 1 and 2 replace slot 0, and leaves
+ * the sampler as it was.  lapf_sampler_reset empties the reservoir; checkpoints carry it as the last
+ * section, behind a 32-byte descriptor (int64 magic 'LAPFRS01', K, P+1, 0) that lapf_sampler_load checks;
+ * blobs of samplers without draws keep their layout and size. */
+int lapf_sampler_draws_enable(lapf_sampler* s, int32_t per_walker, void* stream);
+/*   values_out device double [W][K][P+1] or NULL; rows_out device int64 [W][K] or NULL */
+int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, void* stream);
+
 /* Total update count so far (same for every walker). */
 int64_t lapf_sampler_count(const lapf_sampler* s);
 /* Kernel launches issued by this sampler so far (for benchmark accounting). */

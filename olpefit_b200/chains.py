@@ -102,6 +102,39 @@ def write_acceptance(path, accepts, tries):
         fh.write(str(rate))
 
 
+def write_draws_csv(path, walkers, values, rows, names):
+    """Posterior draws of one epoch (``GibbsSampler.draws``): a '#' header line naming the columns, then
+    one line per filled slot -- walker number, recorded-row index, the P parameters, chi-square --
+    sorted by (walker, row).  ``walkers`` [W] are the walkers' numbers, ``values`` [W, K, P+1],
+    ``rows`` [W, K] (-1: empty slot).  Values are printed as repr(float): they parse back to the same
+    doubles.  Returns the number of lines written after the header."""
+    walkers = np.asarray(walkers, dtype=np.int64)
+    values = np.asarray(values, dtype=np.float64)
+    rows = np.asarray(rows, dtype=np.int64)
+    w_idx, k_idx = np.nonzero(rows >= 0)
+    order = np.lexsort((rows[w_idx, k_idx], walkers[w_idx]))
+    w_idx, k_idx = w_idx[order], k_idx[order]
+    with open(path, "w") as fh:
+        fh.write("# " + ",".join(["walker", "row"] + list(names)) + "\n")
+        for w, k in zip(w_idx.tolist(), k_idx.tolist()):
+            fh.write("%d,%d,%s\n" % (walkers[w], rows[w, k], ",".join(map(repr, values[w, k].tolist()))))
+    return len(w_idx)
+
+
+def read_draws_csv(path):
+    """(names, walker [n] int64, row [n] int64, values [n, P+1] float64) of a ``write_draws_csv`` file."""
+    with open(path) as fh:
+        head = fh.readline()
+        if not head.startswith("# "):
+            raise ValueError("%s: not a draws file" % path)
+        names = head[2:].strip().split(",")[2:]
+        lines = [ln.split(",") for ln in fh.read().splitlines() if ln]
+    walker = np.array([int(x[0]) for x in lines], dtype=np.int64)
+    row = np.array([int(x[1]) for x in lines], dtype=np.int64)
+    values = np.array([[float(v) for v in x[2:]] for x in lines], dtype=np.float64).reshape(len(lines), len(names))
+    return names, walker, row, values
+
+
 # ----------------------------------------------------------------------------------------------
 # chain events (LAPF_CHAIN_EVENTS_*, include/lapf.h): the one place on the host that knows the layout
 # ----------------------------------------------------------------------------------------------

@@ -29,6 +29,13 @@ import time
 import numpy as np
 
 
+def _positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be a positive integer, got %s" % text)
+    return v
+
+
 def _parser(kind):
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("image", type=str)
@@ -87,6 +94,10 @@ def _parser(kind):
         ap.add_argument("--rhat-max", type=float, default=None,
                         help="stop once the Gelman-Rubin RC of every parameter of every epoch is at most this "
                              "(needs --walkers >= 2); with --ess-min both must hold")
+        ap.add_argument("--draws", type=_positive_int, default=None, metavar="K",
+                        help="keep a uniformly random sample of K recorded rows of every walker on the device and "
+                             "write them to <results>/step2_draws.csv (also with --no-chains); step2_summary.json "
+                             "gains the separation-PA correlation of these draws")
     ap.add_argument("--quiet", action="store_true")
     return ap
 
@@ -127,6 +138,20 @@ def _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on):
         out["bm"] = {"ess": res["ess"].cpu().numpy(), "mcse": res["mcse"].cpu().numpy(),
                      "batch_rows": res["batch_rows_used"], "names": bm["names"]}
     return out
+
+
+def _gather_draws(d, n_local, rank, world):
+    """``GibbsSampler.draws()`` of every rank's first n_local walkers to rank 0 in global walker order
+    (the interleaved sharding of dist.shard_ids): (values [W_total, K, P+1], rows [W_total, K]) as numpy
+    arrays on rank 0, (None, None) elsewhere.  Every rank must call it."""
+    from . import dist
+    vals = d["values"][:n_local].transpose(0, 1).contiguous()                  # [K, W_local, P+1]
+    rws = d["rows"][:n_local].transpose(0, 1).unsqueeze(-1).contiguous()     # [K, W_local, 1]
+    parts_v, parts_r = dist.gather_chains(vals, rank, world), dist.gather_chains(rws, rank, world)
+    if rank != 0:
+        return None, None
+    return (dist.merge_interleaved(parts_v).transpose(0, 1).cpu().numpy(),
+            dist.merge_interleaved(parts_r)[..., 0].transpose(0, 1).cpu().numpy())
 
 
 def _sep_pa_quantities(nbody):
@@ -172,6 +197,7 @@ def run(kind, nbody, argv=None):
         raise SystemExit("--format events needs --thin 1: rows further apart differ in more than one parameter")
     stop_rule = kind != "step2a" and (args.ess_min is not None or args.rhat_max is not None)
     bm_on = kind != "step2a" and (args.mcse or args.ess_min is not None)
+    draws_k = getattr(args, "draws", None)
     if stop_rule and args.rhat_max is not None and args.walkers < 2:
         raise SystemExit("--rhat-max needs at least 2 walkers per epoch (Gelman-Rubin compares walkers)")
     import torch
@@ -272,6 +298,8 @@ def run(kind, nbody, argv=None):
         sam.enable_sketch(centers=centers)
     if bm_on:
         sam.enable_batch_means(MCSE_BATCH_ROWS, MCSE_LEVELS)
+    if draws_k:
+        sam.enable_draws(draws_k)
 
     record = not args.no_chains
     f32 = args.format != "csv" and args.chain_dtype == "f32"
@@ -384,6 +412,23 @@ def run(kind, nbody, argv=None):
     summaries = [dict(image=images[f], walkers=per_frame, updates=sam.count) for f in range(n_frames)]
     es = _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on)
     n_rows = es["rows"]
+    sep_pa_corr = {}                          # (epoch, companion - 1) -> correlation over the draws
+    if draws_k:
+        # every walker's reservoir to rank 0, in global walker order (g = w * n_frames + frame): the files
+        # do not depend on the number of ranks
+        all_v, all_r = _gather_draws(sam.draws(), n_local, rank, world)
+        if rank == 0:
+            col_names = list(layout.names(nbody)) + ["chi2"]
+            for f in range(n_frames):
+                v_f, r_f = all_v[f::n_frames], all_r[f::n_frames]
+                count = chains.write_draws_csv(outdirs[f] + "step2_draws.csv", np.arange(per_frame), v_f, r_f, col_names)
+                summaries[f]["draws"] = {"per_walker": draws_k, "rows_per_walker": n_rows, "count": count,
+                                         "file": "step2_draws.csv"}
+                pooled = torch.from_numpy(v_f[r_f >= 0])
+                for o in range(1, nbody):
+                    sep, pa = stats.separation_pa(pooled, companion=o)
+                    corr = float(np.corrcoef(sep.numpy(), pa.numpy())[0, 1]) if count > 1 else float("nan")
+                    sep_pa_corr[f, o - 1] = corr
     if es["gelman_rubin"] is not None:
         for f in range(n_frames):
             summaries[f]["gelman_rubin"] = es["gelman_rubin"][f]
@@ -404,6 +449,9 @@ def run(kind, nbody, argv=None):
                                "std": float(res["pa_std"][f, o])},
                     "rows": int(res["count"][f, o]), "outside_histogram": float(res["outside"][f, o].max()),
                     "pixscale_mas": float(chains.PIXSCALE_PRE2015)}
+                if (f, o) in sep_pa_corr:
+                    # Pearson correlation of separation and position angle over the epoch's posterior draws
+                    summaries[f]["sep_pa_%s" % nm]["sep_pa_corr"] = sep_pa_corr[f, o]
         if es["bm"] is not None:
             # Monte Carlo error of the means from the batch means (separation scaled to mas like the summary)
             bm = es["bm"]

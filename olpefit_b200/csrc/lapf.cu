@@ -334,6 +334,11 @@ struct RunArgs {
     int64_t bm_q0;               // complete bm_rows-row batches of every walker before this launch
     int bm_rows, bm_phase;       // batch length of level 0; rows recorded since the last level-0 boundary
     int bm_levels, bm_c;
+    // posterior draws (lapf_sampler_draws_enable), or nullptr: a reservoir of dr_k recorded rows per walker
+    double* dr_val;              // [W][dr_k][P+1]
+    int64_t* dr_row;             // [W][dr_k] recorded-row index of the slot, -1: empty
+    int64_t dr_row0;             // rows every walker recorded before this launch
+    int dr_k;
     double* probe;               // self-test only: [rows][W][3] = parameter index, proposed value, TRIAL chi-square
     unsigned long long* cta_times;   // diagnosis only (LAPF_CTA_TIMES): [CTAs][3] = start, end (globaltimer ns), SM id
     int64_t n_walkers;
@@ -459,6 +464,8 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
             ws.k[lane] = dr.k;
             ws.step[lane] = ((a.log_mask >> dr.k) & 1u) ? exp10(wz) : wz;
             ws.lnu[lane] = dr.lnu;
+            // posterior draws: the next 32 updates record at most 32 rows, row .. row + 31; lane l decides row + l
+            if (a.dr_val && tw == 0) ws.dslot[(row + lane) & 31] = draw_slot(a.seed, gid, (uint64_t)(a.dr_row0 + row + lane), a.dr_k);
             __syncwarp();
         }
         const int k = ws.k[slot];                                     // apf_step2.py:302
@@ -558,6 +565,14 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
                 atomicAdd(&a.moments[2 * mi], dl);                    // single writer: plain RED, in order
                 atomicAdd(&a.moments[2 * mi + 1], dl * dl);
                 if (const int n_lev = bm_closing(a, row)) bm_close<NB>(a, wl, lane, n_lev);   // lane c closes column c
+                if (a.dr_val) {                                          // lane c writes column c of the slot
+                    const int j = ws.dslot[row & 31];
+                    if (j >= 0) {
+                        const size_t di = (size_t)wl * a.dr_k + j;
+                        a.dr_val[di * (P + 1) + lane] = v;
+                        if (lane == 0) a.dr_row[di] = a.dr_row0 + row;
+                    }
+                }
             }
             if (a.sk_hist) {
                 double xy[2 * NB];
@@ -802,6 +817,16 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
         if (u == next_rec) {                                              // :342-351
             if (mine) {
                 const bool dense = a.chain && (row == 0 || !a.chain_ev);   // events: row 0 is the key
+                double* dv = nullptr;                                     // posterior draws: the slot this row takes
+                if (a.dr_val) {
+                    const int64_t n = a.dr_row0 + row;
+                    const int jd = draw_slot(a.seed, gid, (uint64_t)n, a.dr_k);
+                    if (jd >= 0) {
+                        const size_t di = (size_t)wl * a.dr_k + jd;
+                        a.dr_row[di] = n;
+                        dv = a.dr_val + di * (P + 1);
+                    }
+                }
 #pragma unroll 1
                 for (int j = 0; j <= P; ++j) {
                     const size_t mi = (size_t)wl * (P + 1) + j;
@@ -811,6 +836,7 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
                         const size_t ci = ((size_t)row * a.n_walkers + wl) * (P + 1) + j;
                         if (a.chain_f32) static_cast<float*>(a.chain)[ci] = (float)dl; else static_cast<double*>(a.chain)[ci] = v;
                     }
+                    if (dv) dv[j] = v;
                     atomicAdd(&a.moments[2 * mi], dl);                    // single writer: plain RED, in order
                     atomicAdd(&a.moments[2 * mi + 1], dl * dl);
                 }
@@ -1346,6 +1372,10 @@ struct lapf_sampler {
     // batch means (lapf_sampler_batchmeans_enable): [W][bm_c][bm_levels][2]
     double* bm = nullptr;
     int bm_rows = 0, bm_levels = 0, bm_c = 0;
+    // posterior draws (lapf_sampler_draws_enable): [W][dr_k][P+1] values, [W][dr_k] row indices
+    double* dr_val = nullptr;
+    int64_t* dr_row = nullptr;
+    int dr_k = 0;
     int chunk = 0;                 // batched kernel: walkers per item at most (warps x walkers per warp)
     int launch_grid = 0;           // batched kernel: CTAs that have work
 };
@@ -1598,6 +1628,7 @@ static void free_sampler(lapf_sampler* s) {
     cudaFree(s->item_frame2); cudaFree(s->item_count_a); cudaFree(s->item_slot_a);
     cudaFree(s->sk_hist); cudaFree(s->sk_center); cudaFree(s->sk_mom);
     cudaFree(s->bm);
+    cudaFree(s->dr_val); cudaFree(s->dr_row);
     delete s;
 }
 
@@ -1760,6 +1791,14 @@ int lapf_sampler_create(const lapf_config* cfg, lapf_sampler** out, void* stream
 static size_t bm_state_bytes(const lapf_sampler* s) {
     return s->bm ? sizeof(double) * (size_t)s->cfg.n_walkers * s->bm_c * s->bm_levels * 2 : 0;
 }
+static size_t draws_val_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.n_walkers * s->dr_k * (s->P + 1); }
+static size_t draws_row_bytes(const lapf_sampler* s) { return sizeof(int64_t) * (size_t)s->cfg.n_walkers * s->dr_k; }
+// An empty reservoir: every row index -1, every value the all-ones NaN
+static int draws_clear(lapf_sampler* s, cudaStream_t st) {
+    CU(cudaMemsetAsync(s->dr_val, 0xFF, draws_val_bytes(s), st));
+    CU(cudaMemsetAsync(s->dr_row, 0xFF, draws_row_bytes(s), st));
+    return LAPF_OK;
+}
 
 int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed, void* stream) {
     if (!s || !init_params) return fail(LAPF_ERR_INVALID, "sampler/init_params is NULL");
@@ -1794,15 +1833,19 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
         }
     }
     if (s->bm) CU(cudaMemsetAsync(s->bm, 0, bm_state_bytes(s), st));
-    return LAPF_OK;
+    return s->dr_val ? draws_clear(s, st) : LAPF_OK;
 }
 
 // Checkpoint layout (device blob, 8-byte units): [count][seed][jump widths x LAPF_MAX_PARAMS] state shift
 // moments(2x) exps tries accepts [sketch sums, sketch histograms] [batch-means descriptor, batch-means state]
+// [draws descriptor, draw values, draw row indices]
 constexpr size_t kCkptHead = 8 * (2 + LAPF_MAX_PARAMS);
 // batch-means descriptor: int64 [magic, batch_rows, levels, C]
 constexpr size_t kCkptBmDesc = 32;
 constexpr int64_t kBmMagic = 0x31304d424650414cLL;   // the bytes 'LAPFBM01'
+// draws descriptor: int64 [magic, K, P+1, 0]
+constexpr size_t kCkptDrDesc = 32;
+constexpr int64_t kDrMagic = 0x313053524650414cLL;   // the bytes 'LAPFRS01'
 static size_t sketch_hist_bytes(const lapf_sampler* s) {
     return s->sk_hist ? sizeof(uint32_t) * (size_t)s->cfg.problem.n_frames * 2 * (s->cfg.problem.nbody - 1) * (s->sk_bins + 2) : 0;
 }
@@ -1813,7 +1856,8 @@ static size_t checkpoint_bytes(const lapf_sampler* s) {
     const size_t W = (size_t)s->cfg.n_walkers, P = (size_t)s->P, nst = W * (P + 1);
     return kCkptHead + sizeof(double) * nst * 4 + sizeof(unsigned long long) * W + sizeof(uint32_t) * W * P * 2 +
            sketch_mom_bytes(s) + sketch_hist_bytes(s) +     // the sketches too, once they are enabled
-           (s->bm ? kCkptBmDesc + bm_state_bytes(s) : 0);   // and the batch means
+           (s->bm ? kCkptBmDesc + bm_state_bytes(s) : 0) +  // and the batch means
+           (s->dr_val ? kCkptDrDesc + draws_val_bytes(s) + draws_row_bytes(s) : 0);   // and the posterior draws
 }
 
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s) {
@@ -1839,12 +1883,27 @@ static int checkpoint_copy(lapf_sampler* s, unsigned char* blob, bool save, cuda
         off += kCkptBmDesc;
         CU(cudaMemcpyAsync(save ? (void*)(blob + off) : (void*)s->bm, save ? (const void*)s->bm : (const void*)(blob + off),
                            bm_state_bytes(s), cudaMemcpyDeviceToDevice, st));
+        off += bm_state_bytes(s);
+    }
+    if (s->dr_val) {
+        off += kCkptDrDesc;   // written or checked by the caller, like the batch-means descriptor
+        const Part dr[] = {{s->dr_val, draws_val_bytes(s)}, {s->dr_row, draws_row_bytes(s)}};
+        for (const Part& p : dr) {
+            CU(cudaMemcpyAsync(save ? (void*)(blob + off) : p.dev, save ? p.dev : (const void*)(blob + off), p.bytes,
+                               cudaMemcpyDeviceToDevice, st));
+            off += p.bytes;
+        }
     }
     return LAPF_OK;
 }
 
-// Offset of the batch-means descriptor in the blob (batch means on)
-static size_t bm_desc_offset(const lapf_sampler* s) { return checkpoint_bytes(s) - bm_state_bytes(s) - kCkptBmDesc; }
+// Offsets of the descriptors in the blob (batch means on; draws on): the draws are the last section
+static size_t dr_desc_offset(const lapf_sampler* s) {
+    return checkpoint_bytes(s) - draws_val_bytes(s) - draws_row_bytes(s) - kCkptDrDesc;
+}
+static size_t bm_desc_offset(const lapf_sampler* s) {
+    return (s->dr_val ? dr_desc_offset(s) : checkpoint_bytes(s)) - bm_state_bytes(s) - kCkptBmDesc;
+}
 
 int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* stream) {
     if (!s || !blob) return fail(LAPF_ERR_INVALID, "sampler/blob is NULL");
@@ -1855,7 +1914,9 @@ int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* str
     CU(cudaMemcpyAsync(blob, head, kCkptHead, cudaMemcpyHostToDevice, st));
     const int64_t desc[4] = {kBmMagic, s->bm_rows, s->bm_levels, s->bm_c};
     if (s->bm) CU(cudaMemcpyAsync((unsigned char*)blob + bm_desc_offset(s), desc, kCkptBmDesc, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));   // `head` and `desc` live on this stack frame
+    const int64_t dr_desc[4] = {kDrMagic, s->dr_k, s->P + 1, 0};
+    if (s->dr_val) CU(cudaMemcpyAsync((unsigned char*)blob + dr_desc_offset(s), dr_desc, kCkptDrDesc, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));   // `head`, `desc` and `dr_desc` live on this stack frame
     return checkpoint_copy(s, (unsigned char*)blob, true, st);
 }
 
@@ -1879,6 +1940,14 @@ int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, voi
             return fail(LAPF_ERR_INVALID, "checkpoint batch means (batch_rows %lld, levels %lld, %lld quantities) do not match "
                         "this sampler's (%d, %d, %d)", (long long)desc[1], (long long)desc[2], (long long)desc[3],
                         s->bm_rows, s->bm_levels, s->bm_c);
+    }
+    if (s->dr_val) {
+        int64_t desc[4] = {0, 0, 0, 0};
+        CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + dr_desc_offset(s), kCkptDrDesc, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (desc[0] != kDrMagic || desc[1] != s->dr_k || desc[2] != s->P + 1 || desc[3] != 0)
+            return fail(LAPF_ERR_INVALID, "checkpoint draws (%lld per walker, %lld columns) do not match this sampler's (%d, %d)",
+                        (long long)desc[1], (long long)desc[2], s->dr_k, s->P + 1);
     }
     s->count = head[0];
     s->cfg.seed = (uint64_t)head[1];
@@ -1964,6 +2033,8 @@ static void fill_run_args(const lapf_sampler* s, RunArgs& a, int64_t n_updates, 
         a.bm_q0 = r0 / s->bm_rows;
         a.bm_phase = (int)(r0 % s->bm_rows);
     }
+    a.dr_val = s->dr_val; a.dr_row = s->dr_row; a.dr_k = s->dr_k;
+    a.dr_row0 = s->dr_val ? rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) : 0;
     a.probe = nullptr;
     a.cta_times = nullptr;
 }
@@ -2096,6 +2167,9 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     // batch means (if on) with batch length 1: every recorded row closes a batch, so the update after each
     // closing row is checked too; the load below restores their state
     a.bm_rows = 1; a.bm_q0 = 0; a.bm_phase = 0;
+    // posterior draws (if on) with one slot per walker: rows 1 and 2 take the replacement path (the slots
+    // [W][1] lie inside the reservoir, which the load below restores)
+    a.dr_k = 1; a.dr_row0 = 0;
     a.probe = probe;
     rc = launch_dispatch(s, a, st);
     if (rc) { cleanup(); return rc; }
@@ -2250,6 +2324,36 @@ int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_o
         CU(cudaGetLastError());
         s->launches++;
     }
+    return LAPF_OK;
+}
+
+int lapf_sampler_draws_enable(lapf_sampler* s, int32_t per_walker, void* stream) {
+    if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
+    if (per_walker < 1 || per_walker > 65536) return fail(LAPF_ERR_INVALID, "draws need per_walker in [1, 65536]");
+    if (s->dr_val) return fail(LAPF_ERR_INVALID, "draws are already enabled");
+    if (rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) > 0)
+        return fail(LAPF_ERR_INVALID, "draws must be enabled before the first recorded row");
+    cudaStream_t st = (cudaStream_t)stream;
+    s->dr_k = per_walker;
+    cudaError_t e = cudaMalloc((void**)&s->dr_val, draws_val_bytes(s));
+    if (e == cudaSuccess) e = cudaMalloc((void**)&s->dr_row, draws_row_bytes(s));
+    int rc = e == cudaSuccess ? draws_clear(s, st)
+                              : fail(LAPF_ERR_CUDA, "cudaMalloc of the draws failed: %s", cudaGetErrorString(e));
+    if (!rc && !getenv("LAPF_NO_SELFTEST")) rc = lapf_sampler_selftest(s, st);
+    if (rc) {
+        cudaStreamSynchronize(st);
+        cudaFree(s->dr_val); cudaFree(s->dr_row);
+        s->dr_val = nullptr; s->dr_row = nullptr; s->dr_k = 0;
+    }
+    return rc;
+}
+
+int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, void* stream) {
+    if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
+    if (!s->dr_val) return fail(LAPF_ERR_INVALID, "draws are not enabled (lapf_sampler_draws_enable)");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (values_out) CU(cudaMemcpyAsync(values_out, s->dr_val, draws_val_bytes(s), cudaMemcpyDeviceToDevice, st));
+    if (rows_out) CU(cudaMemcpyAsync(rows_out, s->dr_row, draws_row_bytes(s), cudaMemcpyDeviceToDevice, st));
     return LAPF_OK;
 }
 

@@ -1339,6 +1339,7 @@ struct WarpScratch {
     double step[32];     // proposal step of update slot i: w*z, or 10^(w*z) for log10 parameters
     double lnu[32];      // log of the accept/reject uniform of update slot i
     int k[32];           // parameter index of update slot i
+    int dslot[32];       // posterior draws: reservoir slot (or -1) of the recorded row r at [r & 31]
     float shape[8];      // sa0 sb0 sc0 - sa1 sb1 sc1 -  of the CURRENT state
     float trig[4];       // sin, cos of theta (narrow), sin, cos of theta2 (wide) of the CURRENT state
 };
@@ -1359,6 +1360,22 @@ __device__ __forceinline__ Draw make_draw(uint64_t seed, uint64_t walker_id, uin
     const double u = (double)m * 0x1p-53;                    // [0, 1)
     d.lnu = log(u);                                          // -inf for u = 0 (probability 2^-53)
     return d;
+}
+
+// Posterior draws (DESIGN.md 4, "Posterior draws"): the reservoir slot that recorded row n of walker
+// walker_id takes among K, or -1 -- algorithm R.  Rows n < K fill slot n; row n >= K replaces slot
+// j = mulhi64(r, n + 1) if j < K, r the 64-bit word of its own Philox stream (tag 'LAPR', so the
+// update stream is untouched).  Integer-only, so the host restates it bit for bit; mulhi64 without
+// rejection favours some j by at most (n + 1) / 2^64.
+constexpr uint32_t kPhiloxTagDraws = 0x4C415052u;   // 'LAPR'
+
+__device__ __forceinline__ int draw_slot(uint64_t seed, uint64_t walker_id, uint64_t n, int K) {
+    if (n < (uint64_t)K) return (int)n;
+    const uint4 r = philox4x32_10(
+        make_uint4((uint32_t)n, (uint32_t)(n >> 32), (uint32_t)(seed >> 32), kPhiloxTagDraws),
+        make_uint2((uint32_t)seed, (uint32_t)walker_id));
+    const uint64_t j = __umul64hi(((uint64_t)r.y << 32) | r.x, n + 1);
+    return j < (uint64_t)K ? (int)j : -1;
 }
 
 }  // namespace lapf

@@ -48,6 +48,7 @@ class GibbsSampler:
         self.events = False
         self._sketch = None
         self._bm = None
+        self._draws = None
         handle = C.c_void_p()
         _lib.check(self.lib.lapf_sampler_create(C.byref(cfg), C.byref(handle), _stream_ptr(dev)))
         self._h = handle
@@ -182,6 +183,25 @@ class GibbsSampler:
         _lib.check(self.lib.lapf_sampler_batchmeans(self._h, walker.data_ptr(), frame.data_ptr(), _stream_ptr(dev)))
         return {"walker": walker, "frame": frame, "batch_rows": batch_rows, "levels": levels,
                 "rows": self.rows_recorded(), "names": names}
+
+    # -- posterior draws: a uniform sample of every walker's recorded rows -----------------------
+    def enable_draws(self, per_walker):
+        """From now on every walker keeps a uniformly random sample of ``per_walker`` of its recorded
+        rows (reservoir sampling on the device, see include/lapf.h).  Call before the first recorded row."""
+        _lib.check(self.lib.lapf_sampler_draws_enable(self._h, int(per_walker), _stream_ptr(self.domain.device)))
+        self._draws = int(per_walker)
+
+    def draws(self):
+        """dict(values [W, K, P+1] float64 (the rows: parameters, chi-square), rows [W, K] int64 (the
+        walker's recorded-row index of each slot, -1: empty) as device tensors, per_walker K, filled
+        = min(K, rows_recorded()): the slots that hold a row)."""
+        if self._draws is None:
+            raise _lib.LapfError("draws are not enabled")
+        dev, k = self.domain.device, self._draws
+        values = torch.empty((self.n_walkers, k, self.nparam + 1), dtype=torch.float64, device=dev)
+        rows = torch.empty((self.n_walkers, k), dtype=torch.int64, device=dev)
+        _lib.check(self.lib.lapf_sampler_draws(self._h, values.data_ptr(), rows.data_ptr(), _stream_ptr(dev)))
+        return {"values": values, "rows": rows, "per_walker": k, "filled": min(k, self.rows_recorded())}
 
     def rows_recorded(self) -> int:
         """Chain rows every walker has recorded since the last reset."""
