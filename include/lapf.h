@@ -150,7 +150,8 @@ int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* str
 int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, void* stream);
 
 /* Replace the jump widths (HOST [P]) for the following runs.  The reference's widths are fixed
- * (apf_step2.py:234); this exists for burn-in-only tuning, which the CLI offers as --adapt. */
+ * (apf_step2.py:234); this exists for burn-in-only tuning, which the CLI offers as --adapt.
+ * LAPF_ERR_INVALID once per-frame widths are on (lapf_sampler_set_frame_widths). */
 int lapf_sampler_set_widths(lapf_sampler* s, const double* widths);
 
 /* Chain rows a run of n_updates starting at the sampler's current count will produce. */
@@ -273,12 +274,42 @@ int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_o
  * 1 <= per_walker <= 65536.  LAPF_ERR_INVALID once any row has been recorded, or if draws are already on.
  * Independent of sketches and batch means, in either order.  Runs lapf_sampler_selftest with the reservoir
  * active and one slot (unless LAPF_NO_SELFTEST), so that self-test rows 1 and 2 replace slot 0, and leaves
- * the sampler as it was.  lapf_sampler_reset empties the reservoir; checkpoints carry it as the last
- * section, behind a 32-byte descriptor (int64 magic 'LAPFRS01', K, P+1, 0) that lapf_sampler_load checks;
- * blobs of samplers without draws keep their layout and size. */
+ * the sampler as it was.  lapf_sampler_reset empties the reservoir; checkpoints carry it after the batch
+ * means (and before the per-frame widths, the last section), behind a 32-byte descriptor (int64 magic
+ * 'LAPFRS01', K, P+1, 0) that lapf_sampler_load checks; blobs of samplers without draws keep their layout
+ * and size. */
 int lapf_sampler_draws_enable(lapf_sampler* s, int32_t per_walker, void* stream);
 /*   values_out device double [W][K][P+1] or NULL; rows_out device int64 [W][K] or NULL */
 int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, void* stream);
+
+/* K4e -- per-frame jump widths, tuned on the device (DESIGN.md, "Per-epoch jump widths").  Epochs differ in
+ * flux, seeing and Strehl, so one width vector cannot suit them all.  Once on, the proposal of a walker of
+ * frame f reads widths[f][k] instead of the batch's widths[k]; widths change only between runs.
+ *   widths  HOST double [F][P], or NULL: the batch widths (lapf_sampler_set_widths / the config) in every row.
+ * The first call allocates the table and an adaptation snapshot (int64 [F][P][2], zero) and runs
+ * lapf_sampler_selftest with the table active (unless LAPF_NO_SELFTEST); later calls replace the widths and
+ * keep the snapshot.  Widths that are negative or not finite give LAPF_ERR_INVALID.  While the table is on,
+ * lapf_sampler_set_widths returns LAPF_ERR_INVALID (one source of truth).  lapf_sampler_reset keeps the
+ * widths and zeroes the snapshot, because the counters start again.  Checkpoints carry the table and the
+ * snapshot as the last section, behind a 32-byte descriptor (int64 magic 'LAPFFW01', F, P, 0) that
+ * lapf_sampler_load checks; a blob with the section is refused by a sampler without the table and the other
+ * way round; blobs of samplers without the table keep their layout and size.  With every row equal to the
+ * batch widths the chains are bit for bit those without the table. */
+int lapf_sampler_set_frame_widths(lapf_sampler* s, const double* widths, void* stream);
+/*   out device double [F][P]: the current table.  LAPF_ERR_INVALID without the table. */
+int lapf_sampler_frame_widths(lapf_sampler* s, double* out, void* stream);
+/* Per-frame acceptance, with or without the table: out device int64 [F][P][2], per frame and parameter the
+ * sum over the frame's walkers of tries and of accepts since the last reset.  Integer sums: exact, in any
+ * order; all-reduce them over ranks. */
+int lapf_sampler_frame_counts(lapf_sampler* s, int64_t* out, void* stream);
+/* One adaptation step from cumulative counts (lapf_sampler_frame_counts, already summed over ranks):
+ * per (f, j), with (T, A) = counts[f][j] and (T', A') = the snapshot, dt = T - T', da = A - A'; if dt > 0,
+ * widths[f][j] *= min(max(exp(da / dt - target), 0.5), 2.0) (the CLI's --adapt rule on the window since
+ * the previous step, per frame; division, subtraction and product rounded to nearest, never fused); a
+ * (f, j) with dt = 0 keeps its width.  Then snapshot = counts.  Stream-ordered, no host synchronisation:
+ * ranks that apply it to the same counts keep the same widths.  LAPF_ERR_INVALID without the table or
+ * unless 0 < target < 1. */
+int lapf_sampler_adapt_widths(lapf_sampler* s, const int64_t* counts, double target, void* stream);
 
 /* Total update count so far (same for every walker). */
 int64_t lapf_sampler_count(const lapf_sampler* s);

@@ -55,6 +55,10 @@ SYMBOLS = {
     "lapf_sampler_batchmeans": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "lapf_sampler_draws_enable": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "lapf_sampler_draws": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lapf_sampler_set_frame_widths": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_void_p]),
+    "lapf_sampler_frame_widths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lapf_sampler_frame_counts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "lapf_sampler_adapt_widths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
     "lapf_frame_outside": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                      C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "lapf_sampler_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

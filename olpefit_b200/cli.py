@@ -98,11 +98,25 @@ def _parser(kind):
                         help="keep a uniformly random sample of K recorded rows of every walker on the device and "
                              "write them to <results>/step2_draws.csv (also with --no-chains); step2_summary.json "
                              "gains the separation-PA correlation of these draws")
+        ap.add_argument("--adapt-per-epoch", action="store_true",
+                        help="give every epoch its own jump widths, tuned on the device DURING BURN-IN ONLY from that "
+                             "epoch's acceptance in windows of at most %d updates (target %.2f); step2_summary.json "
+                             "gains each epoch's widths and its acceptance after burn-in" % (ADAPT_WINDOW, ADAPT_TARGET))
     ap.add_argument("--quiet", action="store_true")
     return ap
 
 
 MCSE_BATCH_ROWS, MCSE_LEVELS = 64, 16
+# --adapt-per-epoch: windows [512 i, 512 (i + 1)) cut at the end of burn-in, and the acceptance they aim for
+# (the constants of --adapt).  The windows are fixed in update counts, so a run resumed from a checkpoint
+# adapts at the same counts as one that was never interrupted.
+ADAPT_WINDOW, ADAPT_TARGET = 512, 0.35
+
+
+def _burn_in(args, kind, nbody):
+    if args.burn_in is not None:
+        return args.burn_in
+    return 6000 if (kind == "step2" and nbody == 2) else 0    # apf_step2.py:38; 3body :38; 2a: SURVEY C3
 
 
 def _epoch_stats(sam, kind, nbody, n_frames, per_frame, n_local, world, bm_on):
@@ -200,6 +214,12 @@ def run(kind, nbody, argv=None):
     draws_k = getattr(args, "draws", None)
     if stop_rule and args.rhat_max is not None and args.walkers < 2:
         raise SystemExit("--rhat-max needs at least 2 walkers per epoch (Gelman-Rubin compares walkers)")
+    burn_in = _burn_in(args, kind, nbody)
+    adapt_pe = getattr(args, "adapt_per_epoch", False)
+    if adapt_pe and args.adapt:
+        raise SystemExit("--adapt-per-epoch and --adapt both tune the jump widths: give one of them")
+    if adapt_pe and burn_in <= 0:
+        raise SystemExit("--adapt-per-epoch tunes the widths during burn-in, and burn-in is 0: give --burn-in")
     import torch
     from . import chains, dist, frame, layout, sampler as smp, stats
 
@@ -230,10 +250,6 @@ def run(kind, nbody, argv=None):
         guess = np.loadtxt(open(chains.initial_guess_path(path), "rb"), delimiter=" ")   # :258-273
         return frame.initial_parameters(image, guess, nbody)
 
-    if args.burn_in is not None:
-        burn_in = args.burn_in
-    else:
-        burn_in = 6000 if (kind == "step2" and nbody == 2) else 0    # apf_step2.py:38; 3body :38; 2a: SURVEY C3
     floor_index = layout.bkgd_index(nbody) if (args.fix_bkgd and nbody == 2) else layout.REFERENCE_FLOOR_INDEX
     dom, params, cuts, headers = frame.load_epochs(images, start_fn, nbody=nbody, size=args.stamp,
                                                    floor_index=floor_index, device=device,
@@ -300,6 +316,14 @@ def run(kind, nbody, argv=None):
         sam.enable_batch_means(MCSE_BATCH_ROWS, MCSE_LEVELS)
     if draws_k:
         sam.enable_draws(draws_k)
+    if adapt_pe:
+        sam.set_frame_widths()                # the default widths in every epoch's row, until burn-in tunes them
+
+    def frame_counts():
+        # per-epoch tries / accepts summed over ranks (a rank without walkers adds zeros); every rank must call it
+        c = sam.frame_counts()
+        return dist.allreduce_sum(c if n_local else torch.zeros_like(c))
+    burn_counts = None                        # frame_counts() at the end of burn-in
 
     record = not args.no_chains
     f32 = args.format != "csv" and args.chain_dtype == "f32"
@@ -330,6 +354,8 @@ def run(kind, nbody, argv=None):
             raise SystemExit("checkpoint %s does not match this run" % ckpt_path)
         sam.load(ck["blob"])
         seed = ck["seed"]
+        if adapt_pe and ck.get("burn_counts") is not None:
+            burn_counts = ck["burn_counts"].to(device)
         first[0] = False                      # append to the chain files that are already there
         say("Resumed at update", sam.count)
     widths, _is_log = layout.default_widths(nbody)
@@ -378,7 +404,15 @@ def run(kind, nbody, argv=None):
                     rate = (accepts.double() / tries.double().clamp(min=1)).cpu().numpy()
                     widths = widths * np.clip(np.exp(rate - 0.35), 0.5, 2.0)
                     sam.set_widths(widths)
+            if adapt_pe and sam.count < burn_in:
+                n = min(n, burn_in - sam.count, ADAPT_WINDOW - sam.count % ADAPT_WINDOW)
             advance(n)
+            if adapt_pe and sam.count <= burn_in and (sam.count % ADAPT_WINDOW == 0 or sam.count == burn_in):
+                # the window that just ended lay in burn-in: every rank applies the same all-reduced counts
+                counts = frame_counts()
+                sam.adapt_widths(counts, ADAPT_TARGET)
+                if sam.count == burn_in:
+                    burn_counts = counts
             if sam.count % (10 * args.segment) < n:
                 say("Loop count:", sam.count, " min tries:", int(mn.item()),
                     " acceptance rate:", (accepts.double() / tries.double().clamp(min=1)).cpu().numpy())
@@ -402,8 +436,10 @@ def run(kind, nbody, argv=None):
     if args.adapt:
         say("Jump widths after burn-in tuning:", widths)
     if args.checkpoint and n_local:
-        torch.save({"blob": sam.save().cpu(), "n_walkers": sam.n_walkers, "nbody": nbody, "seed": seed,
-                    "count": sam.count}, ckpt_path)
+        ck = {"blob": sam.save().cpu(), "n_walkers": sam.n_walkers, "nbody": nbody, "seed": seed, "count": sam.count}
+        if adapt_pe:
+            ck["burn_counts"] = None if burn_counts is None else burn_counts.cpu()
+        torch.save(ck, ckpt_path)
 
     # Summary per epoch from statistics reduced on the device and summed over ranks -- no chain file
     # is read back: Gelman-Rubin per parameter (apf_step3.py:260-278), separation and position angle
@@ -479,6 +515,20 @@ def run(kind, nbody, argv=None):
                     say("epoch %d %s: ESS r %.0f pa %.0f, MCSE r %.4f mas pa %.5f deg  [batches of %s rows]"
                         % (f, nm, s_["sep_mas"]["ess"], s_["pa_deg"]["ess"], s_["sep_mas"]["mcse"],
                            s_["pa_deg"]["mcse"], summaries[f]["batch_rows"]))
+    if adapt_pe:
+        # the widths every epoch ended burn-in with, and its acceptance over the updates after burn-in
+        fw = sam.frame_widths().cpu().numpy()
+        end = frame_counts().cpu().numpy()
+        after = end - burn_counts.cpu().numpy() if burn_counts is not None else np.zeros_like(end)
+        pnames = list(layout.names(nbody))
+        for f in range(n_frames):
+            summaries[f]["widths"] = {nm: float(fw[f, j]) for j, nm in enumerate(pnames)}
+            summaries[f]["acceptance"] = {nm: (float(after[f, j, 1]) / float(after[f, j, 0]) if after[f, j, 0] > 0 else None)
+                                          for j, nm in enumerate(pnames)}
+        for f in range(min(n_frames, 8)):
+            rate = after[f, :, 1] / np.maximum(after[f, :, 0], 1)
+            say("epoch %d: acceptance after burn-in %s, jump widths %s"
+                % (f, np.array2string(rate, precision=3), np.array2string(fw[f], precision=4)))
     if stop_rule or bm_on:
         stop["updates"] = sam.count
         for f in range(n_frames):

@@ -339,6 +339,9 @@ struct RunArgs {
     int64_t* dr_row;             // [W][dr_k] recorded-row index of the slot, -1: empty
     int64_t dr_row0;             // rows every walker recorded before this launch
     int dr_k;
+    // per-frame jump widths (lapf_sampler_set_frame_widths), or nullptr: the proposal of a walker of frame f
+    // reads fwidths[f * P + k] instead of widths[k]
+    const double* fwidths;       // [F][P]
     double* probe;               // self-test only: [rows][W][3] = parameter index, proposed value, TRIAL chi-square
     unsigned long long* cta_times;   // diagnosis only (LAPF_CTA_TIMES): [CTAs][3] = start, end (globaltimer ns), SM id
     int64_t n_walkers;
@@ -459,7 +462,8 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
         if (slot == 0) {
             // lane l prepares the draws of update t0+u+l: 32 updates of random numbers at once
             const Draw dr = make_draw(a.seed, gid, (uint64_t)(a.t0 + u + lane), P);
-            const double wz = __dmul_rn(a.widths[dr.k], dr.z);    // never contracted into the sum below (lapf_device.cuh, set_shape_sc)
+            const double wk = a.fwidths ? a.fwidths[(size_t)frame * P + dr.k] : a.widths[dr.k];   // (uniform branch)
+            const double wz = __dmul_rn(wk, dr.z);    // never contracted into the sum below (lapf_device.cuh, set_shape_sc)
             __syncwarp();
             ws.k[lane] = dr.k;
             ws.step[lane] = ((a.log_mask >> dr.k) & 1u) ? exp10(wz) : wz;
@@ -696,7 +700,9 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
             const double oxd = (double)((two && slot) ? ox1 : ox0), oyd = (double)((two && slot) ? oy1 : oy0);
             k = dr.k;
             lnu = dr.lnu;
-            const double wz = __dmul_rn(a.widths[k], dr.z);
+            // per-frame widths: the lane's frame, picked like its origin (uniform branch)
+            const double wk = a.fwidths ? a.fwidths[(size_t)((two && slot) ? frame1 : frame0) * P + k] : a.widths[k];
+            const double wz = __dmul_rn(wk, dr.z);
             const bool is_log = (a.log_mask >> k) & 1u;
             double v[P];
 #pragma unroll
@@ -1198,6 +1204,46 @@ __global__ void batchmeans_reduce_kernel(const double* __restrict__ bm, const do
     }
 }
 
+// Per-frame acceptance: one CTA per frame, one warp per parameter, over the frame's walkers in the
+// order of moments_kernel.  Integer sums: exact in any order, and ranks may add them.
+__global__ void frame_counts_kernel(const uint32_t* __restrict__ tries, const uint32_t* __restrict__ accepts,
+                                    const int32_t* __restrict__ walker_of, const int32_t* __restrict__ frame_start,
+                                    int P, long long* __restrict__ out /*[F][P][2]*/) {
+    const int f = blockIdx.x, j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (j >= P) return;
+    unsigned long long st = 0, sa = 0;
+    for (int i = frame_start[f] + lane; i < frame_start[f + 1]; i += 32) {
+        const size_t w = (size_t)walker_of[i];
+        st += tries[w * P + j];
+        sa += accepts[w * P + j];
+    }
+    for (int off = 16; off >= 1; off >>= 1) {
+        st += __shfl_xor_sync(kFull, st, off);
+        sa += __shfl_xor_sync(kFull, sa, off);
+    }
+    if (lane == 0) {
+        out[((size_t)f * P + j) * 2] = (long long)st;
+        out[((size_t)f * P + j) * 2 + 1] = (long long)sa;
+    }
+}
+
+// Per-frame width update from the window since the last one (lapf_sampler_adapt_widths): dt = T - T_prev,
+// da = A - A_prev; if dt > 0, w *= min(max(exp(da / dt - target), 0.5), 2); the snapshot becomes the counts.
+// Every operation rounded to nearest and never contracted (DESIGN.md 5): the tests restate it in numpy.
+__global__ void adapt_widths_kernel(const long long* __restrict__ counts, long long* __restrict__ snap,
+                                    double* __restrict__ fw, int n /*F * P*/, double target) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const long long t = counts[2 * i], ac = counts[2 * i + 1];
+    const long long dt = t - snap[2 * i], da = ac - snap[2 * i + 1];
+    if (dt > 0) {
+        const double e = exp(__dsub_rn(__ddiv_rn((double)da, (double)dt), target));
+        fw[i] = __dmul_rn(fw[i], fmin(fmax(e, 0.5), 2.0));
+    }
+    snap[2 * i] = t;
+    snap[2 * i + 1] = ac;
+}
+
 // The same cut-out + mask + noise map with the pixels fetched by the TMA unit: a 3-D tensor map over
 // the frames [F][fy][fx] and one box of kPrepRows x (nx + 4) pixels per CTA (cp.async.bulk.tensor,
 // SASS UTMALDG) -- rows of a cut-out are nx * 4 bytes long and fx * 4 bytes apart, which is exactly
@@ -1376,6 +1422,10 @@ struct lapf_sampler {
     double* dr_val = nullptr;
     int64_t* dr_row = nullptr;
     int dr_k = 0;
+    // per-frame jump widths (lapf_sampler_set_frame_widths): [F][P], and the counts of the last
+    // adaptation [F][P][2] (tries, accepts summed over the frame's walkers and over ranks)
+    double* fw = nullptr;
+    long long* fw_snap = nullptr;
     int chunk = 0;                 // batched kernel: walkers per item at most (warps x walkers per warp)
     int launch_grid = 0;           // batched kernel: CTAs that have work
 };
@@ -1629,6 +1679,7 @@ static void free_sampler(lapf_sampler* s) {
     cudaFree(s->sk_hist); cudaFree(s->sk_center); cudaFree(s->sk_mom);
     cudaFree(s->bm);
     cudaFree(s->dr_val); cudaFree(s->dr_row);
+    cudaFree(s->fw); cudaFree(s->fw_snap);
     delete s;
 }
 
@@ -1793,6 +1844,8 @@ static size_t bm_state_bytes(const lapf_sampler* s) {
 }
 static size_t draws_val_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.n_walkers * s->dr_k * (s->P + 1); }
 static size_t draws_row_bytes(const lapf_sampler* s) { return sizeof(int64_t) * (size_t)s->cfg.n_walkers * s->dr_k; }
+static size_t fw_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.problem.n_frames * s->P; }
+static size_t fw_snap_bytes(const lapf_sampler* s) { return 2 * sizeof(long long) * (size_t)s->cfg.problem.n_frames * s->P; }
 // An empty reservoir: every row index -1, every value the all-ones NaN
 static int draws_clear(lapf_sampler* s, cudaStream_t st) {
     CU(cudaMemsetAsync(s->dr_val, 0xFF, draws_val_bytes(s), st));
@@ -1833,12 +1886,13 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
         }
     }
     if (s->bm) CU(cudaMemsetAsync(s->bm, 0, bm_state_bytes(s), st));
+    if (s->fw) CU(cudaMemsetAsync(s->fw_snap, 0, fw_snap_bytes(s), st));   // the counters start again: so does the window
     return s->dr_val ? draws_clear(s, st) : LAPF_OK;
 }
 
 // Checkpoint layout (device blob, 8-byte units): [count][seed][jump widths x LAPF_MAX_PARAMS] state shift
 // moments(2x) exps tries accepts [sketch sums, sketch histograms] [batch-means descriptor, batch-means state]
-// [draws descriptor, draw values, draw row indices]
+// [draws descriptor, draw values, draw row indices] [frame-widths descriptor, frame widths, adaptation snapshot]
 constexpr size_t kCkptHead = 8 * (2 + LAPF_MAX_PARAMS);
 // batch-means descriptor: int64 [magic, batch_rows, levels, C]
 constexpr size_t kCkptBmDesc = 32;
@@ -1846,6 +1900,9 @@ constexpr int64_t kBmMagic = 0x31304d424650414cLL;   // the bytes 'LAPFBM01'
 // draws descriptor: int64 [magic, K, P+1, 0]
 constexpr size_t kCkptDrDesc = 32;
 constexpr int64_t kDrMagic = 0x313053524650414cLL;   // the bytes 'LAPFRS01'
+// frame-widths descriptor: int64 [magic, F, P, 0]
+constexpr size_t kCkptFwDesc = 32;
+constexpr int64_t kFwMagic = 0x313057464650414cLL;   // the bytes 'LAPFFW01'
 static size_t sketch_hist_bytes(const lapf_sampler* s) {
     return s->sk_hist ? sizeof(uint32_t) * (size_t)s->cfg.problem.n_frames * 2 * (s->cfg.problem.nbody - 1) * (s->sk_bins + 2) : 0;
 }
@@ -1857,7 +1914,8 @@ static size_t checkpoint_bytes(const lapf_sampler* s) {
     return kCkptHead + sizeof(double) * nst * 4 + sizeof(unsigned long long) * W + sizeof(uint32_t) * W * P * 2 +
            sketch_mom_bytes(s) + sketch_hist_bytes(s) +     // the sketches too, once they are enabled
            (s->bm ? kCkptBmDesc + bm_state_bytes(s) : 0) +  // and the batch means
-           (s->dr_val ? kCkptDrDesc + draws_val_bytes(s) + draws_row_bytes(s) : 0);   // and the posterior draws
+           (s->dr_val ? kCkptDrDesc + draws_val_bytes(s) + draws_row_bytes(s) : 0) +  // and the posterior draws
+           (s->fw ? kCkptFwDesc + fw_bytes(s) + fw_snap_bytes(s) : 0);                 // and the per-frame widths
 }
 
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s) {
@@ -1894,15 +1952,27 @@ static int checkpoint_copy(lapf_sampler* s, unsigned char* blob, bool save, cuda
             off += p.bytes;
         }
     }
+    if (s->fw) {
+        off += kCkptFwDesc;   // written or checked by the caller
+        const Part fw[] = {{s->fw, fw_bytes(s)}, {s->fw_snap, fw_snap_bytes(s)}};
+        for (const Part& p : fw) {
+            CU(cudaMemcpyAsync(save ? (void*)(blob + off) : p.dev, save ? p.dev : (const void*)(blob + off), p.bytes,
+                               cudaMemcpyDeviceToDevice, st));
+            off += p.bytes;
+        }
+    }
     return LAPF_OK;
 }
 
-// Offsets of the descriptors in the blob (batch means on; draws on): the draws are the last section
+// Offsets of the descriptors in the blob (batch means on; draws on; frame widths on): the frame widths are the
+// last section
+static size_t fw_section_bytes(const lapf_sampler* s) { return s->fw ? kCkptFwDesc + fw_bytes(s) + fw_snap_bytes(s) : 0; }
+static size_t fw_desc_offset(const lapf_sampler* s) { return checkpoint_bytes(s) - fw_section_bytes(s); }
 static size_t dr_desc_offset(const lapf_sampler* s) {
-    return checkpoint_bytes(s) - draws_val_bytes(s) - draws_row_bytes(s) - kCkptDrDesc;
+    return fw_desc_offset(s) - draws_val_bytes(s) - draws_row_bytes(s) - kCkptDrDesc;
 }
 static size_t bm_desc_offset(const lapf_sampler* s) {
-    return (s->dr_val ? dr_desc_offset(s) : checkpoint_bytes(s)) - bm_state_bytes(s) - kCkptBmDesc;
+    return (s->dr_val ? dr_desc_offset(s) : fw_desc_offset(s)) - bm_state_bytes(s) - kCkptBmDesc;
 }
 
 int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* stream) {
@@ -1916,7 +1986,9 @@ int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* str
     if (s->bm) CU(cudaMemcpyAsync((unsigned char*)blob + bm_desc_offset(s), desc, kCkptBmDesc, cudaMemcpyHostToDevice, st));
     const int64_t dr_desc[4] = {kDrMagic, s->dr_k, s->P + 1, 0};
     if (s->dr_val) CU(cudaMemcpyAsync((unsigned char*)blob + dr_desc_offset(s), dr_desc, kCkptDrDesc, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));   // `head`, `desc` and `dr_desc` live on this stack frame
+    const int64_t fw_desc[4] = {kFwMagic, s->cfg.problem.n_frames, s->P, 0};
+    if (s->fw) CU(cudaMemcpyAsync((unsigned char*)blob + fw_desc_offset(s), fw_desc, kCkptFwDesc, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));   // `head` and the descriptors live on this stack frame
     return checkpoint_copy(s, (unsigned char*)blob, true, st);
 }
 
@@ -1949,6 +2021,23 @@ int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, voi
             return fail(LAPF_ERR_INVALID, "checkpoint draws (%lld per walker, %lld columns) do not match this sampler's (%d, %d)",
                         (long long)desc[1], (long long)desc[2], s->dr_k, s->P + 1);
     }
+    {
+        // with frame widths the descriptor must be there; without them, a blob that carries them is refused
+        // too (its frame-widths section starts where this sampler's blob ends)
+        const size_t at = s->fw ? fw_desc_offset(s) : checkpoint_bytes(s);
+        int64_t desc[4] = {0, 0, 0, 0};
+        if (s->fw || (size_t)blob_bytes >= at + kCkptFwDesc) {
+            CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + at, kCkptFwDesc, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+        }
+        if (!s->fw && desc[0] == kFwMagic)
+            return fail(LAPF_ERR_INVALID, "checkpoint carries per-frame jump widths, this sampler has none "
+                        "(lapf_sampler_set_frame_widths before lapf_sampler_load)");
+        if (s->fw && (desc[0] != kFwMagic || desc[1] != s->cfg.problem.n_frames || desc[2] != s->P || desc[3] != 0))
+            return fail(LAPF_ERR_INVALID, "checkpoint per-frame widths (%lld frames, %lld parameters) do not match this "
+                        "sampler's (%d, %d)", desc[0] == kFwMagic ? (long long)desc[1] : 0LL,
+                        desc[0] == kFwMagic ? (long long)desc[2] : 0LL, s->cfg.problem.n_frames, s->P);
+    }
     s->count = head[0];
     s->cfg.seed = (uint64_t)head[1];
     memcpy(s->widths, wd, sizeof(wd));
@@ -1957,6 +2046,7 @@ int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, voi
 
 int lapf_sampler_set_widths(lapf_sampler* s, const double* widths) {
     if (!s || !widths) return fail(LAPF_ERR_INVALID, "sampler/widths is NULL");
+    if (s->fw) return fail(LAPF_ERR_INVALID, "per-frame jump widths are on: set them with lapf_sampler_set_frame_widths");
     for (int i = 0; i < s->P; ++i)
         if (!(widths[i] >= 0.0)) return fail(LAPF_ERR_INVALID, "widths[%d] = %g is not a valid jump width", i, widths[i]);
     for (int i = 0; i < s->P; ++i) s->widths[i] = widths[i];
@@ -2035,6 +2125,7 @@ static void fill_run_args(const lapf_sampler* s, RunArgs& a, int64_t n_updates, 
     }
     a.dr_val = s->dr_val; a.dr_row = s->dr_row; a.dr_k = s->dr_k;
     a.dr_row0 = s->dr_val ? rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) : 0;
+    a.fwidths = s->fw;
     a.probe = nullptr;
     a.cta_times = nullptr;
 }
@@ -2354,6 +2445,68 @@ int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, v
     cudaStream_t st = (cudaStream_t)stream;
     if (values_out) CU(cudaMemcpyAsync(values_out, s->dr_val, draws_val_bytes(s), cudaMemcpyDeviceToDevice, st));
     if (rows_out) CU(cudaMemcpyAsync(rows_out, s->dr_row, draws_row_bytes(s), cudaMemcpyDeviceToDevice, st));
+    return LAPF_OK;
+}
+
+int lapf_sampler_set_frame_widths(lapf_sampler* s, const double* widths, void* stream) {
+    if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
+    const int F = s->cfg.problem.n_frames, P = s->P;
+    std::vector<double> h((size_t)F * P);
+    for (int f = 0; f < F; ++f)
+        for (int j = 0; j < P; ++j) {
+            const double v = widths ? widths[(size_t)f * P + j] : s->widths[j];
+            if (!(v >= 0.0) || !std::isfinite(v))
+                return fail(LAPF_ERR_INVALID, "widths[%d][%d] = %g is not a valid jump width", f, j, v);
+            h[(size_t)f * P + j] = v;
+        }
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool first = s->fw == nullptr;
+    if (first) {
+        cudaError_t e = cudaMalloc((void**)&s->fw, fw_bytes(s));
+        if (e == cudaSuccess) e = cudaMalloc((void**)&s->fw_snap, fw_snap_bytes(s));
+        if (e == cudaSuccess) e = cudaMemsetAsync(s->fw_snap, 0, fw_snap_bytes(s), st);
+        if (e != cudaSuccess) {
+            cudaFree(s->fw); cudaFree(s->fw_snap);
+            s->fw = nullptr; s->fw_snap = nullptr;
+            return fail(LAPF_ERR_CUDA, "allocation of the per-frame widths failed: %s", cudaGetErrorString(e));
+        }
+    }
+    CU(cudaMemcpyAsync(s->fw, h.data(), fw_bytes(s), cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));   // `h` is pageable and lives on this stack frame
+    int rc = LAPF_OK;
+    if (first && !getenv("LAPF_NO_SELFTEST") && (rc = lapf_sampler_selftest(s, st))) {
+        cudaStreamSynchronize(st);
+        cudaFree(s->fw); cudaFree(s->fw_snap);
+        s->fw = nullptr; s->fw_snap = nullptr;
+    }
+    return rc;
+}
+
+int lapf_sampler_frame_widths(lapf_sampler* s, double* out, void* stream) {
+    if (!s || !out) return fail(LAPF_ERR_INVALID, "sampler/out is NULL");
+    if (!s->fw) return fail(LAPF_ERR_INVALID, "per-frame widths are not on (lapf_sampler_set_frame_widths)");
+    CU(cudaMemcpyAsync(out, s->fw, fw_bytes(s), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return LAPF_OK;
+}
+
+int lapf_sampler_frame_counts(lapf_sampler* s, int64_t* out, void* stream) {
+    if (!s || !out) return fail(LAPF_ERR_INVALID, "sampler/out is NULL");
+    frame_counts_kernel<<<s->cfg.problem.n_frames, 32 * s->P, 0, (cudaStream_t)stream>>>(
+        s->tries, s->accepts, s->walker_of, s->frame_start, s->P, (long long*)out);
+    CU(cudaGetLastError());
+    s->launches++;
+    return LAPF_OK;
+}
+
+int lapf_sampler_adapt_widths(lapf_sampler* s, const int64_t* counts, double target, void* stream) {
+    if (!s || !counts) return fail(LAPF_ERR_INVALID, "sampler/counts is NULL");
+    if (!s->fw) return fail(LAPF_ERR_INVALID, "per-frame widths are not on (lapf_sampler_set_frame_widths)");
+    if (!(target > 0.0 && target < 1.0)) return fail(LAPF_ERR_INVALID, "target acceptance %g is not in (0, 1)", target);
+    const int n = s->cfg.problem.n_frames * s->P;
+    adapt_widths_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>((const long long*)counts, s->fw_snap, s->fw, n,
+                                                                           target);
+    CU(cudaGetLastError());
+    s->launches++;
     return LAPF_OK;
 }
 

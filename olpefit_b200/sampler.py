@@ -203,6 +203,44 @@ class GibbsSampler:
         _lib.check(self.lib.lapf_sampler_draws(self._h, values.data_ptr(), rows.data_ptr(), _stream_ptr(dev)))
         return {"values": values, "rows": rows, "per_walker": k, "filled": min(k, self.rows_recorded())}
 
+    # -- per-epoch jump widths, tuned on the device ----------------------------------------------
+    def set_frame_widths(self, widths=None):
+        """From now on the walkers of frame f propose with the jump widths of row f: ``widths`` [F, P]
+        (host values), or None for the batch widths in every row.  The first call turns the table on;
+        ``set_widths`` is then refused.  See include/lapf.h."""
+        nf = self.domain.n_frames
+        w_arr = None
+        if widths is not None:
+            w_np = np.ascontiguousarray(widths.cpu().numpy() if torch.is_tensor(widths) else widths, dtype=np.float64)
+            if w_np.shape != (nf, self.nparam):
+                raise ValueError("widths must be [%d, %d]" % (nf, self.nparam))
+            w_arr = (C.c_double * w_np.size)(*w_np.reshape(-1).tolist())
+        _lib.check(self.lib.lapf_sampler_set_frame_widths(self._h, w_arr, _stream_ptr(self.domain.device)))
+
+    def frame_widths(self):
+        """[F, P] float64 device tensor: the per-frame jump widths."""
+        dev = self.domain.device
+        out = torch.empty((self.domain.n_frames, self.nparam), dtype=torch.float64, device=dev)
+        _lib.check(self.lib.lapf_sampler_frame_widths(self._h, out.data_ptr(), _stream_ptr(dev)))
+        return out
+
+    def frame_counts(self):
+        """[F, P, 2] int64 device tensor: per frame and parameter, the tries and accepts of the frame's
+        walkers since the last reset (exact integer sums: all-reduce them over ranks)."""
+        dev = self.domain.device
+        out = torch.empty((self.domain.n_frames, self.nparam, 2), dtype=torch.int64, device=dev)
+        _lib.check(self.lib.lapf_sampler_frame_counts(self._h, out.data_ptr(), _stream_ptr(dev)))
+        return out
+
+    def adapt_widths(self, counts, target=0.35):
+        """One adaptation step of the per-frame widths from cumulative ``frame_counts()`` (summed over
+        ranks): each width is scaled by exp(rate - target), clipped to [0.5, 2], where rate is the
+        acceptance over the window since the previous step; on the device, without a host sync."""
+        c = counts.to(self.domain.device, torch.int64).contiguous()
+        if tuple(c.shape) != (self.domain.n_frames, self.nparam, 2):
+            raise ValueError("counts must be [%d, %d, 2]" % (self.domain.n_frames, self.nparam))
+        _lib.check(self.lib.lapf_sampler_adapt_widths(self._h, c.data_ptr(), float(target), _stream_ptr(self.domain.device)))
+
     def rows_recorded(self) -> int:
         """Chain rows every walker has recorded since the last reset."""
         n = self.count
