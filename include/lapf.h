@@ -142,9 +142,24 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
  * its random stream is a pure function of (seed, walker id, update count), so a saved blob restores
  * the batch exactly: run(a); save; ...; load; run(b) gives the bits of run(a+b).  The blob is a
  * device buffer of lapf_sampler_checkpoint_bytes() bytes owned by the caller; load() expects a
- * sampler created with the same shape (walkers, model, frame_of) and, if the sketches below are in
- * use, with them enabled the same way before either call (they travel in the blob).  The reference's only resume
- * point is the chain file / step2a.csv (apf_step2.py:248-256). */
+ * sampler created with the same shape (walkers, model, frame_of) and with the same optional state
+ * below enabled the same way before either call (it travels in the blob).  The reference's only resume
+ * point is the chain file / step2a.csv (apf_step2.py:248-256).
+ *
+ * Layout: a head, then one section per kind of state, in this order; a section that is off is absent.
+ * A descriptor is 32 bytes, int64 {magic, a, b, c}.
+ *   head                  int64 count, int64 seed, double jump widths [LAPF_MAX_PARAMS]
+ *   core                  state, shift (lapf_sampler_start), moments, exps, tries, accepts
+ *   sketches, if on       no descriptor; walker sums, histograms
+ *   batch means, if on    {'LAPFBM01', batch_rows, levels, C}; walker state
+ *   draws, if on          {'LAPFRS01', K, P+1, 0}; values, row indices
+ *   frame widths, if on   {'LAPFFW01', F, P, 0}; widths, adaptation snapshot
+ * load() refuses a blob (LAPF_ERR_INVALID, the sampler unchanged) that is smaller than this sampler's
+ * layout, whose head is corrupt, that lacks a descriptor this sampler expects or differs in one, or
+ * whose bytes just past this sampler's layout start with a known magic (a section this sampler does
+ * not have).  So a blob loads only into a sampler with the same batch means, draws and frame widths.
+ * The sketch section has no descriptor: a blob whose sketch setting differs from the sampler's is
+ * refused only when that shifts a later descriptor or the blob is too small. */
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s);
 int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* stream);
 int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, void* stream);
@@ -251,8 +266,8 @@ int lapf_sampler_sketch(lapf_sampler* s, uint32_t* hist_out, double* summary_out
  * (1 <= batch_rows <= 2^30, 1 <= levels <= 24).  LAPF_ERR_INVALID once any row has been recorded.  Runs
  * lapf_sampler_selftest with the batch means active (unless LAPF_NO_SELFTEST) and leaves the sampler as
  * it was.  Once they are on, lapf_sampler_sketch_enable returns LAPF_ERR_INVALID (C would change);
- * lapf_sampler_reset zeroes them; checkpoints carry them after the sketch sections, behind a 32-byte
- * descriptor (int64 magic, batch_rows, levels, C) that lapf_sampler_load checks against the sampler. */
+ * lapf_sampler_reset zeroes them; checkpoints carry them (see lapf_sampler_save for the layout and the
+ * load rule). */
 int lapf_sampler_batchmeans_enable(lapf_sampler* s, int32_t batch_rows, int32_t levels, void* stream);
 /*   walker_out device double [W][C][levels][2] (snap, s2) or NULL
  *   frame_out  device double [F][C][1 + levels] or NULL: [0] sum over the frame's walkers of the
@@ -274,10 +289,8 @@ int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_o
  * 1 <= per_walker <= 65536.  LAPF_ERR_INVALID once any row has been recorded, or if draws are already on.
  * Independent of sketches and batch means, in either order.  Runs lapf_sampler_selftest with the reservoir
  * active and one slot (unless LAPF_NO_SELFTEST), so that self-test rows 1 and 2 replace slot 0, and leaves
- * the sampler as it was.  lapf_sampler_reset empties the reservoir; checkpoints carry it after the batch
- * means (and before the per-frame widths, the last section), behind a 32-byte descriptor (int64 magic
- * 'LAPFRS01', K, P+1, 0) that lapf_sampler_load checks; blobs of samplers without draws keep their layout
- * and size. */
+ * the sampler as it was.  lapf_sampler_reset empties the reservoir; checkpoints carry it (see
+ * lapf_sampler_save for the layout and the load rule). */
 int lapf_sampler_draws_enable(lapf_sampler* s, int32_t per_walker, void* stream);
 /*   values_out device double [W][K][P+1] or NULL; rows_out device int64 [W][K] or NULL */
 int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, void* stream);
@@ -291,10 +304,8 @@ int lapf_sampler_draws(lapf_sampler* s, double* values_out, int64_t* rows_out, v
  * keep the snapshot.  Widths that are negative or not finite give LAPF_ERR_INVALID.  While the table is on,
  * lapf_sampler_set_widths returns LAPF_ERR_INVALID (one source of truth).  lapf_sampler_reset keeps the
  * widths and zeroes the snapshot, because the counters start again.  Checkpoints carry the table and the
- * snapshot as the last section, behind a 32-byte descriptor (int64 magic 'LAPFFW01', F, P, 0) that
- * lapf_sampler_load checks; a blob with the section is refused by a sampler without the table and the other
- * way round; blobs of samplers without the table keep their layout and size.  With every row equal to the
- * batch widths the chains are bit for bit those without the table. */
+ * snapshot (see lapf_sampler_save for the layout and the load rule).  With every row equal to the batch
+ * widths the chains are bit for bit those without the table. */
 int lapf_sampler_set_frame_widths(lapf_sampler* s, const double* widths, void* stream);
 /*   out device double [F][P]: the current table.  LAPF_ERR_INVALID without the table. */
 int lapf_sampler_frame_widths(lapf_sampler* s, double* out, void* stream);

@@ -82,7 +82,8 @@ def _parser(kind):
     ap.add_argument("--checkpoint", action="store_true",
                     help="write <results>/checkpoint_rank<r>.pt when done (exact state of every walker)")
     ap.add_argument("--resume", action="store_true",
-                    help="continue from <results>/checkpoint_rank<r>.pt, appending to the existing chain files")
+                    help="continue from <results>/checkpoint_rank<r>.pt, appending to the existing chain files "
+                         "(give the --mcse / --ess-min, --draws and --adapt-per-epoch of the run that wrote it)")
     if kind != "step2a":
         ap.add_argument("--mcse", action="store_true",
                         help="keep batch means of every recorded value on the device: step2_summary.json gains the "

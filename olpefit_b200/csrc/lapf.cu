@@ -17,6 +17,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <limits>
 #include <new>
 #include <string>
@@ -1839,18 +1840,80 @@ int lapf_sampler_create(const lapf_config* cfg, lapf_sampler** out, void* stream
     return LAPF_OK;
 }
 
+static size_t sketch_hist_bytes(const lapf_sampler* s) {
+    return sizeof(uint32_t) * (size_t)s->cfg.problem.n_frames * 2 * (s->cfg.problem.nbody - 1) * (s->sk_bins + 2);
+}
+static size_t sketch_mom_bytes(const lapf_sampler* s) {
+    return sizeof(double) * (size_t)s->cfg.n_walkers * 2 * (s->cfg.problem.nbody - 1) * 2;
+}
 static size_t bm_state_bytes(const lapf_sampler* s) {
-    return s->bm ? sizeof(double) * (size_t)s->cfg.n_walkers * s->bm_c * s->bm_levels * 2 : 0;
+    return sizeof(double) * (size_t)s->cfg.n_walkers * s->bm_c * s->bm_levels * 2;
 }
 static size_t draws_val_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.n_walkers * s->dr_k * (s->P + 1); }
 static size_t draws_row_bytes(const lapf_sampler* s) { return sizeof(int64_t) * (size_t)s->cfg.n_walkers * s->dr_k; }
 static size_t fw_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.problem.n_frames * s->P; }
 static size_t fw_snap_bytes(const lapf_sampler* s) { return 2 * sizeof(long long) * (size_t)s->cfg.problem.n_frames * s->P; }
-// An empty reservoir: every row index -1, every value the all-ones NaN
-static int draws_clear(lapf_sampler* s, cudaStream_t st) {
-    CU(cudaMemsetAsync(s->dr_val, 0xFF, draws_val_bytes(s), st));
-    CU(cudaMemsetAsync(s->dr_row, 0xFF, draws_row_bytes(s), st));
-    return LAPF_OK;
+
+// Checkpoint layout: see lapf_sampler_save in lapf.h.  The head [count][seed][jump widths x LAPF_MAX_PARAMS] is
+// built on the host; checkpoint_layout lists the sections that follow it, and every size, offset, copy, reset
+// fill and load check is derived from that list.
+constexpr size_t kCkptHead = 8 * (2 + LAPF_MAX_PARAMS);
+constexpr size_t kCkptDesc = 32;   // int64 {magic, a, b, c}
+constexpr int kKeep = -1;          // a part lapf_sampler_reset does not overwrite
+// A device buffer of the sampler (the address of the field that owns it), its size and the byte that
+// lapf_sampler_reset writes over it (or kKeep)
+struct Part { void** dev; size_t bytes; int fill; };
+// The sections that start with a descriptor; its magic identifies the section in any blob
+struct Described { int64_t magic; const char* name; const char* fields; const char* enable; };
+static const Described kBatchMeans = {0x31304d424650414cLL, "batch means", "batch_rows, levels, quantities",   // 'LAPFBM01'
+                                      "lapf_sampler_batchmeans_enable"};
+static const Described kDraws = {0x313053524650414cLL, "posterior draws", "per walker, columns, 0",            // 'LAPFRS01'
+                                  "lapf_sampler_draws_enable"};
+static const Described kFrameWidths = {0x313057464650414cLL, "per-frame jump widths", "frames, parameters, 0", // 'LAPFFW01'
+                                       "lapf_sampler_set_frame_widths"};
+static const Described* const kDescribed[] = {&kBatchMeans, &kDraws, &kFrameWidths};
+struct Section {
+    const Described* desc;   // nullptr: no descriptor
+    int64_t val[3];          // the descriptor's a, b, c
+    int n_parts;
+    Part part[6];
+    size_t at;               // offset in the blob (of the descriptor, if any)
+};
+constexpr int kSections = 5;   // core, sketches, batch means, draws, per-frame widths
+struct CkptLayout { int n; Section sec[kSections]; size_t bytes; };
+
+static CkptLayout checkpoint_layout(lapf_sampler* s) {
+    const size_t W = (size_t)s->cfg.n_walkers, P = (size_t)s->P, nst = W * (P + 1);
+    CkptLayout L = {};
+    L.sec[L.n++] = {nullptr, {}, 6, {{(void**)&s->state, sizeof(double) * nst, kKeep},   // pack_state_kernel in reset
+                                     {(void**)&s->shift, sizeof(double) * nst, kKeep},
+                                     {(void**)&s->moments, sizeof(double) * nst * 2, 0},
+                                     {(void**)&s->exps, sizeof(unsigned long long) * W, 0},
+                                     {(void**)&s->tries, sizeof(uint32_t) * W * P, 0},
+                                     {(void**)&s->accepts, sizeof(uint32_t) * W * P, 0}}};
+    if (s->sk_hist)
+        L.sec[L.n++] = {nullptr, {}, 2, {{(void**)&s->sk_mom, sketch_mom_bytes(s), 0},
+                                         {(void**)&s->sk_hist, sketch_hist_bytes(s), 0}}};
+    if (s->bm)
+        L.sec[L.n++] = {&kBatchMeans, {s->bm_rows, s->bm_levels, s->bm_c}, 1, {{(void**)&s->bm, bm_state_bytes(s), 0}}};
+    if (s->dr_val)   // an empty reservoir: every row index -1, every value the all-ones NaN
+        L.sec[L.n++] = {&kDraws, {s->dr_k, s->P + 1, 0}, 2, {{(void**)&s->dr_val, draws_val_bytes(s), 0xFF},
+                                                              {(void**)&s->dr_row, draws_row_bytes(s), 0xFF}}};
+    if (s->fw)       // reset keeps the widths; the counters start again, so does the adaptation window
+        L.sec[L.n++] = {&kFrameWidths, {s->cfg.problem.n_frames, s->P, 0}, 2,
+                        {{(void**)&s->fw, fw_bytes(s), kKeep}, {(void**)&s->fw_snap, fw_snap_bytes(s), 0}}};
+    L.bytes = kCkptHead;
+    for (int i = 0; i < L.n; ++i) {
+        Section& c = L.sec[i];
+        c.at = L.bytes;
+        L.bytes += c.desc ? kCkptDesc : 0;
+        for (int j = 0; j < c.n_parts; ++j) L.bytes += c.part[j].bytes;
+    }
+    return L;
+}
+
+static size_t checkpoint_bytes(const lapf_sampler* s) {
+    return checkpoint_layout(const_cast<lapf_sampler*>(s)).bytes;   // reads sizes only
 }
 
 int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed, void* stream) {
@@ -1859,10 +1922,12 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
     const int P = s->P;
     const int64_t W = s->cfg.n_walkers;
     const size_t nst = (size_t)W * (P + 1);
-    CU(cudaMemsetAsync(s->moments, 0, sizeof(double) * nst * 2, st));
-    CU(cudaMemsetAsync(s->tries, 0, sizeof(uint32_t) * W * P, st));
-    CU(cudaMemsetAsync(s->accepts, 0, sizeof(uint32_t) * W * P, st));
-    CU(cudaMemsetAsync(s->exps, 0, sizeof(unsigned long long) * W, st));
+    const CkptLayout L = checkpoint_layout(s);
+    for (int i = 0; i < L.n; ++i)
+        for (int j = 0; j < L.sec[i].n_parts; ++j) {
+            const Part& p = L.sec[i].part[j];
+            if (p.fill != kKeep) CU(cudaMemsetAsync(*p.dev, p.fill, p.bytes, st));
+        }
     // initial chi-square (apf_step2.py:283-289) through K1, then pack the state
     double* chi0 = nullptr;
     CU(cudaMallocAsync((void**)&chi0, sizeof(double) * W, st));
@@ -1874,48 +1939,14 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
     s->launches += 2;
     s->cfg.seed = seed;
     s->count = 0;
-    if (s->sk_hist) {
-        const int F = s->cfg.problem.n_frames, slots = 2 * (s->cfg.problem.nbody - 1);
-        CU(cudaMemsetAsync(s->sk_hist, 0, sizeof(uint32_t) * (size_t)F * slots * (s->sk_bins + 2), st));
-        CU(cudaMemsetAsync(s->sk_mom, 0, sizeof(double) * (size_t)W * slots * 2, st));
-        if (s->sk_auto_center) {
-            sketch_center_kernel<<<(F * (slots / 2) + 127) / 128, 128, 0, st>>>(s->shift, s->walker_of, s->frame_start, F, P,
-                                                                              s->cfg.problem.nbody, s->sk_center);
-            CU(cudaGetLastError());
-            s->launches++;
-        }
+    if (s->sk_hist && s->sk_auto_center) {
+        const int F = s->cfg.problem.n_frames, nbody = s->cfg.problem.nbody;
+        sketch_center_kernel<<<(F * (nbody - 1) + 127) / 128, 128, 0, st>>>(s->shift, s->walker_of, s->frame_start, F, P,
+                                                                          nbody, s->sk_center);
+        CU(cudaGetLastError());
+        s->launches++;
     }
-    if (s->bm) CU(cudaMemsetAsync(s->bm, 0, bm_state_bytes(s), st));
-    if (s->fw) CU(cudaMemsetAsync(s->fw_snap, 0, fw_snap_bytes(s), st));   // the counters start again: so does the window
-    return s->dr_val ? draws_clear(s, st) : LAPF_OK;
-}
-
-// Checkpoint layout (device blob, 8-byte units): [count][seed][jump widths x LAPF_MAX_PARAMS] state shift
-// moments(2x) exps tries accepts [sketch sums, sketch histograms] [batch-means descriptor, batch-means state]
-// [draws descriptor, draw values, draw row indices] [frame-widths descriptor, frame widths, adaptation snapshot]
-constexpr size_t kCkptHead = 8 * (2 + LAPF_MAX_PARAMS);
-// batch-means descriptor: int64 [magic, batch_rows, levels, C]
-constexpr size_t kCkptBmDesc = 32;
-constexpr int64_t kBmMagic = 0x31304d424650414cLL;   // the bytes 'LAPFBM01'
-// draws descriptor: int64 [magic, K, P+1, 0]
-constexpr size_t kCkptDrDesc = 32;
-constexpr int64_t kDrMagic = 0x313053524650414cLL;   // the bytes 'LAPFRS01'
-// frame-widths descriptor: int64 [magic, F, P, 0]
-constexpr size_t kCkptFwDesc = 32;
-constexpr int64_t kFwMagic = 0x313057464650414cLL;   // the bytes 'LAPFFW01'
-static size_t sketch_hist_bytes(const lapf_sampler* s) {
-    return s->sk_hist ? sizeof(uint32_t) * (size_t)s->cfg.problem.n_frames * 2 * (s->cfg.problem.nbody - 1) * (s->sk_bins + 2) : 0;
-}
-static size_t sketch_mom_bytes(const lapf_sampler* s) {
-    return s->sk_hist ? sizeof(double) * (size_t)s->cfg.n_walkers * 2 * (s->cfg.problem.nbody - 1) * 2 : 0;
-}
-static size_t checkpoint_bytes(const lapf_sampler* s) {
-    const size_t W = (size_t)s->cfg.n_walkers, P = (size_t)s->P, nst = W * (P + 1);
-    return kCkptHead + sizeof(double) * nst * 4 + sizeof(unsigned long long) * W + sizeof(uint32_t) * W * P * 2 +
-           sketch_mom_bytes(s) + sketch_hist_bytes(s) +     // the sketches too, once they are enabled
-           (s->bm ? kCkptBmDesc + bm_state_bytes(s) : 0) +  // and the batch means
-           (s->dr_val ? kCkptDrDesc + draws_val_bytes(s) + draws_row_bytes(s) : 0) +  // and the posterior draws
-           (s->fw ? kCkptFwDesc + fw_bytes(s) + fw_snap_bytes(s) : 0);                 // and the per-frame widths
+    return LAPF_OK;
 }
 
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s) {
@@ -1923,40 +1954,14 @@ int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s) {
     return (int64_t)checkpoint_bytes(s);
 }
 
-static int checkpoint_copy(lapf_sampler* s, unsigned char* blob, bool save, cudaStream_t st) {
-    const size_t W = (size_t)s->cfg.n_walkers, P = (size_t)s->P, nst = W * (P + 1);
-    struct Part { void* dev; size_t bytes; } parts[] = {
-        {s->state, sizeof(double) * nst}, {s->shift, sizeof(double) * nst}, {s->moments, sizeof(double) * nst * 2},
-        {s->exps, sizeof(unsigned long long) * W}, {s->tries, sizeof(uint32_t) * W * P}, {s->accepts, sizeof(uint32_t) * W * P},
-        {s->sk_mom, sketch_mom_bytes(s)}, {s->sk_hist, sketch_hist_bytes(s)}};
-    size_t off = kCkptHead;
-    for (const Part& p : parts) {
-        if (!p.bytes) continue;
-        CU(cudaMemcpyAsync(save ? (void*)(blob + off) : p.dev, save ? p.dev : (const void*)(blob + off), p.bytes,
-                           cudaMemcpyDeviceToDevice, st));
-        off += p.bytes;
-    }
-    if (s->bm) {
-        // the descriptor was written (save) or checked (load) by the caller
-        off += kCkptBmDesc;
-        CU(cudaMemcpyAsync(save ? (void*)(blob + off) : (void*)s->bm, save ? (const void*)s->bm : (const void*)(blob + off),
-                           bm_state_bytes(s), cudaMemcpyDeviceToDevice, st));
-        off += bm_state_bytes(s);
-    }
-    if (s->dr_val) {
-        off += kCkptDrDesc;   // written or checked by the caller, like the batch-means descriptor
-        const Part dr[] = {{s->dr_val, draws_val_bytes(s)}, {s->dr_row, draws_row_bytes(s)}};
-        for (const Part& p : dr) {
-            CU(cudaMemcpyAsync(save ? (void*)(blob + off) : p.dev, save ? p.dev : (const void*)(blob + off), p.bytes,
-                               cudaMemcpyDeviceToDevice, st));
-            off += p.bytes;
-        }
-    }
-    if (s->fw) {
-        off += kCkptFwDesc;   // written or checked by the caller
-        const Part fw[] = {{s->fw, fw_bytes(s)}, {s->fw_snap, fw_snap_bytes(s)}};
-        for (const Part& p : fw) {
-            CU(cudaMemcpyAsync(save ? (void*)(blob + off) : p.dev, save ? p.dev : (const void*)(blob + off), p.bytes,
+// Copies every part between the sampler and the blob; the descriptors are written (save) or checked (load) by
+// the caller
+static int checkpoint_copy(const CkptLayout& L, unsigned char* blob, bool save, cudaStream_t st) {
+    for (int i = 0; i < L.n; ++i) {
+        size_t off = L.sec[i].at + (L.sec[i].desc ? kCkptDesc : 0);
+        for (int j = 0; j < L.sec[i].n_parts; ++j) {
+            const Part& p = L.sec[i].part[j];
+            CU(cudaMemcpyAsync(save ? (void*)(blob + off) : *p.dev, save ? *p.dev : (const void*)(blob + off), p.bytes,
                                cudaMemcpyDeviceToDevice, st));
             off += p.bytes;
         }
@@ -1964,84 +1969,74 @@ static int checkpoint_copy(lapf_sampler* s, unsigned char* blob, bool save, cuda
     return LAPF_OK;
 }
 
-// Offsets of the descriptors in the blob (batch means on; draws on; frame widths on): the frame widths are the
-// last section
-static size_t fw_section_bytes(const lapf_sampler* s) { return s->fw ? kCkptFwDesc + fw_bytes(s) + fw_snap_bytes(s) : 0; }
-static size_t fw_desc_offset(const lapf_sampler* s) { return checkpoint_bytes(s) - fw_section_bytes(s); }
-static size_t dr_desc_offset(const lapf_sampler* s) {
-    return fw_desc_offset(s) - draws_val_bytes(s) - draws_row_bytes(s) - kCkptDrDesc;
-}
-static size_t bm_desc_offset(const lapf_sampler* s) {
-    return (s->dr_val ? dr_desc_offset(s) : fw_desc_offset(s)) - bm_state_bytes(s) - kCkptBmDesc;
-}
-
 int lapf_sampler_save(lapf_sampler* s, void* blob, int64_t blob_bytes, void* stream) {
     if (!s || !blob) return fail(LAPF_ERR_INVALID, "sampler/blob is NULL");
-    if ((size_t)blob_bytes < checkpoint_bytes(s)) return fail(LAPF_ERR_INVALID, "checkpoint buffer too small");
+    const CkptLayout L = checkpoint_layout(s);
+    if ((size_t)blob_bytes < L.bytes) return fail(LAPF_ERR_INVALID, "checkpoint buffer too small");
     cudaStream_t st = (cudaStream_t)stream;
     int64_t head[2 + LAPF_MAX_PARAMS] = {s->count, (int64_t)s->cfg.seed};
     memcpy(head + 2, s->widths, sizeof(double) * LAPF_MAX_PARAMS);   // --adapt may have changed them
     CU(cudaMemcpyAsync(blob, head, kCkptHead, cudaMemcpyHostToDevice, st));
-    const int64_t desc[4] = {kBmMagic, s->bm_rows, s->bm_levels, s->bm_c};
-    if (s->bm) CU(cudaMemcpyAsync((unsigned char*)blob + bm_desc_offset(s), desc, kCkptBmDesc, cudaMemcpyHostToDevice, st));
-    const int64_t dr_desc[4] = {kDrMagic, s->dr_k, s->P + 1, 0};
-    if (s->dr_val) CU(cudaMemcpyAsync((unsigned char*)blob + dr_desc_offset(s), dr_desc, kCkptDrDesc, cudaMemcpyHostToDevice, st));
-    const int64_t fw_desc[4] = {kFwMagic, s->cfg.problem.n_frames, s->P, 0};
-    if (s->fw) CU(cudaMemcpyAsync((unsigned char*)blob + fw_desc_offset(s), fw_desc, kCkptFwDesc, cudaMemcpyHostToDevice, st));
+    int64_t desc[kSections][4];
+    for (int i = 0; i < L.n; ++i) {
+        const Section& c = L.sec[i];
+        if (!c.desc) continue;
+        desc[i][0] = c.desc->magic;
+        memcpy(desc[i] + 1, c.val, sizeof(c.val));
+        CU(cudaMemcpyAsync((unsigned char*)blob + c.at, desc[i], kCkptDesc, cudaMemcpyHostToDevice, st));
+    }
     CU(cudaStreamSynchronize(st));   // `head` and the descriptors live on this stack frame
-    return checkpoint_copy(s, (unsigned char*)blob, true, st);
+    return checkpoint_copy(L, (unsigned char*)blob, true, st);
+}
+
+static const Described* described_by(int64_t magic) {
+    for (const Described* d : kDescribed)
+        if (d->magic == magic) return d;
+    return nullptr;
 }
 
 int lapf_sampler_load(lapf_sampler* s, const void* blob, int64_t blob_bytes, void* stream) {
     if (!s || !blob) return fail(LAPF_ERR_INVALID, "sampler/blob is NULL");
-    if ((size_t)blob_bytes < checkpoint_bytes(s)) return fail(LAPF_ERR_INVALID, "checkpoint buffer too small");
+    const CkptLayout L = checkpoint_layout(s);
+    if ((size_t)blob_bytes < L.bytes) return fail(LAPF_ERR_INVALID, "checkpoint buffer too small");
     cudaStream_t st = (cudaStream_t)stream;
+    const unsigned char* b = (const unsigned char*)blob;
+    // the head, every descriptor this sampler expects, and the 32 bytes past its layout (where a section it
+    // does not have would start), in one round trip
     int64_t head[2 + LAPF_MAX_PARAMS] = {0, 0};
-    CU(cudaMemcpyAsync(head, blob, kCkptHead, cudaMemcpyDeviceToHost, st));
+    int64_t desc[kSections + 1][4] = {};
+    CU(cudaMemcpyAsync(head, b, kCkptHead, cudaMemcpyDeviceToHost, st));
+    for (int i = 0; i < L.n; ++i)
+        if (L.sec[i].desc) CU(cudaMemcpyAsync(desc[i], b + L.sec[i].at, kCkptDesc, cudaMemcpyDeviceToHost, st));
+    if ((size_t)blob_bytes >= L.bytes + kCkptDesc) CU(cudaMemcpyAsync(desc[L.n], b + L.bytes, kCkptDesc, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     double wd[LAPF_MAX_PARAMS];
     memcpy(wd, head + 2, sizeof(wd));
     bool ok = head[0] >= 0;
     for (int i = 0; i < s->P; ++i) ok = ok && wd[i] >= 0.0 && std::isfinite(wd[i]);
     if (!ok) return fail(LAPF_ERR_INVALID, "corrupt checkpoint (count %lld)", (long long)head[0]);
-    if (s->bm) {
-        int64_t desc[4] = {0, 0, 0, 0};
-        CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + bm_desc_offset(s), kCkptBmDesc, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        if (desc[0] != kBmMagic || desc[1] != s->bm_rows || desc[2] != s->bm_levels || desc[3] != s->bm_c)
-            return fail(LAPF_ERR_INVALID, "checkpoint batch means (batch_rows %lld, levels %lld, %lld quantities) do not match "
-                        "this sampler's (%d, %d, %d)", (long long)desc[1], (long long)desc[2], (long long)desc[3],
-                        s->bm_rows, s->bm_levels, s->bm_c);
-    }
-    if (s->dr_val) {
-        int64_t desc[4] = {0, 0, 0, 0};
-        CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + dr_desc_offset(s), kCkptDrDesc, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        if (desc[0] != kDrMagic || desc[1] != s->dr_k || desc[2] != s->P + 1 || desc[3] != 0)
-            return fail(LAPF_ERR_INVALID, "checkpoint draws (%lld per walker, %lld columns) do not match this sampler's (%d, %d)",
-                        (long long)desc[1], (long long)desc[2], s->dr_k, s->P + 1);
-    }
-    {
-        // with frame widths the descriptor must be there; without them, a blob that carries them is refused
-        // too (its frame-widths section starts where this sampler's blob ends)
-        const size_t at = s->fw ? fw_desc_offset(s) : checkpoint_bytes(s);
-        int64_t desc[4] = {0, 0, 0, 0};
-        if (s->fw || (size_t)blob_bytes >= at + kCkptFwDesc) {
-            CU(cudaMemcpyAsync(desc, (const unsigned char*)blob + at, kCkptFwDesc, cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
+    for (int i = 0; i < L.n; ++i) {
+        const Described* want = L.sec[i].desc;
+        const int64_t* got = desc[i];
+        const int64_t* val = L.sec[i].val;
+        if (!want) continue;
+        if (got[0] != want->magic) {
+            if (const Described* found = described_by(got[0]))
+                return fail(LAPF_ERR_INVALID, "checkpoint carries %s where this sampler expects %s", found->name, want->name);
+            return fail(LAPF_ERR_INVALID, "checkpoint carries no %s where this sampler expects them", want->name);
         }
-        if (!s->fw && desc[0] == kFwMagic)
-            return fail(LAPF_ERR_INVALID, "checkpoint carries per-frame jump widths, this sampler has none "
-                        "(lapf_sampler_set_frame_widths before lapf_sampler_load)");
-        if (s->fw && (desc[0] != kFwMagic || desc[1] != s->cfg.problem.n_frames || desc[2] != s->P || desc[3] != 0))
-            return fail(LAPF_ERR_INVALID, "checkpoint per-frame widths (%lld frames, %lld parameters) do not match this "
-                        "sampler's (%d, %d)", desc[0] == kFwMagic ? (long long)desc[1] : 0LL,
-                        desc[0] == kFwMagic ? (long long)desc[2] : 0LL, s->cfg.problem.n_frames, s->P);
+        if (got[1] != val[0] || got[2] != val[1] || got[3] != val[2])
+            return fail(LAPF_ERR_INVALID, "checkpoint %s (%s) = (%lld, %lld, %lld) do not match this sampler's (%lld, %lld, "
+                        "%lld)", want->name, want->fields, (long long)got[1], (long long)got[2], (long long)got[3],
+                        (long long)val[0], (long long)val[1], (long long)val[2]);
     }
+    if (const Described* extra = described_by(desc[L.n][0]))
+        return fail(LAPF_ERR_INVALID, "checkpoint carries %s, this sampler has none (%s before lapf_sampler_load)",
+                    extra->name, extra->enable);
     s->count = head[0];
     s->cfg.seed = (uint64_t)head[1];
     memcpy(s->widths, wd, sizeof(wd));
-    return checkpoint_copy(s, (unsigned char*)const_cast<void*>(blob), false, st);
+    return checkpoint_copy(L, (unsigned char*)const_cast<void*>(blob), false, st);
 }
 
 int lapf_sampler_set_widths(lapf_sampler* s, const double* widths) {
@@ -2323,6 +2318,33 @@ int lapf_sampler_start(lapf_sampler* s, double* start_out, void* stream) {
     return LAPF_OK;
 }
 
+// Turns on optional device state, all or nothing: frees whatever the parts hold (re-enabling), allocates every
+// part, writes its fill (kKeep: `init` fills it), then runs the self-test if asked (unless LAPF_NO_SELFTEST).  On
+// any failure every part is freed and nulled again.
+extern "C++" {
+template <class Init>
+static int enable_parts(lapf_sampler* s, std::initializer_list<Part> parts, bool selftest, cudaStream_t st, Init&& init) {
+    auto drop = [&]() {
+        cudaStreamSynchronize(st);
+        for (const Part& p : parts) { cudaFree(*p.dev); *p.dev = nullptr; }
+    };
+    drop();
+    int rc = LAPF_OK;
+    for (const Part& p : parts) {
+        cudaError_t e = cudaMalloc(p.dev, p.bytes);
+        if (e == cudaSuccess && p.fill != kKeep) e = cudaMemsetAsync(*p.dev, p.fill, p.bytes, st);
+        if (e != cudaSuccess) {
+            rc = fail(LAPF_ERR_CUDA, "allocating %zu bytes of device state failed: %s", p.bytes, cudaGetErrorString(e));
+            break;
+        }
+    }
+    if (!rc) rc = init();
+    if (!rc && selftest && !getenv("LAPF_NO_SELFTEST")) rc = lapf_sampler_selftest(s, st);
+    if (rc) drop();
+    return rc;
+}
+}  // extern "C++"
+
 int lapf_sampler_sketch_enable(lapf_sampler* s, int32_t n_bins, double sep_bin, double pa_bin, const double* centers,
                                void* stream) {
     if (!s) return fail(LAPF_ERR_INVALID, "sampler is NULL");
@@ -2330,31 +2352,27 @@ int lapf_sampler_sketch_enable(lapf_sampler* s, int32_t n_bins, double sep_bin, 
         return fail(LAPF_ERR_INVALID, "sketch needs an even n_bins in [2, 2^20] and positive bin widths");
     cudaStream_t st = (cudaStream_t)stream;
     const int F = s->cfg.problem.n_frames, nbody = s->cfg.problem.nbody, slots = 2 * (nbody - 1);
-    const int64_t W = s->cfg.n_walkers;
     if (s->bm)
         return fail(LAPF_ERR_INVALID, "sketches cannot be enabled after batch means (the batch means would change shape)");
-    CU(cudaStreamSynchronize(st));
-    cudaFree(s->sk_hist); cudaFree(s->sk_center); cudaFree(s->sk_mom);
-    s->sk_hist = nullptr; s->sk_center = nullptr; s->sk_mom = nullptr;
-    s->sk_bins = 0;
-    CU(cudaMalloc((void**)&s->sk_hist, sizeof(uint32_t) * (size_t)F * slots * (n_bins + 2)));
-    CU(cudaMalloc((void**)&s->sk_center, sizeof(double) * (size_t)F * slots));
-    CU(cudaMalloc((void**)&s->sk_mom, sizeof(double) * (size_t)W * slots * 2));
-    CU(cudaMemsetAsync(s->sk_hist, 0, sizeof(uint32_t) * (size_t)F * slots * (n_bins + 2), st));
-    CU(cudaMemsetAsync(s->sk_mom, 0, sizeof(double) * (size_t)W * slots * 2, st));
-    s->sk_auto_center = centers == nullptr;
-    if (centers) {
-        CU(cudaMemcpyAsync(s->sk_center, centers, sizeof(double) * (size_t)F * slots, cudaMemcpyDeviceToDevice, st));
-    } else {
-        sketch_center_kernel<<<(F * (nbody - 1) + 127) / 128, 128, 0, st>>>(s->shift, s->walker_of, s->frame_start, F, s->P,
-                                                                          nbody, s->sk_center);
-        CU(cudaGetLastError());
-        s->launches++;
-    }
     s->sk_bins = n_bins;
     s->sk_sep_bin = sep_bin;
     s->sk_pa_bin = pa_bin;
-    return LAPF_OK;
+    s->sk_auto_center = centers == nullptr;
+    const int rc = enable_parts(s, {{(void**)&s->sk_hist, sketch_hist_bytes(s), 0},
+                                    {(void**)&s->sk_center, sizeof(double) * (size_t)F * slots, kKeep},
+                                    {(void**)&s->sk_mom, sketch_mom_bytes(s), 0}}, false, st, [&]() -> int {
+        if (centers) {
+            CU(cudaMemcpyAsync(s->sk_center, centers, sizeof(double) * (size_t)F * slots, cudaMemcpyDeviceToDevice, st));
+        } else {
+            sketch_center_kernel<<<(F * (nbody - 1) + 127) / 128, 128, 0, st>>>(s->shift, s->walker_of, s->frame_start, F,
+                                                                              s->P, nbody, s->sk_center);
+            CU(cudaGetLastError());
+            s->launches++;
+        }
+        return LAPF_OK;
+    });
+    if (rc) s->sk_bins = 0;
+    return rc;
 }
 
 int lapf_sampler_sketch(lapf_sampler* s, uint32_t* hist_out, double* summary_out, void* stream) {
@@ -2362,9 +2380,7 @@ int lapf_sampler_sketch(lapf_sampler* s, uint32_t* hist_out, double* summary_out
     if (!s->sk_hist) return fail(LAPF_ERR_INVALID, "sketches are not enabled (lapf_sampler_sketch_enable)");
     cudaStream_t st = (cudaStream_t)stream;
     const int F = s->cfg.problem.n_frames, slots = 2 * (s->cfg.problem.nbody - 1);
-    if (hist_out)
-        CU(cudaMemcpyAsync(hist_out, s->sk_hist, sizeof(uint32_t) * (size_t)F * slots * (s->sk_bins + 2),
-                           cudaMemcpyDeviceToDevice, st));
+    if (hist_out) CU(cudaMemcpyAsync(hist_out, s->sk_hist, sketch_hist_bytes(s), cudaMemcpyDeviceToDevice, st));
     if (summary_out) {
         // rows recorded since the sketches were last zeroed = rows recorded so far (enable before the first run)
         const int64_t n_rows = rows_upto(s->count, s->cfg.burn_in, s->cfg.thin);
@@ -2382,24 +2398,10 @@ int lapf_sampler_batchmeans_enable(lapf_sampler* s, int32_t batch_rows, int32_t 
         return fail(LAPF_ERR_INVALID, "batch means need batch_rows in [1, 2^30] and levels in [1, 24]");
     if (rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) > 0)
         return fail(LAPF_ERR_INVALID, "batch means must be enabled before the first recorded row");
-    cudaStream_t st = (cudaStream_t)stream;
-    CU(cudaStreamSynchronize(st));
-    cudaFree(s->bm);
-    s->bm = nullptr;
-    const int C = s->P + 1 + (s->sk_hist ? 2 * (s->cfg.problem.nbody - 1) : 0);
-    const size_t bytes = sizeof(double) * (size_t)s->cfg.n_walkers * C * levels * 2;
-    CU(cudaMalloc((void**)&s->bm, bytes));
     s->bm_rows = batch_rows;
     s->bm_levels = levels;
-    s->bm_c = C;
-    CU(cudaMemsetAsync(s->bm, 0, bytes, st));
-    int rc = LAPF_OK;
-    if (!getenv("LAPF_NO_SELFTEST") && (rc = lapf_sampler_selftest(s, st))) {
-        cudaStreamSynchronize(st);
-        cudaFree(s->bm);
-        s->bm = nullptr;
-    }
-    return rc;
+    s->bm_c = s->P + 1 + (s->sk_hist ? 2 * (s->cfg.problem.nbody - 1) : 0);
+    return enable_parts(s, {{(void**)&s->bm, bm_state_bytes(s), 0}}, true, (cudaStream_t)stream, [] { return LAPF_OK; });
 }
 
 int lapf_sampler_batchmeans(lapf_sampler* s, double* walker_out, double* frame_out, void* stream) {
@@ -2424,18 +2426,10 @@ int lapf_sampler_draws_enable(lapf_sampler* s, int32_t per_walker, void* stream)
     if (s->dr_val) return fail(LAPF_ERR_INVALID, "draws are already enabled");
     if (rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) > 0)
         return fail(LAPF_ERR_INVALID, "draws must be enabled before the first recorded row");
-    cudaStream_t st = (cudaStream_t)stream;
     s->dr_k = per_walker;
-    cudaError_t e = cudaMalloc((void**)&s->dr_val, draws_val_bytes(s));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&s->dr_row, draws_row_bytes(s));
-    int rc = e == cudaSuccess ? draws_clear(s, st)
-                              : fail(LAPF_ERR_CUDA, "cudaMalloc of the draws failed: %s", cudaGetErrorString(e));
-    if (!rc && !getenv("LAPF_NO_SELFTEST")) rc = lapf_sampler_selftest(s, st);
-    if (rc) {
-        cudaStreamSynchronize(st);
-        cudaFree(s->dr_val); cudaFree(s->dr_row);
-        s->dr_val = nullptr; s->dr_row = nullptr; s->dr_k = 0;
-    }
+    const int rc = enable_parts(s, {{(void**)&s->dr_val, draws_val_bytes(s), 0xFF}, {(void**)&s->dr_row, draws_row_bytes(s), 0xFF}},
+                                true, (cudaStream_t)stream, [] { return LAPF_OK; });
+    if (rc) s->dr_k = 0;
     return rc;
 }
 
@@ -2460,26 +2454,13 @@ int lapf_sampler_set_frame_widths(lapf_sampler* s, const double* widths, void* s
             h[(size_t)f * P + j] = v;
         }
     cudaStream_t st = (cudaStream_t)stream;
-    const bool first = s->fw == nullptr;
-    if (first) {
-        cudaError_t e = cudaMalloc((void**)&s->fw, fw_bytes(s));
-        if (e == cudaSuccess) e = cudaMalloc((void**)&s->fw_snap, fw_snap_bytes(s));
-        if (e == cudaSuccess) e = cudaMemsetAsync(s->fw_snap, 0, fw_snap_bytes(s), st);
-        if (e != cudaSuccess) {
-            cudaFree(s->fw); cudaFree(s->fw_snap);
-            s->fw = nullptr; s->fw_snap = nullptr;
-            return fail(LAPF_ERR_CUDA, "allocation of the per-frame widths failed: %s", cudaGetErrorString(e));
-        }
-    }
-    CU(cudaMemcpyAsync(s->fw, h.data(), fw_bytes(s), cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));   // `h` is pageable and lives on this stack frame
-    int rc = LAPF_OK;
-    if (first && !getenv("LAPF_NO_SELFTEST") && (rc = lapf_sampler_selftest(s, st))) {
-        cudaStreamSynchronize(st);
-        cudaFree(s->fw); cudaFree(s->fw_snap);
-        s->fw = nullptr; s->fw_snap = nullptr;
-    }
-    return rc;
+    auto put = [&]() -> int {
+        CU(cudaMemcpyAsync(s->fw, h.data(), fw_bytes(s), cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));   // `h` is pageable and lives on this stack frame
+        return LAPF_OK;
+    };
+    if (s->fw) return put();   // later calls replace the widths and keep the snapshot
+    return enable_parts(s, {{(void**)&s->fw, fw_bytes(s), kKeep}, {(void**)&s->fw_snap, fw_snap_bytes(s), 0}}, true, st, put);
 }
 
 int lapf_sampler_frame_widths(lapf_sampler* s, double* out, void* stream) {
