@@ -134,7 +134,9 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream);
  * counters, moments and update count back to zero, initial chi-square re-evaluated against the
  * CURRENT contents of the problem's data/weight buffers (which the caller may have overwritten
  * with new frames of the same shape).  frame_of, widths, burn_in and thin are kept.  Lets a
- * stream of epochs reuse one handle without reallocating device memory. */
+ * stream of epochs reuse one handle without reallocating device memory.  With priors on
+ * (lapf_sampler_set_priors) the table is kept, and starting points outside its boxes give
+ * LAPF_ERR_INVALID, naming the frame and the parameter, with the sampler unchanged. */
 int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed, void* stream);
 
 /* Checkpoint / resume.  A walker is (parameters, chi-square, counters, moments, update count; the
@@ -154,10 +156,11 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
  *   batch means, if on    {'LAPFBM01', batch_rows, levels, C}; walker state
  *   draws, if on          {'LAPFRS01', K, P+1, 0}; values, row indices
  *   frame widths, if on   {'LAPFFW01', F, P, 0}; widths, adaptation snapshot
+ *   priors, if on         {'LAPFPR01', F, P, 0}; table {lo, hi, mu, h}, table as given {lo, hi, mu, sigma}
  * load() refuses a blob (LAPF_ERR_INVALID, the sampler unchanged) that is smaller than this sampler's
  * layout, whose head is corrupt, that lacks a descriptor this sampler expects or differs in one, or
  * whose bytes just past this sampler's layout start with a known magic (a section this sampler does
- * not have).  So a blob loads only into a sampler with the same batch means, draws and frame widths.
+ * not have).  So a blob loads only into a sampler with the same batch means, draws, frame widths and priors.
  * The sketch section has no descriptor: a blob whose sketch setting differs from the sampler's is
  * refused only when that shifts a later descriptor or the blob is too small. */
 int64_t lapf_sampler_checkpoint_bytes(const lapf_sampler* s);
@@ -321,6 +324,25 @@ int lapf_sampler_frame_counts(lapf_sampler* s, int64_t* out, void* stream);
  * ranks that apply it to the same counts keep the same widths.  LAPF_ERR_INVALID without the table or
  * unless 0 < target < 1. */
 int lapf_sampler_adapt_widths(lapf_sampler* s, const int64_t* counts, double target, void* stream);
+
+/* K4f -- per-frame parameter priors (DESIGN.md, "Priors").  The reference's accept rule is the bare likelihood
+ * ratio; with a table, the walkers of frame f see, on parameter j, the box lo <= value <= hi and the Gaussian
+ * term N(mu, sigma), in chain units (the columns of the chain rows: frame coordinates, and the log10-proposed
+ * parameters as values, so the user's prior multiplies the reference's implicit log-uniform one).  An update
+ * of parameter k from pk to nv of a walker of frame f:
+ *   a proposal outside [lo, hi] (or nan) is rejected: it counts as a try, and the batched kernel skips its pass;
+ *   otherwise accept iff ln u < -0.5 (chi_t - chi_c) - g,  g = h ((nv - mu)^2 - (pk - mu)^2),  h = 0.5 / sigma^2,
+ *   with g = 0 where sigma = +inf, and every operation rounded to nearest, never fused.
+ *   table  HOST double [F][P][4] {lo, hi, mu, sigma}; lo = -inf / hi = +inf: no bound, sigma = +inf: no term.
+ * LAPF_ERR_INVALID (the sampler unchanged) if an entry is nan, lo > hi, sigma <= 0, sigma is so small that h
+ * overflows, mu is not finite while sigma is, or any walker's current state lies outside its frame's box (the
+ * message names the first frame and parameter).  The first call allocates the table and runs
+ * lapf_sampler_selftest with it active (unless LAPF_NO_SELFTEST); later calls replace it between runs.
+ * lapf_sampler_reset keeps it and refuses starts outside it.  Checkpoints carry it (see lapf_sampler_save).  A
+ * table with every box infinite and every sigma +inf gives the chains of no table bit for bit. */
+int lapf_sampler_set_priors(lapf_sampler* s, const double* table, void* stream);
+/*   out device double [F][P][4]: the table as given ({lo, hi, mu, sigma}).  LAPF_ERR_INVALID without a table. */
+int lapf_sampler_priors(lapf_sampler* s, double* out, void* stream);
 
 /* Total update count so far (same for every walker). */
 int64_t lapf_sampler_count(const lapf_sampler* s);

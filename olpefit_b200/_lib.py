@@ -59,6 +59,8 @@ SYMBOLS = {
     "lapf_sampler_frame_widths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "lapf_sampler_frame_counts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "lapf_sampler_adapt_widths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]),
+    "lapf_sampler_set_priors": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.c_void_p]),
+    "lapf_sampler_priors": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "lapf_frame_outside": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                      C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "lapf_sampler_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

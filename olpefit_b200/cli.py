@@ -83,7 +83,12 @@ def _parser(kind):
                     help="write <results>/checkpoint_rank<r>.pt when done (exact state of every walker)")
     ap.add_argument("--resume", action="store_true",
                     help="continue from <results>/checkpoint_rank<r>.pt, appending to the existing chain files "
-                         "(give the --mcse / --ess-min, --draws and --adapt-per-epoch of the run that wrote it)")
+                         "(give the --mcse / --ess-min, --draws, --adapt-per-epoch and --prior of the run that wrote it)")
+    ap.add_argument("--prior", type=str, default=None, metavar="FILE",
+                    help="JSON priors on the parameters, in chain units: {\"all\": {NAME: {\"min\", \"max\", \"mean\", "
+                         "\"sigma\"}}, \"epochs\": {\"<N>\": {NAME: {...}}}}; a proposal outside [min, max] is rejected, "
+                         "mean / sigma add a Gaussian term to the accept rule; an epoch's entry for a parameter replaces "
+                         "the \"all\" one; step2_summary.json gains \"priors\"")
     if kind != "step2a":
         ap.add_argument("--mcse", action="store_true",
                         help="keep batch means of every recorded value on the device: step2_summary.json gains the "
@@ -112,6 +117,92 @@ MCSE_BATCH_ROWS, MCSE_LEVELS = 64, 16
 # (the constants of --adapt).  The windows are fixed in update counts, so a run resumed from a checkpoint
 # adapts at the same counts as one that was never interrupted.
 ADAPT_WINDOW, ADAPT_TARGET = 512, 0.35
+
+
+_PRIOR_KEYS = {"min": 0, "max": 1, "mean": 2, "sigma": 3}
+
+
+def load_prior_file(path, nbody, epochs):
+    """The [F, P, 4] {lo, hi, mu, sigma} table of a --prior FILE for the epochs numbered ``epochs`` (the <N>
+    of each frame, in frame order).  Refuses (SystemExit, with a message) unknown parameter names, keys or
+    epochs, min >= max, sigma <= 0, a mean without a sigma or the other way round, and values that are not
+    finite numbers."""
+    from . import layout
+    try:
+        with open(path) as fh:
+            spec = json.load(fh)
+    except (OSError, ValueError) as e:
+        raise SystemExit("--prior %s: %s" % (path, e))
+    names = list(layout.names(nbody))
+    epochs = [str(e) for e in epochs]
+
+    def entries(block, where):
+        if not isinstance(block, dict):
+            raise SystemExit("--prior %s: %s must be an object of parameter names" % (path, where))
+        out = {}
+        for name, d in block.items():
+            if name not in names:
+                raise SystemExit("--prior %s: unknown parameter %r in %s (known: %s)" % (path, name, where, ", ".join(names)))
+            if not isinstance(d, dict) or not d:
+                raise SystemExit("--prior %s: %s.%s must be an object with min, max, mean, sigma" % (path, where, name))
+            e = [-np.inf, np.inf, 0.0, np.inf]
+            for key, v in d.items():
+                if key not in _PRIOR_KEYS:
+                    raise SystemExit("--prior %s: unknown key %r in %s.%s (known: min, max, mean, sigma)" % (path, key, where, name))
+                if isinstance(v, bool) or not isinstance(v, (int, float)) or not np.isfinite(v):
+                    raise SystemExit("--prior %s: %s.%s.%s = %r is not a finite number" % (path, where, name, key, v))
+                e[_PRIOR_KEYS[key]] = float(v)
+            if not e[0] < e[1]:
+                raise SystemExit("--prior %s: %s.%s has min %g >= max %g" % (path, where, name, e[0], e[1]))
+            if ("mean" in d) != ("sigma" in d):
+                raise SystemExit("--prior %s: %s.%s needs mean and sigma together" % (path, where, name))
+            if not e[3] > 0:
+                raise SystemExit("--prior %s: %s.%s has sigma %g <= 0" % (path, where, name, e[3]))
+            out[names.index(name)] = e
+        return out
+
+    if not isinstance(spec, dict) or set(spec) - {"all", "epochs"}:
+        raise SystemExit("--prior %s: the top level takes \"all\" and \"epochs\" only" % path)
+    common = entries(spec.get("all", {}), "all")
+    per_epoch = spec.get("epochs", {})
+    if not isinstance(per_epoch, dict):
+        raise SystemExit("--prior %s: \"epochs\" must be an object keyed by epoch number" % path)
+    for ep in per_epoch:
+        if ep not in epochs:
+            raise SystemExit("--prior %s: unknown epoch %r (this run has %s)" % (path, ep, ", ".join(epochs)))
+    table = np.empty((len(epochs), len(names), 4))
+    table[:] = [-np.inf, np.inf, 0.0, np.inf]
+    for f, ep in enumerate(epochs):
+        for j, e in common.items():
+            table[f, j] = e
+        for j, e in entries(per_epoch.get(ep, {}), "epochs.%s" % ep).items():
+            table[f, j] = e
+    return table
+
+
+def prior_summary(table_f, nbody):
+    """step2_summary.json's "priors" of one epoch: per parameter that has a bound or a Gaussian term,
+    {min, max, mean, sigma} as applied, None for what it does not have."""
+    from . import layout
+    out = {}
+    for j, name in enumerate(layout.names(nbody)):
+        lo, hi, mu, sg = (float(v) for v in table_f[j])
+        if np.isinf(lo) and np.isinf(hi) and np.isinf(sg):
+            continue
+        finite = np.isfinite(sg)
+        out[name] = {"min": lo if np.isfinite(lo) else None, "max": hi if np.isfinite(hi) else None,
+                     "mean": mu if finite else None, "sigma": sg if finite else None}
+    return out
+
+
+def check_prior_starts(table, starts, nbody, epochs):
+    """SystemExit naming the epoch and the parameter if a start (``starts`` [F, P]) lies outside its box."""
+    from . import layout
+    out = ~((starts >= table[..., 0]) & (starts <= table[..., 1]))
+    if out.any():
+        f, j = (int(v) for v in np.argwhere(out)[0])
+        raise SystemExit("--prior: the start of epoch %s has %s = %.17g outside [%g, %g]"
+                         % (epochs[f], layout.names(nbody)[j], starts[f, j], table[f, j, 0], table[f, j, 1]))
 
 
 def _burn_in(args, kind, nbody):
@@ -221,8 +312,13 @@ def run(kind, nbody, argv=None):
         raise SystemExit("--adapt-per-epoch and --adapt both tune the jump widths: give one of them")
     if adapt_pe and burn_in <= 0:
         raise SystemExit("--adapt-per-epoch tunes the widths during burn-in, and burn-in is 0: give --burn-in")
+    from . import chains
+    prior = None
+    if args.prior:
+        prior_epochs = [chains.split_image_path(p)[1] for p in _frame_list(args)]
+        prior = load_prior_file(args.prior, nbody, prior_epochs)
     import torch
-    from . import chains, dist, frame, layout, sampler as smp, stats
+    from . import dist, frame, layout, sampler as smp, stats
 
     rank, local_rank, world = dist.init()
     if not torch.cuda.is_available():
@@ -255,6 +351,8 @@ def run(kind, nbody, argv=None):
     dom, params, cuts, headers = frame.load_epochs(images, start_fn, nbody=nbody, size=args.stamp,
                                                    floor_index=floor_index, device=device,
                                                    whole_frame=(args.domain == "frame"))
+    if prior is not None:
+        check_prior_starts(prior, np.asarray(params, dtype=np.float64), nbody, prior_epochs)
     if n_frames == 1:
         say("Masking pixels greater than ", 0.8 * frame.saturation_level(headers[0]))
     say("I have masked", int((dom.weight == 0).sum().item()), "pixels (inside the %dx%d domain%s)"
@@ -319,6 +417,8 @@ def run(kind, nbody, argv=None):
         sam.enable_draws(draws_k)
     if adapt_pe:
         sam.set_frame_widths()                # the default widths in every epoch's row, until burn-in tunes them
+    if prior is not None:
+        sam.set_priors(prior[..., 0], prior[..., 1], prior[..., 2], prior[..., 3])
 
     def frame_counts():
         # per-epoch tries / accepts summed over ranks (a rank without walkers adds zeros); every rank must call it
@@ -354,6 +454,11 @@ def run(kind, nbody, argv=None):
         if ck["n_walkers"] != sam.n_walkers or ck["nbody"] != nbody:
             raise SystemExit("checkpoint %s does not match this run" % ckpt_path)
         sam.load(ck["blob"])
+        if prior is not None:
+            got = sam.priors().cpu().numpy()
+            if not np.array_equal(got, prior):
+                raise SystemExit("checkpoint %s was written with other priors than --prior %s: give the same file"
+                                 % (ckpt_path, args.prior))
         seed = ck["seed"]
         if adapt_pe and ck.get("burn_counts") is not None:
             burn_counts = ck["burn_counts"].to(device)
@@ -530,6 +635,9 @@ def run(kind, nbody, argv=None):
             rate = after[f, :, 1] / np.maximum(after[f, :, 0], 1)
             say("epoch %d: acceptance after burn-in %s, jump widths %s"
                 % (f, np.array2string(rate, precision=3), np.array2string(fw[f], precision=4)))
+    if prior is not None:
+        for f in range(n_frames):
+            summaries[f]["priors"] = prior_summary(prior[f], nbody)
     if stop_rule or bm_on:
         stop["updates"] = sam.count
         for f in range(n_frames):

@@ -343,7 +343,11 @@ struct RunArgs {
     // per-frame jump widths (lapf_sampler_set_frame_widths), or nullptr: the proposal of a walker of frame f
     // reads fwidths[f * P + k] instead of widths[k]
     const double* fwidths;       // [F][P]
-    double* probe;               // self-test only: [rows][W][3] = parameter index, proposed value, TRIAL chi-square
+    // parameter priors (lapf_sampler_set_priors), or nullptr: per frame and parameter the box [lo, hi] and the
+    // Gaussian term's mu and h = 0.5 / sigma^2 (0: none)
+    const double* prior;         // [F][P][4] lo, hi, mu, h
+    double* probe;               // self-test only: [rows][W][3] = parameter index (-1 - index: the proposal lay
+                                 // outside its box, no pass), proposed value, TRIAL chi-square
     unsigned long long* cta_times;   // diagnosis only (LAPF_CTA_TIMES): [CTAs][3] = start, end (globaltimer ns), SM id
     int64_t n_walkers;
     int64_t t0, n_updates;       // first update index, updates in this launch
@@ -415,6 +419,19 @@ __device__ __forceinline__ void record_sketch(const RunArgs& a, int wl, int fram
             atomicAdd(m + 1, d * d);
         }
     }
+}
+
+// Priors (lapf_sampler_set_priors): `pr` is the table entry {lo, hi, mu, h} of the walker's frame and the
+// updated parameter.  A value outside the box (or nan) is outside.
+__device__ __forceinline__ bool prior_outside(const double* pr, double v) { return !(v >= pr[0] && v <= pr[1]); }
+// The Gaussian term of the Metropolis ratio for a move pk -> nv, g = h ((nv - mu)^2 - (pk - mu)^2); 0 without one
+// (h = 0: never multiplied, 0 * inf would be nan).  Rounded to nearest and never contracted (DESIGN.md 5): the
+// tests restate it in numpy.
+__device__ __forceinline__ double prior_g(const double* pr, double nv, double pk) {
+    const double h = pr[3];
+    if (h == 0.0) return 0.0;
+    const double dn = __dsub_rn(nv, pr[2]), dp = __dsub_rn(pk, pr[2]);
+    return __dmul_rn(h, __dsub_rn(__dmul_rn(dn, dn), __dmul_rn(dp, dp)));
 }
 
 // One walker for n_updates updates.  TEAM = 1: one warp does everything.  TEAM > 1 (few walkers,
@@ -536,8 +553,17 @@ __device__ __forceinline__ void run_walker(const RunArgs& a, const float* sd, co
         }
         if (a.outside) chi_t += outside_chi2(a.outside, frame, (k == a.floor_index) ? nv : shfl_f64(p, a.floor_index));
 
-        // accept iff u < exp(-(chi_t - chi_c)/2) (apf_step2.py:139-148); false on nan
-        const bool acc = ws.lnu[slot] < -0.5 * (chi_t - chi_c);
+        // priors: a proposal outside its box was evaluated like any other (every warp of the team keeps the
+        // barrier count) and is rejected here; the Gaussian term joins the ratio
+        bool in_box = true;
+        double g = 0.0;
+        if (a.prior) {                                                // (uniform branch)
+            const double* pr = a.prior + ((size_t)frame * P + k) * 4;
+            in_box = !prior_outside(pr, nv);
+            g = prior_g(pr, nv, shfl_f64(p, k));                      // p is still the state before the update
+        }
+        // accept iff u < exp(-(chi_t - chi_c)/2 - g) (apf_step2.py:139-148); false on nan
+        const bool acc = in_box && ws.lnu[slot] < __dsub_rn(__dmul_rn(-0.5, __dsub_rn(chi_t, chi_c)), g);
         if (lane == 0 && tw == 0) {
             atomicAdd(&a.tries[(size_t)wl * P + k], 1u);              // :304
             if (acc) atomicAdd(&a.accepts[(size_t)wl * P + k], 1u);   // :323
@@ -728,7 +754,8 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
             // with a negative background never moves it) has chi-square nan and is rejected (:139-148): its
             // pass is skipped instead of sending a nan vector through the plain loop at twice the cost of a
             // pass.  (With two vectors per pass it keeps its partner company in the factorised loop instead.)
-            skip = nv != nv;
+            // With priors, so is a proposal outside its frame's box (nan is outside every box).
+            skip = a.prior ? prior_outside(a.prior + ((size_t)((two && slot) ? frame1 : frame0) * P + k) * 4, nv) : nv != nv;
             if (skip && WPP > 1) cf.fast = true;
             if (LANE_SUMS && !skip) n_exps += cf.nexp;
             store_coef<NB, Geo<NX>::PANELS>(img + lane * I::STRIDE, cf, slot | (skip ? 2 : 0));
@@ -800,8 +827,11 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
                 if (k == a.floor_index) fl = nv;
                 chi_t += outside_chi2(a.outside, (two && slot) ? frame1 : frame0, fl);
             }
-            // accept iff u < exp(-(chi_t - chi_c)/2) (apf_step2.py:139-148); false on nan
-            const bool acc = lnu < -0.5 * (chi_t - chi_c);
+            // priors: the Gaussian term from the table and st[k], which still holds pk (a skipped proposal has
+            // chi_t = nan and is rejected whatever g is)
+            const double g = a.prior ? prior_g(a.prior + ((size_t)((two && slot) ? frame1 : frame0) * P + k) * 4, nv, st[k]) : 0.0;
+            // accept iff u < exp(-(chi_t - chi_c)/2 - g) (apf_step2.py:139-148); false on nan
+            const bool acc = lnu < __dsub_rn(__dmul_rn(-0.5, __dsub_rn(chi_t, chi_c)), g);
             atomicAdd(&a.tries[(size_t)wl * P + k], 1u);                  // :304
             if (acc) {
                 atomicAdd(&a.accepts[(size_t)wl * P + k], 1u);            // :323
@@ -863,7 +893,7 @@ __device__ __forceinline__ void run_batch(const RunArgs& a, const float* sd, con
                 }
                 if (a.probe) {                                            // lapf_sampler_selftest
                     double* pb = a.probe + ((size_t)row * a.n_walkers + wl) * 3;
-                    pb[0] = (double)k; pb[1] = nv; pb[2] = chi_t;
+                    pb[0] = (a.prior && skip) ? (double)(-1 - k) : (double)k; pb[1] = nv; pb[2] = chi_t;
                 }
             }
             ++row;
@@ -979,16 +1009,22 @@ __global__ void selftest_trials_kernel(const double* __restrict__ start, const d
     if (i >= (int64_t)U * W) return;
     const int64_t u = i / W, w = i % W;
     const double* before = u ? chain + ((u - 1) * W + w) * (P + 1) : start + w * (P + 1);
-    const int k = (int)probe[i * 3];
+    int k = (int)probe[i * 3];
+    if (k < 0) k = -1 - k;                                         // a proposal outside its prior box
     for (int j = 0; j < P; ++j) trials[i * P + j] = (j == k) ? probe[i * 3 + 1] : before[j];
 }
 
+// With priors a probe row marked as outside its box (no pass, no trial chi-square) must hold a proposal that lies
+// outside the box of its frame (`frame_of` [U][W]) and every other row one inside it, so a wrong skip fails too.
 __global__ void selftest_compare_kernel(const double* __restrict__ probe, const double* __restrict__ chi_k1, int64_t n,
+                                        const double* __restrict__ prior, const int32_t* __restrict__ frame_of, int P,
                                         unsigned long long* __restrict__ out /*[2]: mismatches, first index + 1*/) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const double a = probe[i * 3 + 2], b = chi_k1[i];
-    const bool same = (a == b) || (isnan(a) && isnan(b));
+    const double a = probe[i * 3 + 2], b = chi_k1[i], kd = probe[i * 3];
+    const int k = kd < 0.0 ? (int)(-1.0 - kd) : (int)kd;
+    const bool outside = prior && prior_outside(prior + ((size_t)frame_of[i] * P + k) * 4, probe[i * 3 + 1]);
+    const bool same = kd < 0.0 ? outside : ((a == b) || (isnan(a) && isnan(b))) && !outside;
     if (!same) {
         atomicAdd(out, 1ull);
         atomicMin(out + 1, (unsigned long long)i + 1ull);
@@ -1005,6 +1041,26 @@ __global__ void pack_state_kernel(const double* __restrict__ init, const double*
     const double v = (j < P) ? init[w * P + j] : chi[w];
     state[i] = v;
     shift[i] = v;
+}
+
+// Priors: per walker w (of frame frame_of[w]), the parameters params[w * stride + j] outside the frame's box;
+// out[0] += that count, out[1] = min(out[1], w * P + j + 1) over them
+__global__ void prior_outside_kernel(const double* __restrict__ params, int stride, const int32_t* __restrict__ frame_of,
+                                     const double* __restrict__ prior, int P, int64_t W, unsigned long long* __restrict__ out) {
+    const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= W) return;
+    const double* pr = prior + (size_t)frame_of[w] * P * 4;
+    unsigned n = 0;
+    int first = -1;
+    for (int j = 0; j < P; ++j)
+        if (prior_outside(pr + 4 * j, params[w * stride + j])) {
+            if (!n) first = j;
+            ++n;
+        }
+    if (n) {
+        atomicAdd(out, (unsigned long long)n);
+        atomicMin(out + 1, (unsigned long long)(w * P + first) + 1ull);
+    }
 }
 
 // =============================================================================================
@@ -1427,6 +1483,10 @@ struct lapf_sampler {
     // adaptation [F][P][2] (tries, accepts summed over the frame's walkers and over ranks)
     double* fw = nullptr;
     long long* fw_snap = nullptr;
+    // parameter priors (lapf_sampler_set_priors): [F][P][4] {lo, hi, mu, h} for the kernels, and the table as
+    // given, {lo, hi, mu, sigma}
+    double* pr = nullptr;
+    double* pr_given = nullptr;
     int chunk = 0;                 // batched kernel: walkers per item at most (warps x walkers per warp)
     int launch_grid = 0;           // batched kernel: CTAs that have work
 };
@@ -1681,6 +1741,7 @@ static void free_sampler(lapf_sampler* s) {
     cudaFree(s->bm);
     cudaFree(s->dr_val); cudaFree(s->dr_row);
     cudaFree(s->fw); cudaFree(s->fw_snap);
+    cudaFree(s->pr); cudaFree(s->pr_given);
     delete s;
 }
 
@@ -1853,6 +1914,7 @@ static size_t draws_val_bytes(const lapf_sampler* s) { return sizeof(double) * (
 static size_t draws_row_bytes(const lapf_sampler* s) { return sizeof(int64_t) * (size_t)s->cfg.n_walkers * s->dr_k; }
 static size_t fw_bytes(const lapf_sampler* s) { return sizeof(double) * (size_t)s->cfg.problem.n_frames * s->P; }
 static size_t fw_snap_bytes(const lapf_sampler* s) { return 2 * sizeof(long long) * (size_t)s->cfg.problem.n_frames * s->P; }
+static size_t prior_bytes(const lapf_sampler* s) { return 4 * sizeof(double) * (size_t)s->cfg.problem.n_frames * s->P; }
 
 // Checkpoint layout: see lapf_sampler_save in lapf.h.  The head [count][seed][jump widths x LAPF_MAX_PARAMS] is
 // built on the host; checkpoint_layout lists the sections that follow it, and every size, offset, copy, reset
@@ -1871,7 +1933,9 @@ static const Described kDraws = {0x313053524650414cLL, "posterior draws", "per w
                                   "lapf_sampler_draws_enable"};
 static const Described kFrameWidths = {0x313057464650414cLL, "per-frame jump widths", "frames, parameters, 0", // 'LAPFFW01'
                                        "lapf_sampler_set_frame_widths"};
-static const Described* const kDescribed[] = {&kBatchMeans, &kDraws, &kFrameWidths};
+static const Described kPriors = {0x313052504650414cLL, "parameter priors", "frames, parameters, 0",         // 'LAPFPR01'
+                                  "lapf_sampler_set_priors"};
+static const Described* const kDescribed[] = {&kBatchMeans, &kDraws, &kFrameWidths, &kPriors};
 struct Section {
     const Described* desc;   // nullptr: no descriptor
     int64_t val[3];          // the descriptor's a, b, c
@@ -1879,7 +1943,7 @@ struct Section {
     Part part[6];
     size_t at;               // offset in the blob (of the descriptor, if any)
 };
-constexpr int kSections = 5;   // core, sketches, batch means, draws, per-frame widths
+constexpr int kSections = 6;   // core, sketches, batch means, draws, per-frame widths, priors
 struct CkptLayout { int n; Section sec[kSections]; size_t bytes; };
 
 static CkptLayout checkpoint_layout(lapf_sampler* s) {
@@ -1902,6 +1966,9 @@ static CkptLayout checkpoint_layout(lapf_sampler* s) {
     if (s->fw)       // reset keeps the widths; the counters start again, so does the adaptation window
         L.sec[L.n++] = {&kFrameWidths, {s->cfg.problem.n_frames, s->P, 0}, 2,
                         {{(void**)&s->fw, fw_bytes(s), kKeep}, {(void**)&s->fw_snap, fw_snap_bytes(s), 0}}};
+    if (s->pr)       // reset keeps the table (and refuses starts outside it)
+        L.sec[L.n++] = {&kPriors, {s->cfg.problem.n_frames, s->P, 0}, 2,
+                        {{(void**)&s->pr, prior_bytes(s), kKeep}, {(void**)&s->pr_given, prior_bytes(s), kKeep}}};
     L.bytes = kCkptHead;
     for (int i = 0; i < L.n; ++i) {
         Section& c = L.sec[i];
@@ -1916,12 +1983,48 @@ static size_t checkpoint_bytes(const lapf_sampler* s) {
     return checkpoint_layout(const_cast<lapf_sampler*>(s)).bytes;   // reads sizes only
 }
 
+// Priors: LAPF_ERR_INVALID, naming the first walker, frame and parameter, if any parameter of `params` (walker w
+// at params[w * stride], frame s->frame_of[w]) lies outside the box of `table` (device [F][P][4] {lo, hi, ...}).
+static int prior_check(lapf_sampler* s, const double* params, int stride, const double* table, const char* what,
+                       cudaStream_t st) {
+    const int64_t W = s->cfg.n_walkers;
+    const int P = s->P;
+    unsigned long long* out = nullptr;
+    const unsigned long long init[2] = {0ull, ~0ull};
+    unsigned long long res[2] = {0, 0};
+    CU(cudaMallocAsync((void**)&out, sizeof(init), st));
+    cudaError_t e = cudaMemcpyAsync(out, init, sizeof(init), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) {
+        prior_outside_kernel<<<(unsigned)((W + 255) / 256), 256, 0, st>>>(params, stride, s->frame_of, table, P, W, out);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(res, out, sizeof(res), cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(out, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // `init` and `res` live on this stack frame
+    if (e != cudaSuccess) return fail(LAPF_ERR_CUDA, "prior check failed: %s", cudaGetErrorString(e));
+    s->launches++;
+    if (res[0] == 0) return LAPF_OK;
+    const int64_t w = (int64_t)((res[1] - 1) / P);
+    const int j = (int)((res[1] - 1) % P);
+    int32_t f = 0;
+    double v = 0.0, box[2] = {0.0, 0.0};
+    CU(cudaMemcpyAsync(&f, s->frame_of + w, sizeof(f), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&v, params + w * stride + j, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaMemcpyAsync(box, table + ((size_t)f * P + j) * 4, sizeof(box), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return fail(LAPF_ERR_INVALID, "%s: %llu parameter value(s) lie outside their prior box; the first is frame %d, "
+                "parameter %d of walker %lld: %.17g not in [%g, %g]", what, res[0], f, j, (long long)w, v, box[0], box[1]);
+}
+
 int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed, void* stream) {
     if (!s || !init_params) return fail(LAPF_ERR_INVALID, "sampler/init_params is NULL");
     cudaStream_t st = (cudaStream_t)stream;
     const int P = s->P;
     const int64_t W = s->cfg.n_walkers;
     const size_t nst = (size_t)W * (P + 1);
+    int rc = s->pr ? prior_check(s, init_params, P, s->pr, "reset refused", st) : LAPF_OK;
+    if (rc) return rc;                                   // before anything changes
     const CkptLayout L = checkpoint_layout(s);
     for (int i = 0; i < L.n; ++i)
         for (int j = 0; j < L.sec[i].n_parts; ++j) {
@@ -1931,7 +2034,7 @@ int lapf_sampler_reset(lapf_sampler* s, const double* init_params, uint64_t seed
     // initial chi-square (apf_step2.py:283-289) through K1, then pack the state
     double* chi0 = nullptr;
     CU(cudaMallocAsync((void**)&chi0, sizeof(double) * W, st));
-    int rc = lapf_model_chi2(&s->cfg.problem, init_params, W, s->cfg.frame_of, nullptr, chi0, st);
+    rc = lapf_model_chi2(&s->cfg.problem, init_params, W, s->cfg.frame_of, nullptr, chi0, st);
     if (rc) { cudaFreeAsync(chi0, st); return rc; }
     pack_state_kernel<<<(unsigned)((nst + 255) / 256), 256, 0, st>>>(init_params, chi0, P, W, s->state, s->shift);
     CU(cudaGetLastError());
@@ -2121,6 +2224,7 @@ static void fill_run_args(const lapf_sampler* s, RunArgs& a, int64_t n_updates, 
     a.dr_val = s->dr_val; a.dr_row = s->dr_row; a.dr_k = s->dr_k;
     a.dr_row0 = s->dr_val ? rows_upto(s->count, s->cfg.burn_in, s->cfg.thin) : 0;
     a.fwidths = s->fw;
+    a.prior = s->pr;
     a.probe = nullptr;
     a.cta_times = nullptr;
 }
@@ -2266,7 +2370,7 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     if (rc) { cleanup(); return rc; }
     const unsigned long long init[2] = {0ull, ~0ull};
     CUT(cudaMemcpyAsync(out, init, 16, cudaMemcpyHostToDevice, st));
-    selftest_compare_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(probe, chi, n, out);
+    selftest_compare_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(probe, chi, n, s->pr, fo, P, out);
     CUT(cudaGetLastError());
     unsigned long long res[2] = {0, 0};
     CUT(cudaMemcpyAsync(res, out, 16, cudaMemcpyDeviceToHost, st));
@@ -2275,6 +2379,7 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     CUT(cudaStreamSynchronize(st));
     if (const char* path = getenv("LAPF_SELFTEST_DUMP")) {
         // diagnosis of a failing build: [U, W, P] as int64, then probe [U W 3], chi [U W], trials [U W P] as doubles
+        // (a probe row whose index is -1 - k: parameter k, the proposal lay outside its prior box and had no pass)
         std::vector<double> hp((size_t)n * 3), hc((size_t)n), ht((size_t)n * P);
         CUT(cudaMemcpy(hp.data(), probe, sizeof(double) * hp.size(), cudaMemcpyDeviceToHost));
         CUT(cudaMemcpy(hc.data(), chi, sizeof(double) * hc.size(), cudaMemcpyDeviceToHost));
@@ -2294,7 +2399,7 @@ int lapf_sampler_selftest(lapf_sampler* s, void* stream) {
     if (res[0] != 0)
         return fail(LAPF_ERR_SELFTEST,
                     "self-test failed: %llu of %lld trial chi-squares of the batched sampler differ from the stateless "
-                    "operator (first: update %lld of walker %lld).  This build of liblapf.so mis-compiles the sampler "
+                    "operator or mark a wrong prior-box skip (first: update %lld of walker %lld).  This build of liblapf.so mis-compiles the sampler "
                     "kernel; rebuild with the CUDA toolkit the tests were run with (see DESIGN.md 10).",
                     res[0], (long long)n, (long long)((res[1] - 1) / W), (long long)((res[1] - 1) % W));
     return LAPF_OK;
@@ -2461,6 +2566,54 @@ int lapf_sampler_set_frame_widths(lapf_sampler* s, const double* widths, void* s
     };
     if (s->fw) return put();   // later calls replace the widths and keep the snapshot
     return enable_parts(s, {{(void**)&s->fw, fw_bytes(s), kKeep}, {(void**)&s->fw_snap, fw_snap_bytes(s), 0}}, true, st, put);
+}
+
+int lapf_sampler_set_priors(lapf_sampler* s, const double* table, void* stream) {
+    if (!s || !table) return fail(LAPF_ERR_INVALID, "sampler/table is NULL");
+    const int F = s->cfg.problem.n_frames, P = s->P;
+    const size_t n = (size_t)F * P * 4;
+    std::vector<double> h(2 * n);                        // {lo, hi, mu, h} for the kernels, then the table as given
+    for (int f = 0; f < F; ++f)
+        for (int j = 0; j < P; ++j) {
+            const double* e = table + ((size_t)f * P + j) * 4;
+            const double lo = e[0], hi = e[1], mu = e[2], sg = e[3];
+            if (lo != lo || hi != hi || mu != mu || sg != sg)
+                return fail(LAPF_ERR_INVALID, "prior of frame %d, parameter %d has a nan entry", f, j);
+            if (lo > hi) return fail(LAPF_ERR_INVALID, "prior of frame %d, parameter %d: lo %g > hi %g", f, j, lo, hi);
+            if (!(sg > 0.0)) return fail(LAPF_ERR_INVALID, "prior of frame %d, parameter %d: sigma %g <= 0", f, j, sg);
+            if (std::isfinite(sg) && !std::isfinite(mu))
+                return fail(LAPF_ERR_INVALID, "prior of frame %d, parameter %d: mu %g is not finite and sigma %g is", f, j,
+                            mu, sg);
+            const double hh = std::isinf(sg) ? 0.0 : 0.5 / (sg * sg);
+            if (!std::isfinite(hh))
+                return fail(LAPF_ERR_INVALID, "prior of frame %d, parameter %d: sigma %g is too small", f, j, sg);
+            double* d = h.data() + ((size_t)f * P + j) * 4;
+            d[0] = lo; d[1] = hi; d[2] = mu; d[3] = hh;
+            memcpy(h.data() + n + ((size_t)f * P + j) * 4, e, 4 * sizeof(double));
+        }
+    cudaStream_t st = (cudaStream_t)stream;
+    double* tmp = nullptr;
+    CU(cudaMallocAsync((void**)&tmp, 2 * prior_bytes(s), st));
+    cudaError_t e = cudaMemcpyAsync(tmp, h.data(), 2 * prior_bytes(s), cudaMemcpyHostToDevice, st);
+    int rc = e == cudaSuccess ? prior_check(s, s->state, P + 1, tmp, "priors refused", st)   // synchronises: `h` is settled
+                              : fail(LAPF_ERR_CUDA, "copy of the priors failed: %s", cudaGetErrorString(e));
+    auto put = [&]() -> int {
+        CU(cudaMemcpyAsync(s->pr, tmp, prior_bytes(s), cudaMemcpyDeviceToDevice, st));
+        CU(cudaMemcpyAsync(s->pr_given, tmp + n, prior_bytes(s), cudaMemcpyDeviceToDevice, st));
+        return LAPF_OK;
+    };
+    if (!rc) rc = s->pr ? put()             // later calls replace the table
+                        : enable_parts(s, {{(void**)&s->pr, prior_bytes(s), kKeep}, {(void**)&s->pr_given, prior_bytes(s), kKeep}},
+                                       true, st, put);
+    cudaFreeAsync(tmp, st);
+    return rc;
+}
+
+int lapf_sampler_priors(lapf_sampler* s, double* out, void* stream) {
+    if (!s || !out) return fail(LAPF_ERR_INVALID, "sampler/out is NULL");
+    if (!s->pr) return fail(LAPF_ERR_INVALID, "priors are not on (lapf_sampler_set_priors)");
+    CU(cudaMemcpyAsync(out, s->pr_given, prior_bytes(s), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+    return LAPF_OK;
 }
 
 int lapf_sampler_frame_widths(lapf_sampler* s, double* out, void* stream) {

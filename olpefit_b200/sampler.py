@@ -17,6 +17,21 @@ from . import _lib
 from .model import PixelDomain, _stream_ptr
 
 
+def prior_table(n_frames, nparam, lo=None, hi=None, mu=None, sigma=None):
+    """The [F, P, 4] {lo, hi, mu, sigma} table of lapf_sampler_set_priors from per-parameter arrays, each [P]
+    (every frame) or [F, P], or None: no bound (-inf / +inf), no Gaussian term (sigma +inf, mu 0)."""
+    out = np.empty((n_frames, nparam, 4), dtype=np.float64)
+    for i, (v, none) in enumerate(((lo, -np.inf), (hi, np.inf), (mu, 0.0), (sigma, np.inf))):
+        if v is None:
+            out[..., i] = none
+            continue
+        a = np.asarray(v.cpu().numpy() if torch.is_tensor(v) else v, dtype=np.float64)
+        if a.shape not in ((nparam,), (n_frames, nparam)):
+            raise ValueError("prior arrays must be [%d] or [%d, %d], got %s" % (nparam, n_frames, nparam, a.shape))
+        out[..., i] = np.broadcast_to(a, (n_frames, nparam))
+    return out
+
+
 class GibbsSampler:
     def __init__(self, domain: PixelDomain, init_params, frame_of=None, *, seed=0, burn_in=0, thin=1,
                  widths=None, id_base=0, id_stride=1, team_warps=0):
@@ -240,6 +255,23 @@ class GibbsSampler:
         if tuple(c.shape) != (self.domain.n_frames, self.nparam, 2):
             raise ValueError("counts must be [%d, %d, 2]" % (self.domain.n_frames, self.nparam))
         _lib.check(self.lib.lapf_sampler_adapt_widths(self._h, c.data_ptr(), float(target), _stream_ptr(self.domain.device)))
+
+    # -- parameter priors: per-epoch boxes and Gaussian terms in the accept rule ------------------
+    def set_priors(self, lo=None, hi=None, mu=None, sigma=None):
+        """From now on the walkers of frame f see, on parameter j, the box lo <= value <= hi and the Gaussian
+        term N(mu, sigma), in chain units.  Each argument is [P] (every frame) or [F, P]; a missing argument
+        means none (lo -inf, hi +inf, sigma +inf), and so do those values in an array.  Refused if a walker's
+        current state lies outside its box.  See include/lapf.h."""
+        table = prior_table(self.domain.n_frames, self.nparam, lo, hi, mu, sigma)
+        arr = (C.c_double * table.size)(*table.reshape(-1).tolist())
+        _lib.check(self.lib.lapf_sampler_set_priors(self._h, arr, _stream_ptr(self.domain.device)))
+
+    def priors(self):
+        """[F, P, 4] float64 device tensor: the table as given, {lo, hi, mu, sigma}."""
+        dev = self.domain.device
+        out = torch.empty((self.domain.n_frames, self.nparam, 4), dtype=torch.float64, device=dev)
+        _lib.check(self.lib.lapf_sampler_priors(self._h, out.data_ptr(), _stream_ptr(dev)))
+        return out
 
     def rows_recorded(self) -> int:
         """Chain rows every walker has recorded since the last reset."""
